@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SpGEMM hot path: SpGEMM GFLOP/s = 2*flop / time for C = A^2 (or A*A^T).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..5] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" is one full SpGEMM (steps 1-3 including allocation, i.e. one iteration of the
 reference's timed loop, /root/reference/spgemm.cu:1133-1357) on operands already resident in HBM
@@ -35,6 +35,9 @@ CONFIG_TEXT = {
     4: "config4: A^2, synthetic cage15-shaped 19-point stencil 172x173x173 (n=5,147,788)",
     5: "config5: conversion + A^2, synthetic R-MAT (see synth.config(5))",
 }
+
+# --dump-outputs writes at most this many entries of C (three float64 arrays: 48 MiB)
+DUMP_ENTRIES = 1 << 21
 
 
 def hbm_peak():
@@ -252,7 +255,12 @@ def main():
     ap.add_argument("--subpanels", type=int, default=0,
                     help="sequential tile-row panels per rank (0 = auto: config 5's C does not fit one GPU in tiled form "
                          "unless it is produced and consumed panel by panel)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write C of the last timed step to DIR/C_{rows,cols,vals}.npy (float64; every entry, or a seeded sample of "
+                         f"{DUMP_ENTRIES} positions of the (row, col)-sorted COO when C is larger) and DIR/C_nnz.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -293,7 +301,7 @@ def main():
 
     tile_products = 0
 
-    def one_step(times=None, kern=None):
+    def one_step(times=None, kern=None, on_result=None):
         nonlocal tile_products
         nnz = tiles = pairs = tile_products = 0
         for pn in panels:               # this rank's panels, one after the other (results freed in between)
@@ -301,6 +309,8 @@ def main():
             C = ctx.spgemm(A, B, times=tp, panel=pn)
             info = C.info
             nnz += info.nnz; tiles += info.tiles; pairs += info.pairs; tile_products += info.tile_products
+            if on_result is not None:
+                on_result(C)
             C.free()
             if times is not None:
                 for f in ("step1_ms", "step2_ms", "step3_ms"):
@@ -309,11 +319,35 @@ def main():
                 for k, v in ctx.kernel_ms().items():
                     kern[k] = kern.get(k, 0.0) + v
         # the path's only exchange: per-shard sizes -> global offsets of every shard of C
-        layout = pdist.exchange_shard_sizes(nnz, tiles, pairs, device="cuda")
-        return layout.totals
+        return pdist.exchange_shard_sizes(nnz, tiles, pairs, device="cuda")
 
     for _ in range(args.warmup):
-        sizes = one_step()
+        layout = one_step()
+
+    # --dump-outputs: positions in the (row, col)-sorted COO of the whole C, seeded, sized from the warm-up's C;
+    # this rank takes those inside its own shard from each of its panels during the last timed step
+    dump_parts, dump_pauses, dump_launches, seen = [], [], 0, 0
+    if args.dump_outputs:
+        total = int(layout.totals[0])
+        pos = np.arange(total) if total <= DUMP_ENTRIES else np.unique(np.random.default_rng(0).integers(0, total, DUMP_ENTRIES))
+        pos = pos[(pos >= layout.nnz_offset) & (pos < layout.nnz_offset + int(layout.sizes[rank, 0]))] - layout.nnz_offset
+
+    def take_sample(C):
+        """Copies the sampled entries of one panel's C to the host; the events around the copy take its time out of the step."""
+        nonlocal seen, dump_launches
+        p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        p0.record(stream)
+        n, launched = C.info.nnz, ctx.launch_count
+        sel = pos[(pos >= seen) & (pos < seen + n)] - seen
+        if sel.size:
+            r, c, v = C.to_coo()
+            dump_parts.append((r[sel], c[sel], v[sel]))
+            del r, c, v                 # unmapping GBs of host memory takes time as well: before the closing event
+        seen += n
+        dump_launches += ctx.launch_count - launched
+        p1.record(stream)
+        dump_pauses.append((p0, p1))
+
     barrier()
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -321,16 +355,16 @@ def main():
     launches0 = ctx.launch_count
     stalls0 = ctx.size_stalls
     step_ms, own_ms, s1, s2, s3, kms = [], [], [], [], [], []
-    for _ in range(args.steps):
+    for step in range(args.steps):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t = pem.Times()
         e0.record(stream)
         kd = {}
-        sizes = one_step(t, kd)
+        layout = one_step(t, kd, take_sample if args.dump_outputs and step == args.steps - 1 else None)
         e1.record(stream)
         barrier()
-        own = e0.elapsed_time(e1)
+        own = e0.elapsed_time(e1) - sum(p0.elapsed_time(p1) for p0, p1 in dump_pauses)
         ms = torch.tensor([own], dtype=torch.float64, device="cuda")
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -338,10 +372,22 @@ def main():
         own_ms.append(own)
         s1.append(t.step1_ms); s2.append(t.step2_ms); s3.append(t.step3_ms)
         kms.append(kd)
-    launches = ctx.launch_count - launches0
+    launches = ctx.launch_count - launches0 - dump_launches
     stalls = ctx.size_stalls - stalls0
     clocks = sampler.stop() if rank == 0 else None
-    c_nnz, c_tiles, c_pairs = (int(x) for x in sizes.tolist())
+    c_nnz, c_tiles, c_pairs = (int(x) for x in layout.totals.tolist())
+    if args.dump_outputs:
+        part = tuple(np.concatenate([p[i] for p in dump_parts]) if dump_parts else np.zeros(0) for i in range(3))
+        parts = [part]
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, part)
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            out = {"C_nnz": np.array([c_nnz])}
+            out.update({k: np.concatenate([p[i] for p in parts]) for i, k in enumerate(("C_rows", "C_cols", "C_vals"))})
+            for k, a in out.items():
+                np.save(os.path.join(args.dump_outputs, k + ".npy"), a.astype(np.float64))
     ms_per_step = float(np.mean(step_ms))
     value = 2.0 * flop / (ms_per_step * 1e6)
     # per-rank figures (imbalance is visible in rank_ms; the dominant kernel's time is the slowest rank's)
@@ -398,7 +444,7 @@ def main():
         A2.free()
         return float(ms[0].item()), int(ms[1].item())
 
-    e2e_ms = [e2e_pass()[0] for _ in range(e2e_warm + max(3, min(args.steps, 5)))]
+    e2e_ms = [e2e_pass()[0] for _ in range(e2e_warm + args.steps)]
     e2e_t = float(np.mean(e2e_ms[e2e_warm:]))
     h2d = int(I.nbytes + J.nbytes + V.nbytes) if world == 1 else int(h2d_rank) * world
     d2h = (2 * 1024 * 2 * 8 + 3 * 8 * 16) * sub * world    # checksum partials + the size read-backs of one step, all ranks
@@ -408,10 +454,10 @@ def main():
         cap = int(1.25 * c_nnz / (world * sub)) + (1 << 20)
         bufs = (torch.empty(cap, dtype=torch.int32, pin_memory=True), torch.empty(cap, dtype=torch.int32, pin_memory=True),
                 torch.empty(cap, dtype=torch.float64, pin_memory=True))
-        runs = [e2e_pass(bufs) for _ in range(1 + 3)]
+        runs = [e2e_pass(bufs) for _ in range(1 + args.steps)]
         coo_t = float(np.mean([r[0] for r in runs[1:]]))
         e2e_coo = {"value": 2.0 * flop / (coo_t * 1e6), "unit": "GFLOP/s", "ms_per_step": coo_t,
-                   "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": runs[-1][1], "steps": 3, "warmup": 1,
+                   "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": runs[-1][1], "steps": args.steps, "warmup": 1,
                    "what": "as e2e, but C itself is pulled into pinned host buffers as (row, col)-sorted COO through "
                            "pem_result_to_coo: 16 bytes per nonzero of C"}
         del bufs

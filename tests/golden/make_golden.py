@@ -40,6 +40,14 @@ CASES = {
     "webbase270k_a2": (lambda: synth.webbase_like(n=270_007, target_nnz=800_000, max_deg=2000), False),
 }
 SUMMARY_ONLY = {"lap256_a2", "lap600_a2", "webbase270k_a2"}   # keep only counts, checksums and a structure hash for the larger ones
+# summary plus this many entries of the dump, for fixtures whose full COO would exceed 1 MB
+SAMPLED = {"webbase_small_a2": 16_384}
+
+
+def sample(r, c, v, k):
+    """A seeded sample of k dump entries: their positions in the (row, col)-sorted COO and the entries."""
+    p = np.sort(np.random.default_rng(0).choice(r.size, min(k, r.size), replace=False)).astype(np.int32)
+    return dict(sample_pos=p, rows_s=r[p], cols_s=c[p], vals_s=v[p])
 
 
 def struct_hash(r, c):
@@ -101,6 +109,9 @@ def main():
         print(meta, flush=True)
         if name in SUMMARY_ONLY:
             np.savez_compressed(os.path.join(out_dir, name + ".npz"), **{k: np.array(x) for k, x in meta.items()})
+        elif name in SAMPLED:
+            np.savez_compressed(os.path.join(out_dir, name + ".npz"), **sample(r, c, v, SAMPLED[name]),
+                                **{k: np.array(x) for k, x in meta.items()})
         else:
             np.savez_compressed(os.path.join(out_dir, name + ".npz"), rows_c=r, cols_c=c, vals_c=v,
                                 **{k: np.array(x) for k, x in meta.items()})

@@ -38,6 +38,14 @@ def _load(name):
     return np.load(os.path.join(HERE, "golden", name + ".npz"))
 
 
+def _check_sample(g, r, c, v):
+    """Fixtures too large to store whole keep a seeded sample of the dump's entries (make_golden.sample)."""
+    if "sample_pos" in g:
+        p = g["sample_pos"]
+        assert np.array_equal(r[p], g["rows_s"]) and np.array_equal(c[p], g["cols_s"])
+        np.testing.assert_allclose(v[p], g["vals_s"], rtol=1e-12, atol=1e-16)
+
+
 def test_every_fixture_has_a_case():
     names = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(HERE, "golden", "*.npz")))
     assert names == sorted(CASES)
@@ -61,6 +69,7 @@ def test_oracle_matches_reference_dump(name):
     elif "struct_hash" in g:
         r, c, v = C.to_coo()
         assert struct_hash(r, c) == int(g["struct_hash"])
+        _check_sample(g, r, c, v)
 
 
 def test_nsparse_path_fixtures_present():
@@ -95,6 +104,7 @@ def test_engine_matches_reference_dump(engine, name):
         r, c, v = C.to_coo()
         assert struct_hash(r, c) == int(g["struct_hash"])
         np.testing.assert_allclose([v.sum(), np.abs(v).sum()], [float(g["val_sum"]), float(g["val_abs_sum"])], rtol=1e-11)
+        _check_sample(g, r, c, v)
     C.free()
     if B is not A:
         B.free()
