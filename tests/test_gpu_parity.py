@@ -13,6 +13,20 @@ pytestmark = pytest.mark.gpu
 RTOL = 1e-12  # north_star tolerance for fp64 values
 
 
+def _assert_bits(v, vo, tag=""):
+    """Bit equality of two value arrays: the sign of zero counts, and a NaN matches any NaN (payloads
+    legitimately differ between the host and the GPU).  np.array_equal would take -0.0 for +0.0 and fail on NaN."""
+    v, vo = np.asarray(v), np.asarray(vo)
+    assert v.dtype == vo.dtype and v.shape == vo.shape, (v.dtype, vo.dtype, v.shape, vo.shape)
+    u = np.uint32 if v.dtype == np.float32 else np.uint64
+    if np.array_equal(v.view(u), vo.view(u)):
+        return
+    nan, nano = np.isnan(v), np.isnan(vo)
+    assert np.array_equal(nan, nano), f"{tag} NaN at {np.flatnonzero(nan != nano)[:10]}"
+    bad = np.flatnonzero((v.view(u) != vo.view(u)) & ~nan)
+    assert bad.size == 0, f"{tag} {bad.size} values differ in their bits, first at {bad[:10]}: {v[bad[:5]]} vs {vo[bad[:5]]}"
+
+
 def _assert_same_C(Cres, Coracle, exact=True):
     r, c, v = Cres.to_coo()
     ro, co, vo = Coracle.to_coo()
@@ -20,7 +34,7 @@ def _assert_same_C(Cres, Coracle, exact=True):
     assert np.array_equal(r, ro) and np.array_equal(c, co)          # structure: bit-exact
     np.testing.assert_allclose(v, vo, rtol=RTOL, atol=0)            # the stated tolerance
     if exact:
-        assert np.array_equal(v, vo)                                 # same fma order => same bits
+        _assert_bits(v, vo)                                          # same fma order => same bits
 
 
 def _check_tiled(T, O):
@@ -173,7 +187,7 @@ def test_fp32_instantiation_matches_fp32_oracle(engine, k):
     ro, co, vo = oC.to_coo()
     assert v.dtype == np.float32 and np.array_equal(r, ro) and np.array_equal(c, co)
     np.testing.assert_allclose(v, vo, rtol=1e-5, atol=0)             # stated fp32 tolerance
-    assert np.array_equal(v, vo)                                     # same fma order => same bits
+    _assert_bits(v, vo)                                              # same fma order => same bits
     # mixing value types and the fp64-only kernels are refused, not silently converted
     A64 = engine.convert_coo(rows, cols, I, J, V)
     with pytest.raises(pem.PemError):
@@ -768,7 +782,7 @@ def _assert_same_C_lowmem(Cres, oC, row0=0):
     assert cnt.size == oC.rows and np.array_equal(cnt, np.diff(oC.ptr))
     assert r.size == 0 or bool(np.all(np.diff(r) >= 0))
     del r, c
-    assert np.array_equal(v, oC.val)                                   # same fma order => same bits (tolerance 1e-12 is implied)
+    _assert_bits(v, oC.val)                                            # same fma order => same bits (tolerance 1e-12 is implied)
 
 
 def test_config3_full_size_matches_oracle(engine):
@@ -892,7 +906,7 @@ def test_fuzz_all_variants_against_oracle(engine):
         v = np.concatenate([x[2] for x in parts])
         tag = f"case {case}: {m}x{n} nnz {I.size} aat {aat} path {path} owner {owner} keep {keep} parts {nparts}"
         assert np.array_equal(r, ro) and np.array_equal(c, co), tag
-        assert np.array_equal(v, vo), tag
+        _assert_bits(v, vo, tag)
         if B is not A:
             B.free()
         A.free()
