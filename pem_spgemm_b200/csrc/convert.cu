@@ -411,9 +411,8 @@ bool is_device_ptr(const void* p)
 int tile_row_flops(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, unsigned long long** d_out)
 {
     uint32_t* b_row_nnz = nullptr;
-    unsigned long long* trf = nullptr;
-    pem_guard<uint32_t> nnz_guard(ctx, b_row_nnz);
-    pem_guard<unsigned long long> trf_guard(ctx, trf);     // handed to the caller on success (nulled below)
+    unsigned long long* trf = nullptr;     // handed to the caller on success
+    pem_guard g(ctx, b_row_nnz, trf);
     PEM_TRY(pem_alloc(ctx, &b_row_nnz, (size_t)B->tile_rows * 16));
     PEM_TRY(pem_alloc(ctx, &trf, (size_t)A->tile_rows));
     PEM_CK(cudaMemsetAsync(b_row_nnz, 0, (size_t)(B->tile_rows ? B->tile_rows : 1) * 16 * 4, ctx->stream));
@@ -428,8 +427,7 @@ int tile_row_flops(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, unsigne
         PEM_LAUNCHED();
     }
     pem_free(ctx, b_row_nnz);
-    *d_out = trf;
-    trf = nullptr;
+    *d_out = std::exchange(trf, nullptr);
     return PEM_OK;
 }
 
@@ -451,162 +449,158 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
     auto wall0 = std::chrono::high_resolution_clock::now();
     if (transpose) { int32_t t = rows; rows = cols; cols = t; }
 
-    pem_tiled* T = new pem_tiled();
+    auto tiled_free = [ctx](pem_tiled* t) { pem_tiled_free(ctx, t); };
+    std::unique_ptr<pem_tiled, decltype(tiled_free)> T(new pem_tiled(), tiled_free);
     T->uid = pem_next_uid();
     T->dtype = dtype;
     T->rows = rows; T->cols = cols; T->nnz = nnz;
     T->tile_rows = (int32_t)(((int64_t)rows + PEM_TILE - 1) / PEM_TILE);
     T->tile_cols = (int32_t)(((int64_t)cols + PEM_TILE - 1) / PEM_TILE);
-    // every temporary of the conversion, so that one cleanup serves every early return
-    int32_t *dI = nullptr, *dJ = nullptr;
-    char* dV = nullptr;
-    bool own = false;
+    int32_t *sI = nullptr, *sJ = nullptr;      // device copies of a COO that came from the host
+    char* sV = nullptr;
     uint64_t *keys = nullptr, *keys_sorted = nullptr;
     uint32_t *pos = nullptr, *pos_sorted = nullptr, *start_tmp = nullptr;
     char* tmp = nullptr;
-    auto fail = [&](int rc) {
-        cudaStreamSynchronize(ctx->copy_stream);    // nothing may still be writing a buffer that goes back to the cache
-        cudaStreamSynchronize(ctx->stream);
-        if (own) { pem_free(ctx, dI); pem_free(ctx, dJ); pem_free(ctx, dV); }
-        pem_free(ctx, keys); pem_free(ctx, keys_sorted); pem_free(ctx, pos); pem_free(ctx, pos_sorted);
-        pem_free(ctx, start_tmp); pem_free(ctx, tmp);
-        pem_tiled_free(ctx, T);
-        return rc;
-    };
-#define CV_TRY(expr) do { int rc_ = (expr); if (rc_ != PEM_OK) return fail(rc_); } while (0)
-#define CV_CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx->fail_cuda(e_, #call, __FILE__, __LINE__)); } while (0)
+    pem_guard g(ctx, sI, sJ, sV, keys, keys_sorted, pos, pos_sorted, start_tmp, tmp);
+    // on failure nothing may still be writing a buffer that goes back to the cache (the copy stream may still be
+    // filling sV or reading pos_sorted): declared after the guard, so it waits before the guard frees
+    struct wait_on_failure {
+        pem_ctx* ctx;
+        pem_tiled** out;
+        ~wait_on_failure()
+        {
+            if (*out) return;
+            cudaStreamSynchronize(ctx->copy_stream);
+            cudaStreamSynchronize(ctx->stream);
+        }
+    } idle{ctx, out};
 
-    CV_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
-    CV_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
+    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
+    PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
     float kernel_ms = 0.f;
 
     if (nnz > 0) {
         int cb = h_bits_for(T->tile_cols), rb = h_bits_for(T->tile_rows);
         // stage the COO on the device if it came from the host (pinned or pageable)
-        own = !is_device_ptr(I);
+        const bool own = !is_device_ptr(I);
         if (own) {
-            CV_TRY(pem_alloc(ctx, &dI, (size_t)nnz));
-            CV_TRY(pem_alloc(ctx, &dJ, (size_t)nnz));
-            CV_TRY(pem_alloc(ctx, &dV, (size_t)nnz * vsz));
-            CV_CK(cudaMemcpyAsync(dI, I, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
-            CV_CK(cudaMemcpyAsync(dJ, J, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
+            PEM_TRY(pem_alloc(ctx, &sI, (size_t)nnz));
+            PEM_TRY(pem_alloc(ctx, &sJ, (size_t)nnz));
+            PEM_TRY(pem_alloc(ctx, &sV, (size_t)nnz * vsz));
+            PEM_CK(cudaMemcpyAsync(sI, I, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
+            PEM_CK(cudaMemcpyAsync(sJ, J, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
             // the values travel on a second stream, behind the coordinates and under key generation + sort
-            CV_CK(cudaEventRecord(ctx->ev_copy[0], ctx->stream));
-            CV_CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
-            CV_CK(cudaMemcpyAsync(dV, V, (size_t)nnz * vsz, cudaMemcpyHostToDevice, ctx->copy_stream));
-            CV_CK(cudaEventRecord(ctx->ev_copy[1], ctx->copy_stream));
-        } else {
-            dI = const_cast<int32_t*>(I); dJ = const_cast<int32_t*>(J); dV = const_cast<char*>(static_cast<const char*>(V));
+            PEM_CK(cudaEventRecord(ctx->ev_copy[0], ctx->stream));
+            PEM_CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
+            PEM_CK(cudaMemcpyAsync(sV, V, (size_t)nnz * vsz, cudaMemcpyHostToDevice, ctx->copy_stream));
+            PEM_CK(cudaEventRecord(ctx->ev_copy[1], ctx->copy_stream));
         }
-        CV_TRY(pem_alloc(ctx, &keys, (size_t)nnz));
-        CV_TRY(pem_alloc(ctx, &keys_sorted, (size_t)nnz));
-        CV_TRY(pem_alloc(ctx, &pos, (size_t)nnz));
-        CV_TRY(pem_alloc(ctx, &pos_sorted, (size_t)nnz));
-        CV_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, (size_t)nnz * vsz));
-        CV_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
+        const int32_t* dI = own ? sI : I;
+        const int32_t* dJ = own ? sJ : J;
+        const char* dV = own ? sV : static_cast<const char*>(V);
+        PEM_TRY(pem_alloc(ctx, &keys, (size_t)nnz));
+        PEM_TRY(pem_alloc(ctx, &keys_sorted, (size_t)nnz));
+        PEM_TRY(pem_alloc(ctx, &pos, (size_t)nnz));
+        PEM_TRY(pem_alloc(ctx, &pos_sorted, (size_t)nnz));
+        PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, (size_t)nnz * vsz));
+        PEM_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
 
         int grid = (int)std::min<int64_t>(pem_div_up(nnz, 256), (int64_t)ctx->sm_count * 32);
         k_make_keys<<<grid, 256, 0, ctx->stream>>>(dI, dJ, nnz, rows, cols, transpose, cb, keys, pos, ctx->d_scalars);
-        ++ctx->launches;
-        CV_CK(cudaGetLastError());
+        PEM_LAUNCHED();
 
         // one radix sort of (key, original position) over the bits in use
         size_t tmp_bytes = 0, tmp2 = 0;
-        CV_CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys, keys_sorted, pos, pos_sorted, nnz, 0, 8 + cb + rb, ctx->stream));
-        CV_TRY(pem_alloc(ctx, &start_tmp, (size_t)nnz + 1));
+        PEM_CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys, keys_sorted, pos, pos_sorted, nnz, 0, 8 + cb + rb, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &start_tmp, (size_t)nnz + 1));
         cub::CountingInputIterator<uint32_t> iota(0);
         HeadPred pred{keys_sorted};
         int64_t* d_count = ctx->d_scalars + SC_COUNT;
-        CV_CK(cub::DeviceSelect::If(nullptr, tmp2, iota, start_tmp, d_count, nnz, pred, ctx->stream));
-        CV_TRY(pem_alloc(ctx, &tmp, std::max(tmp_bytes, tmp2)));
-        CV_CK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, keys_sorted, pos, pos_sorted, nnz, 0, 8 + cb + rb, ctx->stream));
-        CV_CK(cub::DeviceSelect::If(tmp, tmp2, iota, start_tmp, d_count, nnz, pred, ctx->stream));
-        CV_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)nnz));
+        PEM_CK(cub::DeviceSelect::If(nullptr, tmp2, iota, start_tmp, d_count, nnz, pred, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &tmp, std::max(tmp_bytes, tmp2)));
+        PEM_CK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, keys_sorted, pos, pos_sorted, nnz, 0, 8 + cb + rb, ctx->stream));
+        PEM_CK(cub::DeviceSelect::If(tmp, tmp2, iota, start_tmp, d_count, nnz, pred, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)nnz));
         k_rc_idx<<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(keys_sorted, nnz, T->rc_idx);
-        ++ctx->launches;
-        CV_CK(cudaGetLastError());
+        PEM_LAUNCHED();
         if (own) {
             // The values are gathered into tile order on the COPY stream, behind their upload; the engine's
             // stream does not wait here: tile build and the symbolic steps of a product need masks only, so
             // they run underneath the upload.  pem_tiled_wait_vals joins the two streams for the first reader.
-            CV_CK(cudaEventCreateWithFlags(&T->ev_vals, cudaEventDisableTiming));
-            CV_CK(cudaEventRecord(ctx->ev_copy[0], ctx->stream));                  // sorted positions are final
-            CV_CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
+            PEM_CK(cudaEventCreateWithFlags(&T->ev_vals, cudaEventDisableTiming));
+            PEM_CK(cudaEventRecord(ctx->ev_copy[0], ctx->stream));                  // sorted positions are final
+            PEM_CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
             if (dtype == PEM_F32)
                 k_gather_vals<float><<<pem_div_up(nnz, 256), 256, 0, ctx->copy_stream>>>(pos_sorted, reinterpret_cast<const float*>(dV), nnz, reinterpret_cast<float*>(T->vals));
             else
                 k_gather_vals<double><<<pem_div_up(nnz, 256), 256, 0, ctx->copy_stream>>>(pos_sorted, reinterpret_cast<const double*>(dV), nnz, T->vals);
-            ++ctx->launches;
-            CV_CK(cudaGetLastError());
-            CV_CK(cudaEventRecord(T->ev_vals, ctx->copy_stream));
+            PEM_LAUNCHED();
+            PEM_CK(cudaEventRecord(T->ev_vals, ctx->copy_stream));
             T->vals_pending = true;
-            T->pend_buf[0] = pos_sorted; T->pend_buf[1] = dV;                      // freed once the gather is known to be done
-            pos_sorted = nullptr; dV = nullptr;
+            T->pend_buf[0] = std::exchange(pos_sorted, nullptr);                  // freed once the gather is known to be done
+            T->pend_buf[1] = std::exchange(sV, nullptr);
         } else {
             if (dtype == PEM_F32)
                 k_gather_vals<float><<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(pos_sorted, reinterpret_cast<const float*>(dV), nnz, reinterpret_cast<float*>(T->vals));
             else
                 k_gather_vals<double><<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(pos_sorted, reinterpret_cast<const double*>(dV), nnz, T->vals);
-            ++ctx->launches;
-            CV_CK(cudaGetLastError());
+            PEM_LAUNCHED();
         }
         pem_free(ctx, pos);
         pem_free(ctx, pos_sorted);
-        CV_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, PEM_NSCALARS * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CV_CK(cudaStreamSynchronize(ctx->stream));
+        PEM_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, PEM_NSCALARS * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        PEM_CK(cudaStreamSynchronize(ctx->stream));
         pem_free(ctx, tmp);
         pem_free(ctx, keys);
-        if (own) { pem_free(ctx, dI); pem_free(ctx, dJ); }
+        pem_free(ctx, sI);
+        pem_free(ctx, sJ);
         // default contract: the caller's arrays are free again when this call returns, so the host waits for the
         // values' upload (not for their gather); PEM_OPT_ASYNC_VALUES hands that wait to the caller
-        if (own && !ctx->opt_async_vals) CV_CK(cudaEventSynchronize(ctx->ev_copy[1]));
-        if (ctx->h_scalars[SC_ERR] & 1) return fail(ctx->fail(PEM_ERR_RANGE, "COO coordinate outside the matrix"));
+        if (own && !ctx->opt_async_vals) PEM_CK(cudaEventSynchronize(ctx->ev_copy[1]));
+        if (ctx->h_scalars[SC_ERR] & 1) return ctx->fail(PEM_ERR_RANGE, "COO coordinate outside the matrix");
         int64_t cnt = ctx->h_scalars[SC_COUNT];
-        if (cnt >= (int64_t(1) << 31) - 1) return fail(ctx->fail(PEM_ERR_LIMIT, "more than 2^31 tiles"));
+        if (cnt >= (int64_t(1) << 31) - 1) return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 tiles");
         T->tiles = (int32_t)cnt;
         size_t n = (size_t)cnt;
-        CV_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1));
-        CV_CK(cudaMemcpyAsync(T->tile_nnz_ptr, start_tmp, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1));
+        PEM_CK(cudaMemcpyAsync(T->tile_nnz_ptr, start_tmp, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
         pem_free(ctx, start_tmp);
-        CV_TRY(pem_alloc(ctx, &T->masks, n * 16));
-        CV_TRY(pem_alloc(ctx, &T->masks_t, n * 16));
-        CV_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
-        CV_TRY(pem_alloc(ctx, &T->tile_col_idx, n));
-        CV_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
-        CV_TRY(pem_alloc(ctx, &T->col_occ, n));
-        CV_TRY(pem_alloc(ctx, &T->row_occ, n));
-        CV_CK(cudaEventRecord(ctx->ev[0], ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
+        PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16));
+        PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
+        PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n));
+        PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
+        PEM_TRY(pem_alloc(ctx, &T->col_occ, n));
+        PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
+        PEM_CK(cudaEventRecord(ctx->ev[0], ctx->stream));
         k_build_tiles<<<pem_div_up(cnt, 128), 128, 0, ctx->stream>>>(
             keys_sorted, T->tile_nnz_ptr, (int)cnt, (uint32_t)nnz, cb, T->tile_rows, T->masks, T->masks_t,
             T->row_ptr, T->tile_col_idx, T->tile_row_idx, T->tile_row_ptr, T->col_occ, T->row_occ, ctx->d_scalars);
-        ++ctx->launches;
-        CV_CK(cudaGetLastError());
-        CV_CK(cudaEventRecord(ctx->ev[1], ctx->stream));
+        PEM_LAUNCHED();
+        PEM_CK(cudaEventRecord(ctx->ev[1], ctx->stream));
         T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
-        CV_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        CV_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CV_CK(cudaStreamSynchronize(ctx->stream));
+        PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        PEM_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        PEM_CK(cudaStreamSynchronize(ctx->stream));
         pem_free(ctx, keys_sorted);
-        if (ctx->h_scalars[SC_ERR] & 2) return fail(ctx->fail(PEM_ERR_DUPLICATE, "duplicate (i,j) in the COO input"));
+        if (ctx->h_scalars[SC_ERR] & 2) return ctx->fail(PEM_ERR_DUPLICATE, "duplicate (i,j) in the COO input");
         cudaEventElapsedTime(&kernel_ms, ctx->ev[0], ctx->ev[1]);
     } else {
-        CV_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, 1));
-        CV_CK(cudaMemsetAsync(T->tile_nnz_ptr, 0, 4, ctx->stream));
-        CV_TRY(pem_alloc(ctx, &T->vals, 0)); CV_TRY(pem_alloc(ctx, &T->masks, 0)); CV_TRY(pem_alloc(ctx, &T->masks_t, 0));
-        CV_TRY(pem_alloc(ctx, &T->row_ptr, 0)); CV_TRY(pem_alloc(ctx, &T->tile_col_idx, 0));
-        CV_TRY(pem_alloc(ctx, &T->tile_row_idx, 0)); CV_TRY(pem_alloc(ctx, &T->col_occ, 0)); CV_TRY(pem_alloc(ctx, &T->row_occ, 0));
-        CV_TRY(pem_alloc(ctx, &T->rc_idx, 0));
+        PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, 1));
+        PEM_CK(cudaMemsetAsync(T->tile_nnz_ptr, 0, 4, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &T->vals, 0)); PEM_TRY(pem_alloc(ctx, &T->masks, 0)); PEM_TRY(pem_alloc(ctx, &T->masks_t, 0));
+        PEM_TRY(pem_alloc(ctx, &T->row_ptr, 0)); PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, 0));
+        PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, 0)); PEM_TRY(pem_alloc(ctx, &T->col_occ, 0)); PEM_TRY(pem_alloc(ctx, &T->row_occ, 0));
+        PEM_TRY(pem_alloc(ctx, &T->rc_idx, 0));
         T->h_tile_row_ptr.assign((size_t)T->tile_rows + 1, 0);
-        CV_CK(cudaStreamSynchronize(ctx->stream));
+        PEM_CK(cudaStreamSynchronize(ctx->stream));
     }
-#undef CV_TRY
-#undef CV_CK
     if (times) {
         auto wall1 = std::chrono::high_resolution_clock::now();
         times->convert_kernel_ms = kernel_ms;
         times->convert_total_ms = std::chrono::duration<double, std::milli>(wall1 - wall0).count();
     }
-    *out = T;
+    *out = T.release();
     return PEM_OK;
 }
 
@@ -650,36 +644,28 @@ int pem_convert_csr(pem_ctx* ctx, int32_t rows, int32_t cols, const int32_t* row
     // everything onto the device (the row pointer expands to one row index per nonzero there), then the COO path
     int32_t *d_rp = nullptr, *dI = nullptr, *dJ = nullptr;
     double* dV = nullptr;
-    auto cleanup = [&]() {
-        pem_free(ctx, dI);
-        if (!on_device) { pem_free(ctx, d_rp); pem_free(ctx, dJ); pem_free(ctx, dV); }
-    };
-    int rc = pem_alloc(ctx, &dI, (size_t)nnz);
+    pem_guard g(ctx, dI, d_rp, dJ, dV);
+    PEM_TRY(pem_alloc(ctx, &dI, (size_t)nnz));
     const int32_t* rp = row_ptr;
     const int32_t* J = col_idx;
     const double* V = vals;
-    if (rc == PEM_OK && !on_device) {
-        rc = pem_alloc(ctx, &d_rp, (size_t)rows + 1);
-        if (rc == PEM_OK) rc = pem_alloc(ctx, &dJ, (size_t)nnz);
-        if (rc == PEM_OK) rc = pem_alloc(ctx, &dV, (size_t)nnz);
-        cudaError_t e = cudaSuccess;
-        if (rc == PEM_OK) e = cudaMemcpyAsync(d_rp, row_ptr, ((size_t)rows + 1) * 4, cudaMemcpyHostToDevice, ctx->stream);
-        if (rc == PEM_OK && e == cudaSuccess && nnz) e = cudaMemcpyAsync(dJ, col_idx, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream);
-        if (rc == PEM_OK && e == cudaSuccess && nnz) e = cudaMemcpyAsync(dV, vals, (size_t)nnz * 8, cudaMemcpyHostToDevice, ctx->stream);
-        if (rc == PEM_OK && e != cudaSuccess) rc = ctx->fail_cuda(e, "upload of the CSR arrays", __FILE__, __LINE__);
+    if (!on_device) {
+        PEM_TRY(pem_alloc(ctx, &d_rp, (size_t)rows + 1));
+        PEM_TRY(pem_alloc(ctx, &dJ, (size_t)nnz));
+        PEM_TRY(pem_alloc(ctx, &dV, (size_t)nnz));
+        PEM_CK(cudaMemcpyAsync(d_rp, row_ptr, ((size_t)rows + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+        if (nnz) PEM_CK(cudaMemcpyAsync(dJ, col_idx, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
+        if (nnz) PEM_CK(cudaMemcpyAsync(dV, vals, (size_t)nnz * 8, cudaMemcpyHostToDevice, ctx->stream));
         rp = d_rp; J = dJ; V = dV;
     }
-    if (rc == PEM_OK && nnz > 0) {
+    if (nnz > 0) {
         k_csr_rows<<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(rp, rows, nnz, dI);
-        ++ctx->launches;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) rc = ctx->fail_cuda(e, "k_csr_rows", __FILE__, __LINE__);
+        PEM_LAUNCHED();
     }
-    if (rc == PEM_OK) rc = pem_convert_coo(ctx, rows, cols, nnz, dI, J, V, transpose, out, times);
-    cleanup();
-    if (rc == PEM_OK && times)
+    PEM_TRY(pem_convert_coo(ctx, rows, cols, nnz, dI, J, V, transpose, out, times));
+    if (times)
         times->convert_total_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - wall0).count();
-    return rc;
+    return PEM_OK;
 }
 
 }  // extern "C"
@@ -707,6 +693,9 @@ int pem_tiled_build_srow(pem_ctx* ctx, const pem_tiled* Bc)
     if (ctx->cap) return ctx->fail(PEM_ERR_CUDA, "operand cache built inside a graph capture");
     const size_t rows16 = (size_t)B->tile_rows * 16;
     int64_t* ptr = nullptr;
+    int32_t* tl = nullptr;
+    unsigned* cursor = nullptr;
+    pem_guard g(ctx, ptr, tl, cursor);
     PEM_TRY(pem_alloc(ctx, &ptr, rows16 + 1));
     PEM_CK(cudaMemsetAsync(ptr, 0, (rows16 + 1) * 8, ctx->stream));
     if (B->tiles) {
@@ -718,19 +707,17 @@ int pem_tiled_build_srow(pem_ctx* ctx, const pem_tiled* Bc)
     PEM_CK(cudaMemcpyAsync(ctx->h_scalars, ptr + rows16, 8, cudaMemcpyDeviceToHost, ctx->stream));
     PEM_CK(cudaStreamSynchronize(ctx->stream));
     const int64_t total = ctx->h_scalars[0];
-    int32_t* tl = nullptr;
     PEM_TRY(pem_alloc(ctx, &tl, (size_t)total));
     if (B->tiles) {
-        unsigned* cursor = nullptr;
         PEM_TRY(pem_alloc(ctx, &cursor, rows16));
         PEM_CK(cudaMemsetAsync(cursor, 0, rows16 * 4, ctx->stream));
         k_srow_fill<<<pem_div_up(B->tiles, 256), 256, 0, ctx->stream>>>(B->row_occ, B->tile_row_idx, B->tiles, ptr, cursor, tl);
         PEM_LAUNCHED();
         pem_free(ctx, cursor);
     }
-    B->srow_ptr = ptr;
+    B->srow_ptr = std::exchange(ptr, nullptr);
     B->srow_total = total;
-    B->srow_tile = tl;
+    B->srow_tile = std::exchange(tl, nullptr);
     return PEM_OK;
 }
 
@@ -743,17 +730,19 @@ int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* Tc, bool as_a, bool as_
         return ctx->fail(PEM_ERR_CUDA, "operand cache built inside a graph capture");
     if (as_a && !T->row_rec) {
         uint32_t* rec = nullptr;
+        pem_guard g(ctx, rec);
         PEM_TRY(pem_alloc(ctx, &rec, n16));
         if (n16) {
             k_row_rec<<<pem_div_up((int64_t)n16, 256), 256, 0, ctx->stream>>>(T->masks, T->row_ptr, (int64_t)n16, rec);
             PEM_LAUNCHED();
         }
-        T->row_rec = rec;
+        T->row_rec = std::exchange(rec, nullptr);
     }
     if (as_b && !T->col_rec) {
         PEM_TRY(pem_tiled_wait_vals(ctx, T));
         uint32_t* rec = nullptr;
         double* vt = nullptr;
+        pem_guard g(ctx, rec, vt);
         PEM_TRY(pem_alloc(ctx, &rec, n16));
         PEM_TRY(pem_alloc_bytes(ctx, (void**)&vt, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype))));
         if (T->tiles) {
@@ -765,8 +754,8 @@ int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* Tc, bool as_a, bool as_
                                                                                        T->vals, rec, vt);
             PEM_LAUNCHED();
         }
-        T->col_rec = rec;
-        T->vals_t = vt;
+        T->col_rec = std::exchange(rec, nullptr);
+        T->vals_t = std::exchange(vt, nullptr);
     }
     return PEM_OK;
 }
@@ -780,7 +769,8 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
     *out = nullptr;
     PEM_CK(cudaSetDevice(ctx->device));
     PEM_TRY(pem_tiled_wait_vals(ctx, A));
-    pem_tiled* T = new pem_tiled();
+    auto tiled_free = [ctx](pem_tiled* t) { pem_tiled_free(ctx, t); };
+    std::unique_ptr<pem_tiled, decltype(tiled_free)> T(new pem_tiled(), tiled_free);
     T->uid = pem_next_uid();
     T->dtype = A->dtype;
     T->rows = A->cols; T->cols = A->rows; T->nnz = A->nnz;
@@ -790,42 +780,34 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
     int32_t *ids = nullptr, *perm = nullptr;
     int64_t* nptr = nullptr;
     char* tmp = nullptr;
-    auto fail = [&](int rc) {
-        pem_free(ctx, keys); pem_free(ctx, keys2); pem_free(ctx, ids); pem_free(ctx, perm); pem_free(ctx, nptr); pem_free(ctx, tmp);
-        pem_tiled_free(ctx, T);
-        return rc;
-    };
-#define TR_TRY(expr) do { int rc_ = (expr); if (rc_ != PEM_OK) return fail(rc_); } while (0)
-#define TR_CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx->fail_cuda(e_, #call, __FILE__, __LINE__)); } while (0)
-    TR_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
-    TR_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
-    TR_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype)))); TR_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz));
-    TR_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); TR_TRY(pem_alloc(ctx, &T->masks, n * 16));
-    TR_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); TR_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
-    TR_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); TR_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
-    TR_TRY(pem_alloc(ctx, &T->col_occ, n)); TR_TRY(pem_alloc(ctx, &T->row_occ, n));
+    pem_guard g(ctx, keys, keys2, ids, perm, nptr, tmp);
+    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
+    PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
+    PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype)))); PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz));
+    PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
+    PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
+    PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
+    PEM_TRY(pem_alloc(ctx, &T->col_occ, n)); PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
     if (n == 0) {
-        TR_CK(cudaMemsetAsync(T->tile_nnz_ptr, 0, 4, ctx->stream));
+        PEM_CK(cudaMemsetAsync(T->tile_nnz_ptr, 0, 4, ctx->stream));
         T->h_tile_row_ptr.assign((size_t)T->tile_rows + 1, 0);
-        *out = T;
+        *out = T.release();
         return PEM_OK;
     }
     const int rbits = h_bits_for(A->tile_rows), cbits = h_bits_for(A->tile_cols);
-    TR_TRY(pem_alloc(ctx, &keys, n)); TR_TRY(pem_alloc(ctx, &keys2, n));
-    TR_TRY(pem_alloc(ctx, &ids, n)); TR_TRY(pem_alloc(ctx, &perm, n));
-    TR_TRY(pem_alloc(ctx, &nptr, n + 1));
+    PEM_TRY(pem_alloc(ctx, &keys, n)); PEM_TRY(pem_alloc(ctx, &keys2, n));
+    PEM_TRY(pem_alloc(ctx, &ids, n)); PEM_TRY(pem_alloc(ctx, &perm, n));
+    PEM_TRY(pem_alloc(ctx, &nptr, n + 1));
     k_transpose_keys<<<pem_div_up((int64_t)n, 256), 256, 0, ctx->stream>>>(A->tile_row_idx, A->tile_col_idx, (int)n, rbits, keys, ids);
-    ++ctx->launches;
-    TR_CK(cudaGetLastError());
+    PEM_LAUNCHED();
     size_t tb = 0;
-    TR_CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, keys, keys2, ids, perm, (int64_t)n, 0, rbits + cbits, ctx->stream));
-    TR_TRY(pem_alloc(ctx, &tmp, tb));
-    TR_CK(cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys2, ids, perm, (int64_t)n, 0, rbits + cbits, ctx->stream));
+    PEM_CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, keys, keys2, ids, perm, (int64_t)n, 0, rbits + cbits, ctx->stream));
+    PEM_TRY(pem_alloc(ctx, &tmp, tb));
+    PEM_CK(cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys2, ids, perm, (int64_t)n, 0, rbits + cbits, ctx->stream));
     ctx->launches += 2 + (rbits + cbits + 7) / 8;
     k_transpose_counts<<<pem_div_up((int64_t)n + 1, 256), 256, 0, ctx->stream>>>(perm, A->tile_nnz_ptr, (int)n, nptr);
-    ++ctx->launches;
-    TR_CK(cudaGetLastError());
-    TR_TRY(pem_scan_exclusive_i64(ctx, nptr, (int64_t)n + 1));
+    PEM_LAUNCHED();
+    PEM_TRY(pem_scan_exclusive_i64(ctx, nptr, (int64_t)n + 1));
     if (A->dtype == PEM_F32)
         k_transpose_tiles<float><<<pem_div_up((int64_t)n, 128), 128, 0, ctx->stream>>>(
             (int)n, T->tile_rows, perm, nptr, A->tile_nnz_ptr, A->masks, A->masks_t, A->tile_row_idx, A->tile_col_idx, A->col_occ,
@@ -836,15 +818,12 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
             (int)n, T->tile_rows, perm, nptr, A->tile_nnz_ptr, A->masks, A->masks_t, A->tile_row_idx, A->tile_col_idx, A->col_occ,
             A->row_occ, A->rc_idx, A->vals, T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr, T->tile_row_idx, T->tile_col_idx,
             T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx, T->vals);
-    ++ctx->launches;
-    TR_CK(cudaGetLastError());
+    PEM_LAUNCHED();
     T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
-    TR_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    TR_CK(cudaStreamSynchronize(ctx->stream));
-#undef TR_TRY
-#undef TR_CK
+    PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PEM_CK(cudaStreamSynchronize(ctx->stream));
     pem_free(ctx, keys); pem_free(ctx, keys2); pem_free(ctx, ids); pem_free(ctx, perm); pem_free(ctx, nptr); pem_free(ctx, tmp);
-    *out = T;
+    *out = T.release();
     return PEM_OK;
 }
 
@@ -854,6 +833,7 @@ int pem_count_flop(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, uint64_
     if (A->cols != B->rows) return ctx->fail(PEM_ERR_ARG, "inner dimensions differ");
     PEM_CK(cudaSetDevice(ctx->device));
     unsigned long long* trf = nullptr;
+    pem_guard g(ctx, trf);
     PEM_TRY(tile_row_flops(ctx, A, B, &trf));
     std::vector<unsigned long long> h((size_t)A->tile_rows);
     if (A->tile_rows) PEM_CK(cudaMemcpyAsync(h.data(), trf, h.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -871,7 +851,8 @@ int pem_partition_panels(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, i
     if (A->cols != B->rows) return ctx->fail(PEM_ERR_ARG, "inner dimensions differ");
     PEM_CK(cudaSetDevice(ctx->device));
     const size_t ntr = (size_t)A->tile_rows;
-    unsigned long long* trf = nullptr;
+    unsigned long long *trf = nullptr, *cp = nullptr, *cs = nullptr;
+    pem_guard g(ctx, trf, cp, cs);
     PEM_TRY(tile_row_flops(ctx, A, B, &trf));
     std::vector<unsigned long long> h(ntr), hp(ntr, 0), hs(ntr, 0);
     if (ntr) PEM_CK(cudaMemcpyAsync(h.data(), trf, ntr * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -881,7 +862,6 @@ int pem_partition_panels(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, i
     // (hub rows: many flops in few tiles; ordinary rows: one pair per C tile).
     if (A->tiles && B->tiles) {
         PEM_TRY(pem_tiled_build_srow(ctx, B));
-        unsigned long long *cp = nullptr, *cs = nullptr;
         PEM_TRY(pem_alloc(ctx, &cp, ntr));
         PEM_TRY(pem_alloc(ctx, &cs, ntr));
         PEM_CK(cudaMemsetAsync(cp, 0, ntr * 8, ctx->stream));

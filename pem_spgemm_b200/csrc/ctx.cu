@@ -436,17 +436,11 @@ void pem_result_free(pem_ctx* ctx, pem_result* C)
     if (C->graph) {
         // buffers borrowed from a product graph stay in its arena (the graph may run again now); anything added to
         // the result later (Ctiles_rowColIdx on demand) was allocated the ordinary way
-        void** fields[] = {(void**)&C->row_ptr, (void**)&C->tile_row, (void**)&C->tile_col, (void**)&C->pair_ptr,
-                           (void**)&C->pair_list, (void**)&C->pair_hit, (void**)&C->blk_tile, (void**)&C->pair_blk,
-                           (void**)&C->masks, (void**)&C->tile_nnz_ptr, (void**)&C->row_col_idx, (void**)&C->vals};
-        for (void** f : fields)
+        for (void** f : C->buffers())
             if (*f && C->graph->owned.count(*f)) *f = nullptr;
         C->graph->busy = false;
     }
-    pem_free(ctx, C->row_ptr); pem_free(ctx, C->tile_row); pem_free(ctx, C->tile_col);
-    pem_free(ctx, C->pair_ptr); pem_free(ctx, C->pair_list); pem_free(ctx, C->pair_hit); pem_free(ctx, C->blk_tile); pem_free(ctx, C->pair_blk);
-    pem_free(ctx, C->masks); pem_free(ctx, C->tile_nnz_ptr); pem_free(ctx, C->row_col_idx);
-    pem_free(ctx, C->vals);
+    for (void** f : C->buffers()) pem_free(ctx, *f);
     delete C;
 }
 
@@ -460,6 +454,7 @@ int pem_scan_exclusive_i64(pem_ctx* ctx, int64_t* d, int64_t n)
     size_t tmp_bytes = 0;
     PEM_CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d, d, n, ctx->stream));
     char* tmp = nullptr;
+    pem_guard g(ctx, tmp);
     PEM_TRY(pem_alloc(ctx, &tmp, tmp_bytes));
     PEM_CK(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, d, d, n, ctx->stream));
     pem_free(ctx, tmp);

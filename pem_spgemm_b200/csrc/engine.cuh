@@ -3,14 +3,17 @@
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 
+#include <array>
 #include <cstdint>
 #include <cstdio>
 #include <atomic>
 #include <map>
 #include <memory>
 #include <string>
+#include <tuple>
 #include <unordered_map>
 #include <unordered_set>
+#include <utility>
 #include <vector>
 
 #include "pemspgemm.h"
@@ -151,14 +154,15 @@ static inline void pem_free(pem_ctx* ctx, T*& p)
     p = nullptr;
 }
 
-// a local temporary that goes back to the cache on EVERY return path (the PEM_TRY / PEM_CK early returns included);
-// the success path keeps its explicit pem_free, which nulls the pointer, so nothing is freed twice or later than before
-template <class T>
+// local temporaries that go back to the cache on EVERY return path (the PEM_TRY / PEM_CK early returns included):
+// `pem_guard g(ctx, keys, pos, tmp);`.  Whatever is still held at a return is freed there, in the order listed; a
+// block the code is done with earlier keeps its explicit pem_free, which nulls the pointer, so nothing is freed twice
+template <class... T>
 struct pem_guard {
     pem_ctx* ctx;
-    T*& p;
-    pem_guard(pem_ctx* c, T*& q) : ctx(c), p(q) {}
-    ~pem_guard() { pem_free(ctx, p); }
+    std::tuple<T*&...> p;
+    explicit pem_guard(pem_ctx* c, T*&... q) : ctx(c), p(q...) {}
+    ~pem_guard() { std::apply([this](auto&... q) { (pem_free(ctx, q), ...); }, p); }
     pem_guard(const pem_guard&) = delete;
     pem_guard& operator=(const pem_guard&) = delete;
 };
@@ -241,6 +245,13 @@ struct pem_result {
     int32_t* pair_blk = nullptr;      // first tile of each 256-pair step-2 block (optional by-product of step 1)
     double* vals = nullptr;           // [nnz]
     std::shared_ptr<pem_graph> graph; // set when the buffers above belong to a product graph's arena (pem_result_free hands them back to it)
+    // every device buffer above, in the order pem_result_free releases them
+    std::array<void**, 12> buffers()
+    {
+        return {(void**)&row_ptr, (void**)&tile_row, (void**)&tile_col, (void**)&pair_ptr, (void**)&pair_list,
+                (void**)&pair_hit, (void**)&blk_tile, (void**)&pair_blk, (void**)&masks, (void**)&tile_nnz_ptr,
+                (void**)&row_col_idx, (void**)&vals};
+    }
 };
 
 // A repeated product captured as ONE CUDA graph (PEM_OPT_GRAPHS; pem_spgemm_panel).  The graph bakes device

@@ -101,7 +101,7 @@ int pem_result_to_coo_device(pem_ctx* ctx, const pem_result* C, int32_t* d_rows,
     const int ntr = C->re - C->rb;
     const size_t nrow = (size_t)ntr * 16;
     int64_t* own_rp = nullptr;                 // the row pointer is a temporary unless the caller wants it
-    pem_guard<int64_t> rp_guard(ctx, own_rp);
+    pem_guard g(ctx, own_rp);
     if (!d_row_ptr) PEM_TRY(pem_alloc(ctx, &own_rp, nrow + 1));
     int64_t* rp = d_row_ptr ? d_row_ptr : own_rp;
     PEM_CK(cudaMemsetAsync(rp, 0, (nrow + 1) * 8, ctx->stream));
@@ -133,22 +133,19 @@ static int result_to_coo_any(pem_ctx* ctx, const pem_result* C, int32_t* rows, i
     const size_t vsz = pem_vsize(C->dtype);
     int32_t *dr = nullptr, *dc = nullptr;
     double* dv = nullptr;
+    pem_guard g(ctx, dr, dc, dv);
     size_t n = (size_t)C->nnz;
-    int rc = PEM_OK;
-    if (rows) rc = pem_alloc(ctx, &dr, n);
-    if (cols && rc == PEM_OK) rc = pem_alloc(ctx, &dc, n);
-    if (vals && rc == PEM_OK) rc = pem_alloc_bytes(ctx, (void**)&dv, std::max<size_t>(1, n * vsz));
-    if (rc == PEM_OK) rc = pem_result_to_coo_device(ctx, C, dr, dc, dv, nullptr);
-    if (rc == PEM_OK && n) {
-        cudaError_t e = cudaSuccess;
-        if (rows && e == cudaSuccess) e = cudaMemcpyAsync(rows, dr, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        if (cols && e == cudaSuccess) e = cudaMemcpyAsync(cols, dc, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        if (vals && e == cudaSuccess) e = cudaMemcpyAsync(vals, dv, n * vsz, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = ctx->fail_cuda(e, "D2H copy of the COO result", __FILE__, __LINE__);
+    if (rows) PEM_TRY(pem_alloc(ctx, &dr, n));
+    if (cols) PEM_TRY(pem_alloc(ctx, &dc, n));
+    if (vals) PEM_TRY(pem_alloc_bytes(ctx, (void**)&dv, std::max<size_t>(1, n * vsz)));
+    PEM_TRY(pem_result_to_coo_device(ctx, C, dr, dc, dv, nullptr));
+    if (n) {
+        if (rows) PEM_CK(cudaMemcpyAsync(rows, dr, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (cols) PEM_CK(cudaMemcpyAsync(cols, dc, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (vals) PEM_CK(cudaMemcpyAsync(vals, dv, n * vsz, cudaMemcpyDeviceToHost, ctx->stream));
+        PEM_CK(cudaStreamSynchronize(ctx->stream));
     }
-    pem_free(ctx, dr); pem_free(ctx, dc); pem_free(ctx, dv);
-    return rc;
+    return PEM_OK;
 }
 
 int pem_result_to_coo(pem_ctx* ctx, const pem_result* C, int32_t* rows, int32_t* cols, double* vals)
@@ -171,23 +168,18 @@ int pem_result_to_csr(pem_ctx* ctx, const pem_result* C, int64_t* row_ptr, int32
     int32_t* dc = nullptr;
     double* dv = nullptr;
     int64_t* drp = nullptr;
+    pem_guard g(ctx, dc, dv, drp);
     const size_t n = (size_t)C->nnz;
-    int rc = PEM_OK;
-    if (cols) rc = pem_alloc(ctx, &dc, n);
-    if (vals && rc == PEM_OK) rc = pem_alloc(ctx, &dv, n);
-    if (rc == PEM_OK) rc = pem_alloc(ctx, &drp, (size_t)(C->re - C->rb) * 16 + 1);
-    if (rc == PEM_OK) rc = pem_result_to_coo_device(ctx, C, nullptr, dc, dv, drp);
-    if (rc == PEM_OK) {
-        cudaError_t e = cudaSuccess;
-        // rows past the matrix edge (last tile row) are empty: their pointers equal nnz, so the first nrows + 1 entries are the CSR pointer
-        if (row_ptr) e = cudaMemcpyAsync(row_ptr, drp, ((size_t)nrows + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream);
-        if (cols && n && e == cudaSuccess) e = cudaMemcpyAsync(cols, dc, n * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        if (vals && n && e == cudaSuccess) e = cudaMemcpyAsync(vals, dv, n * 8, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = ctx->fail_cuda(e, "D2H copy of the CSR result", __FILE__, __LINE__);
-    }
-    pem_free(ctx, dc); pem_free(ctx, dv); pem_free(ctx, drp);
-    return rc;
+    if (cols) PEM_TRY(pem_alloc(ctx, &dc, n));
+    if (vals) PEM_TRY(pem_alloc(ctx, &dv, n));
+    PEM_TRY(pem_alloc(ctx, &drp, (size_t)(C->re - C->rb) * 16 + 1));
+    PEM_TRY(pem_result_to_coo_device(ctx, C, nullptr, dc, dv, drp));
+    // rows past the matrix edge (last tile row) are empty: their pointers equal nnz, so the first nrows + 1 entries are the CSR pointer
+    if (row_ptr) PEM_CK(cudaMemcpyAsync(row_ptr, drp, ((size_t)nrows + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (cols && n) PEM_CK(cudaMemcpyAsync(cols, dc, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (vals && n) PEM_CK(cudaMemcpyAsync(vals, dv, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PEM_CK(cudaStreamSynchronize(ctx->stream));
+    return PEM_OK;
 }
 
 int pem_result_checksum(pem_ctx* ctx, const pem_result* C, double* sum, double* abs_sum)
@@ -197,7 +189,7 @@ int pem_result_checksum(pem_ctx* ctx, const pem_result* C, double* sum, double* 
     PEM_CK(cudaSetDevice(ctx->device));
     const int nb = 1024;
     double* part = nullptr;
-    pem_guard<double> part_guard(ctx, part);
+    pem_guard g(ctx, part);
     PEM_TRY(pem_alloc(ctx, &part, (size_t)2 * nb));
     if (C->dtype == PEM_F32) k_checksum_partial<float><<<nb, 256, 0, ctx->stream>>>(reinterpret_cast<const float*>(C->vals), C->nnz, part);
     else k_checksum_partial<double><<<nb, 256, 0, ctx->stream>>>(C->vals, C->nnz, part);

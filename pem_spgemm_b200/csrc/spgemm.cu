@@ -404,12 +404,16 @@ int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem
     if (C->stage != 1) return ctx->fail(PEM_ERR_ARG, "step 2 needs a result fresh from step 1");
     if (C->tiles >= 0x7fffffffLL)
         return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 C' tiles in one result: multiply in tile-row panels (pem_spgemm_panel)");
-    PEM_CK(cudaSetDevice(ctx->device));
-    PEM_TRY(pem_alloc(ctx, &C->masks, (size_t)C->tiles * 16));
-    PEM_TRY(pem_alloc(ctx, &C->tile_nnz_ptr, (size_t)C->tiles + 1));
     const bool rows_variant = ctx->opt_owner == 1;
     if (C->dtype == PEM_F32 && (rows_variant || ctx->opt_owner == 3))
         return ctx->fail(PEM_ERR_ARG, "fp32 products run the default kernels only (PEM_OPT_OWNER 0 / 2 / 4)");
+    const int64_t nblk = (C->pairs + S2P_THREADS - 1) / S2P_THREADS;
+    if (!rows_variant && nblk > 0x7fffffffLL) return ctx->fail(PEM_ERR_LIMIT, "more than 2^39 tile pairs");
+    PEM_CK(cudaSetDevice(ctx->device));
+    // buffers of an earlier call that failed part-way: a retry must not overwrite live blocks
+    pem_free(ctx, C->masks); pem_free(ctx, C->tile_nnz_ptr); pem_free(ctx, C->pair_hit);
+    PEM_TRY(pem_alloc(ctx, &C->masks, (size_t)C->tiles * 16));
+    PEM_TRY(pem_alloc(ctx, &C->tile_nnz_ptr, (size_t)C->tiles + 1));
     if (rows_variant) {
         if (C->tiles > 0) {
             k_step2_masks<<<pem_div_up(C->tiles * 16, 256), 256, 0, ctx->stream>>>(
@@ -420,8 +424,6 @@ int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem
         PEM_LAUNCHED();
         PEM_TRY(pem_scan_exclusive_i64(ctx, C->tile_nnz_ptr, C->tiles + 1));
     } else {
-        const int64_t nblk = (C->pairs + S2P_THREADS - 1) / S2P_THREADS;
-        if (nblk > 0x7fffffffLL) return ctx->fail(PEM_ERR_LIMIT, "more than 2^39 tile pairs");
         // one lane per pair by default; sixteen lanes per C' tile (k_step2_tiles) on request: measured on B200 it
         // loses even on the stencil product it was written for (config 4: 7.1 ms against 3.4 ms)
         const bool by_tiles = ctx->opt_step2_kernel == 2;
@@ -434,7 +436,6 @@ int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem
         // ninth of this kernel's instructions and 4 bytes per pair) are not produced at all
         const bool hits = !(ctx->opt_step2_kernel == 0 && rows_form && !by_tiles && (ctx->opt_owner == 0 || ctx->opt_owner == 4) &&
                             B->nnz >= 8 * (int64_t)B->tiles);
-        C->s2_pairs = true;
         if (hits) PEM_TRY(pem_alloc(ctx, &C->pair_hit, (size_t)nblk * S2P_THREADS));
         if (by_tiles && C->pairs > 0) {
             pem_free(ctx, C->pair_blk);
@@ -449,7 +450,7 @@ int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem
             PEM_CK(cudaMemsetAsync(C->masks, 0, (size_t)C->tiles * 32, ctx->stream));
             int32_t* blk = C->pair_blk;            // expand-sort-compress leaves it behind (k_ctiles)
             C->pair_blk = nullptr;
-            pem_guard<int32_t> blk_guard(ctx, blk);
+            pem_guard g(ctx, blk);
             if (!blk) {
                 PEM_TRY(pem_alloc(ctx, &blk, (size_t)nblk + 1));
                 k_pairblock_tiles<<<pem_div_up(C->tiles, 256), 256, 0, ctx->stream>>>(C->tiles, C->pair_ptr, blk);
@@ -474,7 +475,7 @@ int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem
         size_t tb = 0;
         PEM_CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, nnz_it, C->tile_nnz_ptr, C->tiles + 1, ctx->stream));
         char* tmp = nullptr;
-        pem_guard<char> tmp_guard(ctx, tmp);
+        pem_guard g(ctx, tmp);
         PEM_TRY(pem_alloc(ctx, &tmp, tb));
         PEM_CK(cub::DeviceScan::ExclusiveSum(tmp, tb, nnz_it, C->tile_nnz_ptr, C->tiles + 1, ctx->stream));
         ctx->launches += 2;
@@ -486,6 +487,7 @@ int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem
         PEM_TRY(rd.get(&C->nnz));
     }
     C->stage = 2;
+    C->s2_pairs = !rows_variant;
     // step-3 mapping (step3.cu): the entry-owner kernel unless the tile-class kernel is asked for
     C->s3_entries = ctx->opt_owner != 3;
     return PEM_OK;
@@ -509,21 +511,16 @@ int pem_result_make_rowcolidx(pem_ctx* ctx, pem_result* C)
 // a result whose buffers went back to the allocator behind its back (abandoned graph capture): drop the pointers
 static void result_forget_buffers(pem_result* C)
 {
-    C->row_ptr = nullptr; C->tile_row = nullptr; C->tile_col = nullptr; C->pair_ptr = nullptr; C->pair_list = nullptr;
-    C->pair_hit = nullptr; C->blk_tile = nullptr; C->pair_blk = nullptr; C->masks = nullptr; C->tile_nnz_ptr = nullptr;
-    C->row_col_idx = nullptr; C->vals = nullptr;
+    for (void** f : C->buffers()) *f = nullptr;
 }
 
 // hand every block of an abandoned (or over-budget) graph arena back to ordinary ownership: `keep` are the
 // pointers a live result still uses (they stay live blocks of the context), the rest goes to the cache
-static void graph_dissolve(pem_ctx* ctx, pem_graph* g, const pem_result* keep)
+static void graph_dissolve(pem_ctx* ctx, pem_graph* g, pem_result* keep)
 {
     std::unordered_set<const void*> held;
-    if (keep) {
-        const void* f[] = {keep->row_ptr, keep->tile_row, keep->tile_col, keep->pair_ptr, keep->pair_list, keep->pair_hit,
-                           keep->blk_tile, keep->pair_blk, keep->masks, keep->tile_nnz_ptr, keep->row_col_idx, keep->vals};
-        for (const void* q : f) if (q) held.insert(q);
-    }
+    if (keep)
+        for (void** f : keep->buffers()) if (*f) held.insert(*f);
     for (auto& b : g->arena)
         if (!held.count(b.first) && ctx->live_blocks.count(b.first)) pem_free_bytes(ctx, b.first);
     g->arena.clear(); g->owned.clear(); g->idle.clear(); g->bytes = 0;
@@ -548,13 +545,13 @@ int pem_spgemm_panel(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B,
     // the three steps, enqueued on the context's stream (or captured from it)
     auto run_steps = [&]() -> int {
         PEM_CK(pem_event_record(ctx, ctx->ev[2]));
-        int rc = pem_step1_symbolic(ctx, A, B, rb, re, &C);
+        PEM_TRY(pem_step1_symbolic(ctx, A, B, rb, re, &C));
         pem_event_record(ctx, ctx->ev[3]);
-        if (rc == PEM_OK) rc = pem_step2_symbolic(ctx, A, B, C);
+        PEM_TRY(pem_step2_symbolic(ctx, A, B, C));
         pem_event_record(ctx, ctx->ev[4]);
-        if (rc == PEM_OK) rc = pem_step3_numeric(ctx, A, B, C);
+        PEM_TRY(pem_step3_numeric(ctx, A, B, C));
         pem_event_record(ctx, ctx->ev[5]);
-        return rc;
+        return PEM_OK;
     };
     int redo = 0;
     for (;;) {

@@ -613,7 +613,8 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     if (A->dtype != B->dtype) return ctx->fail(PEM_ERR_ARG, "operands have different value types");
     if (rb < 0 || re < rb || re > A->tile_rows) return ctx->fail(PEM_ERR_ARG, "tile-row panel out of range");
     PEM_CK(cudaSetDevice(ctx->device));
-    pem_result* C = new pem_result();
+    auto result_free = [ctx](pem_result* r) { pem_result_free(ctx, r); };
+    std::unique_ptr<pem_result, decltype(result_free)> C(new pem_result(), result_free);
     C->dtype = A->dtype;
     C->rb = rb; C->re = re; C->rows = A->rows; C->cols = B->cols; C->tile_cols = B->tile_cols;
     const int nrows = re - rb;
@@ -622,11 +623,10 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     // syncs, expand-sort-compress ~20 and 3
     const bool small = (int64_t)A->tiles + B->tiles <= 65536 && B->tile_cols <= 65536;
     if ((ctx->opt_step1_path >= 2 && ctx->opt_step1_path != 5) || (ctx->opt_step1_path == 0 && !small)) {     // expand-sort-compress (step1_esc.cu)
-        int rc = pem_alloc(ctx, &C->row_ptr, (size_t)nrows + 1);
-        if (rc == PEM_OK) rc = pem_step1_esc(ctx, A, B, C);
-        if (rc != PEM_OK) { pem_result_free(ctx, C); return rc; }
+        PEM_TRY(pem_alloc(ctx, &C->row_ptr, (size_t)nrows + 1));
+        PEM_TRY(pem_step1_esc(ctx, A, B, C.get()));
         C->stage = 1;
-        *out = C;
+        *out = C.release();
         return PEM_OK;
     }
     int64_t* pair_row_ptr = nullptr;
@@ -638,25 +638,17 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     int32_t* tmp_j = nullptr;
     unsigned* gscr = nullptr;
     unsigned long long* prof = nullptr;
-    auto cleanup_tmp = [&]() {
-        pem_free(ctx, pair_row_ptr); pem_free(ctx, win); pem_free(ctx, l1s); pem_free(ctx, l1l);
-        pem_free(ctx, l2s); pem_free(ctx, l2l); pem_free(ctx, gscr); pem_free(ctx, prof);
-        pem_free(ctx, lsorted); pem_free(ctx, key_l); pem_free(ctx, key_sorted); pem_free(ctx, sort_tmp);
-        pem_free(ctx, tmp_pq); pem_free(ctx, tmp_j);
-    };
-    auto fail = [&](int rc) { cleanup_tmp(); pem_result_free(ctx, C); return rc; };
-#define S_TRY(expr) do { int rc_ = (expr); if (rc_ != PEM_OK) return fail(rc_); } while (0)
-#define S_CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx->fail_cuda(e_, #call, __FILE__, __LINE__)); } while (0)
-    S_TRY(pem_alloc(ctx, &C->row_ptr, (size_t)nrows + 1));
-    S_TRY(pem_alloc(ctx, &pair_row_ptr, (size_t)nrows + 1));
-    S_TRY(pem_alloc(ctx, &win, (size_t)nrows));
-    S_TRY(pem_alloc(ctx, &l1s, (size_t)nrows)); S_TRY(pem_alloc(ctx, &l1l, (size_t)nrows));
-    S_TRY(pem_alloc(ctx, &l2s, (size_t)nrows)); S_TRY(pem_alloc(ctx, &l2l, (size_t)nrows));
-    S_TRY(pem_alloc(ctx, &lsorted, (size_t)nrows));
-    S_TRY(pem_alloc(ctx, &key_l, (size_t)nrows)); S_TRY(pem_alloc(ctx, &key_sorted, (size_t)nrows));
+    pem_guard g(ctx, pair_row_ptr, win, l1s, l1l, l2s, l2l, gscr, prof, lsorted, key_l, key_sorted, sort_tmp, tmp_pq, tmp_j);
+    PEM_TRY(pem_alloc(ctx, &C->row_ptr, (size_t)nrows + 1));
+    PEM_TRY(pem_alloc(ctx, &pair_row_ptr, (size_t)nrows + 1));
+    PEM_TRY(pem_alloc(ctx, &win, (size_t)nrows));
+    PEM_TRY(pem_alloc(ctx, &l1s, (size_t)nrows)); PEM_TRY(pem_alloc(ctx, &l1l, (size_t)nrows));
+    PEM_TRY(pem_alloc(ctx, &l2s, (size_t)nrows)); PEM_TRY(pem_alloc(ctx, &l2l, (size_t)nrows));
+    PEM_TRY(pem_alloc(ctx, &lsorted, (size_t)nrows));
+    PEM_TRY(pem_alloc(ctx, &key_l, (size_t)nrows)); PEM_TRY(pem_alloc(ctx, &key_sorted, (size_t)nrows));
     size_t sort_bytes = 0;
-    S_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, key_l, key_sorted, l1l, lsorted, nrows > 0 ? nrows : 1, 0, 32, ctx->stream));
-    S_TRY(pem_alloc(ctx, &sort_tmp, sort_bytes));
+    PEM_CK(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, key_l, key_sorted, l1l, lsorted, nrows > 0 ? nrows : 1, 0, 32, ctx->stream));
+    PEM_TRY(pem_alloc(ctx, &sort_tmp, sort_bytes));
     unsigned long long* work = (unsigned long long*)(ctx->d_scalars + SC_WORK0);
     // heavy rows are taken from the work queue heaviest first (longest-processing-time order)
     auto sort_heavy = [&](int32_t*& list, int64_t n) -> int {
@@ -667,9 +659,9 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
         std::swap(list, lsorted);
         return PEM_OK;
     };
-    S_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
-    S_CK(cudaMemsetAsync(C->row_ptr, 0, ((size_t)nrows + 1) * 8, ctx->stream));
-    S_CK(cudaMemsetAsync(pair_row_ptr, 0, ((size_t)nrows + 1) * 8, ctx->stream));
+    PEM_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
+    PEM_CK(cudaMemsetAsync(C->row_ptr, 0, ((size_t)nrows + 1) * 8, ctx->stream));
+    PEM_CK(cudaMemsetAsync(pair_row_ptr, 0, ((size_t)nrows + 1) * 8, ctx->stream));
 
     const bool any = nrows > 0 && A->tiles > 0 && B->tiles > 0;
     int64_t maxwin = 0, maxd = 0, n1s = 0, n1l = 0, n2s = 0, n2l = 0;
@@ -679,12 +671,11 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
         k_row_window<<<pem_div_up((int64_t)nrows * 32, 256), 256, 0, ctx->stream>>>(
             rb, re, A->tile_row_ptr, A->tile_col_idx, B->tile_row_ptr, B->tile_col_idx, win, l1s, l1l, key_l, ctx->d_scalars,
             ctx->opt_step1_path == 5 ? 1 : 0);
-        ++ctx->launches;
-        S_CK(cudaGetLastError());
+        PEM_LAUNCHED();
         int64_t sc[PEM_NSCALARS];
         pem_size_read rd(ctx);
-        S_TRY(rd.add(ctx->d_scalars + SC_MAXWIN, SC_NLARGE2 - SC_MAXWIN + 1));   // the computed sizes only (not the work-queue cursors)
-        S_TRY(rd.get(sc + SC_MAXWIN));
+        PEM_TRY(rd.add(ctx->d_scalars + SC_MAXWIN, SC_NLARGE2 - SC_MAXWIN + 1));   // the computed sizes only (not the work-queue cursors)
+        PEM_TRY(rd.get(sc + SC_MAXWIN));
         maxwin = sc[SC_MAXWIN];
         if (sc[SC_T2]) maxwin = std::max<int64_t>(maxwin, HASH_SLOTS);     // hash rows: table (and sorted columns) in the bitmap's place
         C->tile_products = sc[SC_SUMP];
@@ -699,8 +690,8 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     const int dcap_small = 2048;
     const size_t smem_fill_small = 2 * win_bytes + (size_t)dcap_small * 4;
     if (maxwin > 0 && (smem_fill_small + static_small > budget || 2 * win_bytes + static_large + 32768 > budget))
-        return fail(ctx->fail(PEM_ERR_LIMIT, "step 1: a tile row's column window exceeds the shared-memory bitmap "
-                                             "(more than ~600K tile columns within one tile row's reach)"));
+        return ctx->fail(PEM_ERR_LIMIT, "step 1: a tile row's column window exceeds the shared-memory bitmap "
+                                        "(more than ~600K tile columns within one tile row's reach)");
     // counters of the heavy-row kernel: at most what fits, but only half the SM when 8K counters
     // still fit in that half, so that two heavy-row blocks stay resident per SM
     size_t dl = (budget - 2 * win_bytes - static_large) / 4;
@@ -708,50 +699,48 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     const int dcap_large = (int)dl;
     const size_t smem_fill_large = 2 * win_bytes + (size_t)dcap_large * 4;
     if (n1s + n1l > 0) {
-        S_CK(cudaFuncSetAttribute(k_step1_count<TH_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
-        S_CK(cudaFuncSetAttribute(k_step1_count<TH_LARGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
-        S_TRY(sort_heavy(l1l, n1l));
+        PEM_CK(cudaFuncSetAttribute(k_step1_count<TH_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
+        PEM_CK(cudaFuncSetAttribute(k_step1_count<TH_LARGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
+        PEM_TRY(sort_heavy(l1l, n1l));
         if (n1l > 0) {  // heavy rows first: they are the tail
             int grid = (int)std::min<int64_t>(n1l, (int64_t)ctx->sm_count * 2);
             k_step1_count<TH_LARGE><<<grid, TH_LARGE, win_bytes, ctx->stream>>>(
                 l1l, (int)n1l, rb, A->tile_row_ptr, A->tile_col_idx, A->col_occ, B->tile_row_ptr, B->tile_col_idx,
                 B->row_occ, win, ctx->opt_keep_empty, dcap_small, C->row_ptr, pair_row_ptr, l2s, l2l, key_l, ctx->d_scalars, work + 0);
-            ++ctx->launches;
-            S_CK(cudaGetLastError());
+            PEM_LAUNCHED();
         }
         if (n1s > 0) {
             int grid = (int)std::min<int64_t>(n1s, (int64_t)ctx->sm_count * 16);
             k_step1_count<TH_SMALL><<<grid, TH_SMALL, win_bytes, ctx->stream>>>(
                 l1s, (int)n1s, rb, A->tile_row_ptr, A->tile_col_idx, A->col_occ, B->tile_row_ptr, B->tile_col_idx,
                 B->row_occ, win, ctx->opt_keep_empty, dcap_small, C->row_ptr, pair_row_ptr, l2s, l2l, key_l, ctx->d_scalars, work + 1);
-            ++ctx->launches;
-            S_CK(cudaGetLastError());
+            PEM_LAUNCHED();
         }
-        S_TRY(pem_scan_exclusive_i64(ctx, C->row_ptr, (int64_t)nrows + 1));
-        S_TRY(pem_scan_exclusive_i64(ctx, pair_row_ptr, (int64_t)nrows + 1));
-        S_CK(cudaMemcpyAsync(&ctx->d_scalars[SC_T0], C->row_ptr + nrows, 8, cudaMemcpyDeviceToDevice, ctx->stream));
-        S_CK(cudaMemcpyAsync(&ctx->d_scalars[SC_T1], pair_row_ptr + nrows, 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        PEM_TRY(pem_scan_exclusive_i64(ctx, C->row_ptr, (int64_t)nrows + 1));
+        PEM_TRY(pem_scan_exclusive_i64(ctx, pair_row_ptr, (int64_t)nrows + 1));
+        PEM_CK(cudaMemcpyAsync(&ctx->d_scalars[SC_T0], C->row_ptr + nrows, 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        PEM_CK(cudaMemcpyAsync(&ctx->d_scalars[SC_T1], pair_row_ptr + nrows, 8, cudaMemcpyDeviceToDevice, ctx->stream));
         int64_t sc[PEM_NSCALARS];
         pem_size_read rd(ctx);
-        S_TRY(rd.add(ctx->d_scalars + SC_MAXWIN, SC_NLARGE2 - SC_MAXWIN + 1));   // the computed sizes only (not the work-queue cursors)
-        S_TRY(rd.get(sc + SC_MAXWIN));
+        PEM_TRY(rd.add(ctx->d_scalars + SC_MAXWIN, SC_NLARGE2 - SC_MAXWIN + 1));   // the computed sizes only (not the work-queue cursors)
+        PEM_TRY(rd.get(sc + SC_MAXWIN));
         C->tiles = sc[SC_T0];
         C->pairs = sc[SC_T1];
         maxd = sc[SC_MAXD];
         n2s = sc[SC_NSMALL2]; n2l = sc[SC_NLARGE2];
     }
-    S_TRY(pem_alloc(ctx, &C->tile_row, (size_t)C->tiles));
-    S_TRY(pem_alloc(ctx, &C->tile_col, (size_t)C->tiles));
-    S_TRY(pem_alloc(ctx, &C->pair_ptr, (size_t)C->tiles + 1));
-    S_TRY(pem_alloc(ctx, &C->pair_list, (size_t)C->pairs));
+    PEM_TRY(pem_alloc(ctx, &C->tile_row, (size_t)C->tiles));
+    PEM_TRY(pem_alloc(ctx, &C->tile_col, (size_t)C->tiles));
+    PEM_TRY(pem_alloc(ctx, &C->pair_ptr, (size_t)C->tiles + 1));
+    PEM_TRY(pem_alloc(ctx, &C->pair_list, (size_t)C->pairs));
     if (C->pairs > 0) {
-        S_TRY(pem_alloc(ctx, &tmp_pq, (size_t)C->pairs));
-        S_TRY(pem_alloc(ctx, &tmp_j, (size_t)C->pairs));
+        PEM_TRY(pem_alloc(ctx, &tmp_pq, (size_t)C->pairs));
+        PEM_TRY(pem_alloc(ctx, &tmp_j, (size_t)C->pairs));
     }
     const bool want_prof = ctx->opt_trace > 1;      // PEM_OPT_TRACE = 2: per-phase cycle counters of the bitmap kernels
     if (want_prof) {
-        S_TRY(pem_alloc(ctx, &prof, 16));
-        S_CK(cudaMemsetAsync(prof, 0, 16 * 8, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &prof, 16));
+        PEM_CK(cudaMemsetAsync(prof, 0, 16 * 8, ctx->stream));
     }
     auto report = [&](const char* which, int grid) -> int {
         unsigned long long h[8];
@@ -762,42 +751,36 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
         PEM_CK(cudaMemsetAsync(prof, 0, 16 * 8, ctx->stream));
         return PEM_OK;
     };
-    S_TRY(sort_heavy(l2l, n2l));
+    PEM_TRY(sort_heavy(l2l, n2l));
     if (n2l > 0) {
         const bool two_per_sm = 2 * (smem_fill_large + static_large) <= budget;
         int grid = (int)std::min<int64_t>(n2l, (int64_t)ctx->sm_count * (two_per_sm ? 2 : 1));
         size_t stride = 0;
         if (maxd > dcap_large) {
             stride = (size_t)maxd;
-            S_TRY(pem_alloc(ctx, &gscr, stride * (size_t)grid));
+            PEM_TRY(pem_alloc(ctx, &gscr, stride * (size_t)grid));
         }
-        S_CK(cudaFuncSetAttribute(k_step1_fill<TH_LARGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fill_large));
+        PEM_CK(cudaFuncSetAttribute(k_step1_fill<TH_LARGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fill_large));
         k_step1_fill<TH_LARGE><<<grid, TH_LARGE, smem_fill_large, ctx->stream>>>(
             l2l, (int)n2l, rb, A->tile_row_ptr, A->tile_col_idx, A->col_occ, B->tile_row_ptr, B->tile_col_idx, B->row_occ,
             win, ctx->opt_keep_empty, (int)maxwin, dcap_large, gscr, stride, tmp_pq, tmp_j, C->row_ptr, pair_row_ptr,
             C->tile_row, C->tile_col, C->pair_ptr, C->pair_list, work + 2, prof);
-        ++ctx->launches;
-        S_CK(cudaGetLastError());
-        if (want_prof) S_TRY(report("fill<1024>", grid));
+        PEM_LAUNCHED();
+        if (want_prof) PEM_TRY(report("fill<1024>", grid));
     }
     if (n2s > 0) {
         int grid = (int)std::min<int64_t>(n2s, (int64_t)ctx->sm_count * 16);
-        S_CK(cudaFuncSetAttribute(k_step1_fill<TH_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fill_small));
+        PEM_CK(cudaFuncSetAttribute(k_step1_fill<TH_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fill_small));
         k_step1_fill<TH_SMALL><<<grid, TH_SMALL, smem_fill_small, ctx->stream>>>(
             l2s, (int)n2s, rb, A->tile_row_ptr, A->tile_col_idx, A->col_occ, B->tile_row_ptr, B->tile_col_idx, B->row_occ,
             win, ctx->opt_keep_empty, (int)maxwin, dcap_small, nullptr, 0, tmp_pq, tmp_j, C->row_ptr, pair_row_ptr,
             C->tile_row, C->tile_col, C->pair_ptr, C->pair_list, work + 3, prof);
-        ++ctx->launches;
-        S_CK(cudaGetLastError());
-        if (want_prof) S_TRY(report("fill<128>", grid));
+        PEM_LAUNCHED();
+        if (want_prof) PEM_TRY(report("fill<128>", grid));
     }
     k_set_i64<<<1, 1, 0, ctx->stream>>>(C->pair_ptr, C->tiles, C->pairs);
-    ++ctx->launches;
-    S_CK(cudaGetLastError());
-#undef S_TRY
-#undef S_CK
-    cleanup_tmp();
+    PEM_LAUNCHED();
     C->stage = 1;
-    *out = C;
+    *out = C.release();
     return PEM_OK;
 }

@@ -651,6 +651,20 @@ inline int h_bits(int64_t n)
     return b;
 }
 
+// C's tile arrays, sized for T C' tiles and F pairs (pem_step1_esc left them sized for an empty product)
+int alloc_tiles(pem_ctx* ctx, pem_result* C, int64_t T, int64_t F)
+{
+    if (T >= 0x7fffffffLL)
+        return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 C' tiles in one result: multiply in tile-row panels (pem_spgemm_panel)");
+    C->tiles = T;
+    pem_free(ctx, C->tile_row); pem_free(ctx, C->tile_col); pem_free(ctx, C->pair_ptr);
+    PEM_TRY(pem_alloc(ctx, &C->tile_row, (size_t)T));
+    PEM_TRY(pem_alloc(ctx, &C->tile_col, (size_t)T));
+    PEM_TRY(pem_alloc(ctx, &C->pair_ptr, (size_t)T + 1));
+    pem_free(ctx, C->pair_blk);
+    return pem_alloc(ctx, &C->pair_blk, (size_t)((F + PEM_PAIR_BLOCK - 1) / PEM_PAIR_BLOCK) + 1);
+}
+
 // np work items with product prefix pptr and first-product index bfirst; item_p/srow_tile are null
 // for the tile-level expansion (item i = A tile p0 + i) and set for the row-sliced one
 template <class KeyT, bool SLICED>
@@ -672,18 +686,11 @@ int esc_run(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C,
     char* tmp = nullptr;
     int64_t* heads = nullptr;
     int* seg_off = nullptr;
-    auto cleanup = [&]() {
-        pem_free(ctx, seg_off);
-        pem_free(ctx, split); pem_free(ctx, chunk_off); pem_free(ctx, key_a); pem_free(ctx, key_b);
-        pem_free(ctx, val_a); pem_free(ctx, val_b); pem_free(ctx, tmp); pem_free(ctx, heads);
-    };
-#define E_TRY(expr) do { int rc_ = (expr); if (rc_ != PEM_OK) { cleanup(); return rc_; } } while (0)
-#define E_CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); return ctx->fail_cuda(e_, #call, __FILE__, __LINE__); } } while (0)
-#define E_LAUNCHED() do { ++ctx->launches; E_CK(cudaGetLastError()); } while (0)
-    E_TRY(pem_alloc(ctx, &split, (size_t)nchunks + 1));
-    E_TRY(pem_alloc(ctx, &chunk_off, (size_t)nchunks + 1));
+    pem_guard g(ctx, seg_off, split, chunk_off, key_a, key_b, val_a, val_b, tmp, heads);
+    PEM_TRY(pem_alloc(ctx, &split, (size_t)nchunks + 1));
+    PEM_TRY(pem_alloc(ctx, &chunk_off, (size_t)nchunks + 1));
     k_merge_split<<<pem_div_up((int64_t)nchunks + 1, 256), 256, 0, ctx->stream>>>(nchunks, np, P, pptr, split);
-    E_LAUNCHED();
+    PEM_LAUNCHED();
 
     // One expansion into P-sized buffers (the kept count F <= P is not known on the host yet), compacted on the fly.
     // When P-sized buffers would be too large, count first, read F back and write exactly.
@@ -706,83 +713,74 @@ int esc_run(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C,
     int* ticket = reinterpret_cast<int*>(ctx->d_scalars + SC_T0);      // zeroed with the other scalars at the start of step 1
     if (staged) {
         // one pass: the chunks' counts are chained by look-back while the kernel runs, the kept pairs land compacted
-        E_CK(cudaMemsetAsync(chunk_off, 0, ((size_t)nchunks + 1) * 8, ctx->stream));
-        E_CK(cudaMemsetAsync(ticket, 0, 4, ctx->stream));
+        PEM_CK(cudaMemsetAsync(chunk_off, 0, ((size_t)nchunks + 1) * 8, ctx->stream));
+        PEM_CK(cudaMemsetAsync(ticket, 0, 4, ctx->stream));
         KT_BEGIN(KT_EXPAND);
         k_expand<KeyT, 2, SLICED><<<nchunks, EX_THREADS, 0, ctx->stream>>>(
             np, p0, rb, P, pptr, split, bfirst, item_mask, item_p, B->srow_tile, A->tile_row_idx, B->tile_col_idx,
             B->row_occ, jmin, wbits, ctx->opt_keep_empty, nullptr, chunk_off, ticket, key_a, val_a);
         KT_END(KT_EXPAND);
-        E_LAUNCHED();
+        PEM_LAUNCHED();
     } else {
         k_expand<KeyT, 0, SLICED><<<nchunks, EX_THREADS, 0, ctx->stream>>>(
             np, p0, rb, P, pptr, split, bfirst, item_mask, item_p, B->srow_tile, A->tile_row_idx, B->tile_col_idx,
             B->row_occ, jmin, wbits, ctx->opt_keep_empty, nullptr, chunk_off, nullptr, nullptr, nullptr);
-        E_LAUNCHED();
-        E_CK(cudaMemsetAsync(chunk_off + nchunks, 0, 8, ctx->stream));
-        E_TRY(pem_scan_exclusive_i64(ctx, chunk_off, (int64_t)nchunks + 1));
+        PEM_LAUNCHED();
+        PEM_CK(cudaMemsetAsync(chunk_off + nchunks, 0, 8, ctx->stream));
+        PEM_TRY(pem_scan_exclusive_i64(ctx, chunk_off, (int64_t)nchunks + 1));
     }
     const int64_t* d_F = chunk_off + nchunks;              // kept pairs, on the device
     // Short rows (banded / stencil matrices) are sorted row by row in shared memory: one pass over the
     // pairs.  Power-law inputs have rows of millions of pairs and keep the global radix sort.  Whether every
     // row is short is decided from the longest row, which travels to the host together with F: one stall.
     const bool consider_rows = P < 0x7fffffffLL && wbits + RS_SMALL_BITS <= 32 && !(ctx->opt_esc_variant & 2);
+    // every row's segment of the expanded pairs (key_a) and the longest one, into SC_MAXD (left 0 without consider_rows)
+    auto row_segments = [&]() -> int {
+        PEM_CK(cudaMemsetAsync(ctx->d_scalars + SC_MAXD, 0, 8, ctx->stream));
+        if (!consider_rows) return PEM_OK;
+        PEM_TRY(pem_alloc(ctx, &seg_off, (size_t)nrows + 1));
+        k_row_offsets<KeyT><<<pem_div_up((int64_t)nrows + 1, 256), 256, 0, ctx->stream>>>(nrows, d_F, wbits, key_a, seg_off);
+        PEM_LAUNCHED();
+        k_max_segment<<<pem_div_up(nrows, 256), 256, 0, ctx->stream>>>(nrows, seg_off, ctx->d_scalars);
+        PEM_LAUNCHED();
+        return PEM_OK;
+    };
     if (staged) {
-        E_CK(cudaMemsetAsync(ctx->d_scalars + SC_MAXD, 0, 8, ctx->stream));
-        if (consider_rows) {
-            E_TRY(pem_alloc(ctx, &seg_off, (size_t)nrows + 1));
-            k_row_offsets<KeyT><<<pem_div_up((int64_t)nrows + 1, 256), 256, 0, ctx->stream>>>(nrows, d_F, wbits, key_a, seg_off);
-            E_LAUNCHED();
-            k_max_segment<<<pem_div_up(nrows, 256), 256, 0, ctx->stream>>>(nrows, seg_off, ctx->d_scalars);
-            E_LAUNCHED();
-        }
+        PEM_TRY(row_segments());
         {
             pem_size_read rd(ctx);
             int64_t v[2];
-            E_TRY(rd.add(d_F, 1));
-            E_TRY(rd.add(ctx->d_scalars + SC_MAXD, 1));
-            E_TRY(rd.get(v));
+            PEM_TRY(rd.add(d_F, 1));
+            PEM_TRY(rd.add(ctx->d_scalars + SC_MAXD, 1));
+            PEM_TRY(rd.get(v));
             F = v[0];
             longest_row = v[1];
         }
         tr.mark("expand + compact done, F and the longest row known");
         C->pairs = F;
-        if (F == 0) {
-            cleanup();
-            return PEM_OK;
-        }
+        if (F == 0) return PEM_OK;
     } else {
         {
             pem_size_read rd(ctx);
-            E_TRY(rd.add(d_F, 1));
-            E_TRY(rd.get(&F));
+            PEM_TRY(rd.add(d_F, 1));
+            PEM_TRY(rd.get(&F));
         }
         tr.mark("count pass done, F known");
         C->pairs = F;
-        if (F == 0) {
-            cleanup();
-            return PEM_OK;
-        }
-        E_TRY(pem_alloc(ctx, &key_a, (size_t)F));
-        E_TRY(pem_alloc(ctx, &val_a, (size_t)F));
+        if (F == 0) return PEM_OK;
+        PEM_TRY(pem_alloc(ctx, &key_a, (size_t)F));
+        PEM_TRY(pem_alloc(ctx, &val_a, (size_t)F));
         k_expand<KeyT, 1, SLICED><<<nchunks, EX_THREADS, 0, ctx->stream>>>(
             np, p0, rb, P, pptr, split, bfirst, item_mask, item_p, B->srow_tile, A->tile_row_idx, B->tile_col_idx,
             B->row_occ, jmin, wbits, ctx->opt_keep_empty, chunk_off, nullptr, nullptr, key_a, val_a);
-        E_LAUNCHED();
-        E_TRY(pem_alloc(ctx, &key_b, (size_t)F));
-        E_TRY(pem_alloc(ctx, &val_b, (size_t)F));
-        E_CK(cudaMemsetAsync(ctx->d_scalars + SC_MAXD, 0, 8, ctx->stream));
-        if (consider_rows) {
-            E_TRY(pem_alloc(ctx, &seg_off, (size_t)nrows + 1));
-            k_row_offsets<KeyT><<<pem_div_up((int64_t)nrows + 1, 256), 256, 0, ctx->stream>>>(nrows, d_F, wbits, key_a, seg_off);
-            E_LAUNCHED();
-            k_max_segment<<<pem_div_up(nrows, 256), 256, 0, ctx->stream>>>(nrows, seg_off, ctx->d_scalars);
-            E_LAUNCHED();
-        }
+        PEM_LAUNCHED();
+        PEM_TRY(pem_alloc(ctx, &key_b, (size_t)F));
+        PEM_TRY(pem_alloc(ctx, &val_b, (size_t)F));
+        PEM_TRY(row_segments());
         {
             pem_size_read rd(ctx);
-            E_TRY(rd.add(ctx->d_scalars + SC_MAXD, 1));
-            E_TRY(rd.get(&longest_row));
+            PEM_TRY(rd.add(ctx->d_scalars + SC_MAXD, 1));
+            PEM_TRY(rd.get(&longest_row));
         }
     }
     // (a 1024-thread block sorting up to 32768 pairs of a row was tried for config 3's ~13 K-pair rows:
@@ -798,47 +796,35 @@ int esc_run(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C,
         else
             k_row_sort<KeyT, 128, RS_SMALL_BITS><<<nrows, 128, (size_t)cap * 14 + RS_BMW * 4, ctx->stream>>>(wbits, cap, seg_off, key_a, val_a, key_b, val_b, C->row_ptr);
         KT_END(KT_SORT);
-        E_LAUNCHED();
+        PEM_LAUNCHED();
         std::swap(key_a, key_b);
         std::swap(val_a, val_b);
         pem_free(ctx, key_b);
         pem_free(ctx, val_b);
         // the sort counted every row's C' tiles: their scan is C's row pointer, its last entry the tile count
-        E_TRY(pem_scan_exclusive_i64(ctx, C->row_ptr, (int64_t)nrows + 1));
+        PEM_TRY(pem_scan_exclusive_i64(ctx, C->row_ptr, (int64_t)nrows + 1));
         int64_t T = 0;
         {
             pem_size_read rd(ctx);
-            E_TRY(rd.add(C->row_ptr + nrows, 1));
-            E_TRY(rd.get(&T));
-        }
-        if (T >= 0x7fffffffLL) {
-            cleanup();
-            return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 C' tiles in one result: multiply in tile-row panels (pem_spgemm_panel)");
+            PEM_TRY(rd.add(C->row_ptr + nrows, 1));
+            PEM_TRY(rd.get(&T));
         }
         tr.mark("row sort done, T known");
-        C->tiles = T;
-        pem_free(ctx, C->tile_row); pem_free(ctx, C->tile_col); pem_free(ctx, C->pair_ptr);
-        E_TRY(pem_alloc(ctx, &C->tile_row, (size_t)T));
-        E_TRY(pem_alloc(ctx, &C->tile_col, (size_t)T));
-        E_TRY(pem_alloc(ctx, &C->pair_ptr, (size_t)T + 1));
-        pem_free(ctx, C->pair_blk);
-        E_TRY(pem_alloc(ctx, &C->pair_blk, (size_t)((F + PEM_PAIR_BLOCK - 1) / PEM_PAIR_BLOCK) + 1));
+        PEM_TRY(alloc_tiles(ctx, C, T, F));
         k_row_tiles<KeyT><<<pem_div_up((int64_t)nrows * 32, 256), 256, 0, ctx->stream>>>(
             nrows, rb, wbits, T, F, seg_off, key_a, C->row_ptr, jmin, C->pair_ptr, C->tile_row, C->tile_col, C->pair_blk);
-        E_LAUNCHED();
-        C->pair_list = val_a;
-        val_a = nullptr;
-        cleanup();
+        PEM_LAUNCHED();
+        C->pair_list = std::exchange(val_a, nullptr);
         tr.mark("esc_run end (k_row_tiles launched)");
         return PEM_OK;
     } else {   // stable radix sort by (row, column) over the bits in use
         cub::DoubleBuffer<KeyT> dk(key_a, key_b);
         cub::DoubleBuffer<unsigned long long> dv((unsigned long long*)val_a, (unsigned long long*)val_b);
         size_t tb = 0;
-        E_CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, dk, dv, F, 0, wbits + rbits, ctx->stream));
-        E_TRY(pem_alloc(ctx, &tmp, tb));
+        PEM_CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, dk, dv, F, 0, wbits + rbits, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &tmp, tb));
         KT_BEGIN(KT_SORT);
-        E_CK(cub::DeviceRadixSort::SortPairs(tmp, tb, dk, dv, F, 0, wbits + rbits, ctx->stream));
+        PEM_CK(cub::DeviceRadixSort::SortPairs(tmp, tb, dk, dv, F, 0, wbits + rbits, ctx->stream));
         KT_END(KT_SORT);
         ctx->launches += 2 + (wbits + rbits + 7) / 8;
         pem_free(ctx, tmp);
@@ -848,43 +834,28 @@ int esc_run(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C,
     pem_free(ctx, val_b);
     // heads of the equal-key runs = C' tiles
     int64_t T = 0;
-    E_TRY(pem_alloc(ctx, &heads, (size_t)F));
+    PEM_TRY(pem_alloc(ctx, &heads, (size_t)F));
     {
         size_t tb = 0;
         thrust::counting_iterator<int64_t> iota(0);
         RunHead<KeyT> pred{key_a};
         int64_t* d_n = ctx->d_scalars + SC_COUNT;
-        E_CK(cub::DeviceSelect::If(nullptr, tb, iota, heads, d_n, F, pred, ctx->stream));
-        E_TRY(pem_alloc(ctx, &tmp, tb));
-        E_CK(cub::DeviceSelect::If(tmp, tb, iota, heads, d_n, F, pred, ctx->stream));
+        PEM_CK(cub::DeviceSelect::If(nullptr, tb, iota, heads, d_n, F, pred, ctx->stream));
+        PEM_TRY(pem_alloc(ctx, &tmp, tb));
+        PEM_CK(cub::DeviceSelect::If(tmp, tb, iota, heads, d_n, F, pred, ctx->stream));
         ctx->launches += 2;
         pem_free(ctx, tmp);
         pem_size_read rd(ctx);
-        E_TRY(rd.add(d_n, 1));
-        E_TRY(rd.get(&T));
-    }
-    if (T >= 0x7fffffffLL) {
-        cleanup();
-        return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 C' tiles in one result: multiply in tile-row panels (pem_spgemm_panel)");
+        PEM_TRY(rd.add(d_n, 1));
+        PEM_TRY(rd.get(&T));
     }
     tr.mark("sort+select done, T known");
-    C->tiles = T;
-    pem_free(ctx, C->tile_row); pem_free(ctx, C->tile_col); pem_free(ctx, C->pair_ptr);
-    E_TRY(pem_alloc(ctx, &C->tile_row, (size_t)T));
-    E_TRY(pem_alloc(ctx, &C->tile_col, (size_t)T));
-    E_TRY(pem_alloc(ctx, &C->pair_ptr, (size_t)T + 1));
-    pem_free(ctx, C->pair_blk);
-    E_TRY(pem_alloc(ctx, &C->pair_blk, (size_t)((F + PEM_PAIR_BLOCK - 1) / PEM_PAIR_BLOCK) + 1));
+    PEM_TRY(alloc_tiles(ctx, C, T, F));
     k_ctiles<KeyT><<<pem_div_up(T, 256), 256, 0, ctx->stream>>>(T, F, nrows, rb, wbits, key_a, heads, jmin, C->pair_ptr,
                                                                 C->tile_row, C->tile_col, C->row_ptr, C->pair_blk);
-    E_LAUNCHED();
-    C->pair_list = val_a;
-    val_a = nullptr;
-    cleanup();
+    PEM_LAUNCHED();
+    C->pair_list = std::exchange(val_a, nullptr);
     tr.mark("esc_run end (k_ctiles launched)");
-#undef E_TRY
-#undef E_CK
-#undef E_LAUNCHED
     return PEM_OK;
 }
 
@@ -918,47 +889,39 @@ int pem_step1_esc(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_resu
     int32_t *bfirst = nullptr, *bfirst_s = nullptr, *item_p = nullptr;
     uint16_t* item_mask = nullptr;
     int *jmin = nullptr, *jmax = nullptr;
-    auto cleanup = [&]() {
-        pem_free(ctx, pptr); pem_free(ctx, bfirst); pem_free(ctx, jmin); pem_free(ctx, jmax); pem_free(ctx, icnt);
-        pem_free(ctx, pptr_s); pem_free(ctx, bfirst_s); pem_free(ctx, item_p); pem_free(ctx, item_mask);
-    };
-#define E_TRY(expr) do { int rc_ = (expr); if (rc_ != PEM_OK) { cleanup(); return rc_; } } while (0)
-#define E_CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); return ctx->fail_cuda(e_, #call, __FILE__, __LINE__); } } while (0)
+    pem_guard g(ctx, pptr, bfirst, jmin, jmax, icnt, pptr_s, bfirst_s, item_p, item_mask);
     // PEM_OPT_STEP1_PATH: 3 forces the tile-level expansion, 4 the row-sliced one; otherwise the
     // cheaper of the two (product counts are known before anything is expanded).  Reference-faithful
     // empty tiles exist only at tile level.
     const bool consider_sliced = !ctx->opt_keep_empty && ctx->opt_step1_path != 3;
-    if (consider_sliced) E_TRY(pem_tiled_build_srow(ctx, B));
+    if (consider_sliced) PEM_TRY(pem_tiled_build_srow(ctx, B));
     const int64_t* srow_ptr = consider_sliced ? B->srow_ptr : nullptr;
-    E_TRY(pem_alloc(ctx, &pptr, (size_t)np + 1));
-    E_TRY(pem_alloc(ctx, &bfirst, (size_t)np));
-    if (consider_sliced) E_TRY(pem_alloc(ctx, &icnt, (size_t)np + 1));
-    E_TRY(pem_alloc(ctx, &jmin, (size_t)nrows));
-    E_TRY(pem_alloc(ctx, &jmax, (size_t)nrows));
-    E_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
+    PEM_TRY(pem_alloc(ctx, &pptr, (size_t)np + 1));
+    PEM_TRY(pem_alloc(ctx, &bfirst, (size_t)np));
+    if (consider_sliced) PEM_TRY(pem_alloc(ctx, &icnt, (size_t)np + 1));
+    PEM_TRY(pem_alloc(ctx, &jmin, (size_t)nrows));
+    PEM_TRY(pem_alloc(ctx, &jmax, (size_t)nrows));
+    PEM_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
     k_fill_i32<<<pem_div_up(nrows, 256), 256, 0, ctx->stream>>>(jmin, nrows, INT_MAX);
-    ++ctx->launches;
-    E_CK(cudaMemsetAsync(jmax, 0xFF, (size_t)nrows * 4, ctx->stream));   // -1
+    PEM_LAUNCHED();
+    PEM_CK(cudaMemsetAsync(jmax, 0xFF, (size_t)nrows * 4, ctx->stream));   // -1
     k_tile_products<<<pem_div_up((int64_t)np + 1, 256), 256, 0, ctx->stream>>>(
         p0, np, rb, A->tile_col_idx, A->tile_row_idx, A->col_occ, B->tile_row_ptr, B->tile_col_idx, srow_ptr,
         pptr, bfirst, icnt, jmin, jmax, ctx->d_scalars);
-    ++ctx->launches;
-    E_CK(cudaGetLastError());
-    E_TRY(pem_scan_exclusive_i64(ctx, pptr, (int64_t)np + 1));
+    PEM_LAUNCHED();
+    PEM_TRY(pem_scan_exclusive_i64(ctx, pptr, (int64_t)np + 1));
     k_max_window<<<pem_div_up(nrows, 256), 256, 0, ctx->stream>>>(nrows, jmin, jmax, pptr, np, ctx->d_scalars);
-    ++ctx->launches;
-    E_CK(cudaGetLastError());
+    PEM_LAUNCHED();
     int64_t sc[PEM_NSCALARS];
     {
         pem_size_read rd(ctx);                      // stall 1 of a first product (none when a size plan is replayed)
-        E_TRY(rd.add(ctx->d_scalars + SC_MAXWIN, SC_NLARGE2 - SC_MAXWIN + 1));   // the computed sizes only (not the work-queue cursors)
-        E_TRY(rd.get(sc + SC_MAXWIN));
+        PEM_TRY(rd.add(ctx->d_scalars + SC_MAXWIN, SC_NLARGE2 - SC_MAXWIN + 1));   // the computed sizes only (not the work-queue cursors)
+        PEM_TRY(rd.get(sc + SC_MAXWIN));
     }
     const int64_t P_tile = sc[SC_SUMP];
     const int64_t P_sliced = sc[SC_T2], n_items = sc[SC_T1];
     const int64_t maxw = sc[SC_MAXWIN];
     C->tile_products = P_tile;
-    int rc = PEM_OK;
     if (P_tile > 0) {
         const int wbits = h_bits(maxw), rbits = h_bits(nrows);
         // the sliced expansion pays an extra indirection per product: take it when it at least halves the products
@@ -966,27 +929,23 @@ int pem_step1_esc(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_resu
                             (ctx->opt_step1_path == 4 || 2 * P_sliced < P_tile);
         if (sliced) {
             C->tile_products = P_sliced;
-            E_TRY(pem_scan_exclusive_i64(ctx, icnt, (int64_t)np + 1));
-            E_TRY(pem_alloc(ctx, &pptr_s, (size_t)n_items + 1));
-            E_TRY(pem_alloc(ctx, &bfirst_s, (size_t)n_items));
-            E_TRY(pem_alloc(ctx, &item_p, (size_t)n_items));
-            E_TRY(pem_alloc(ctx, &item_mask, (size_t)n_items));
+            PEM_TRY(pem_scan_exclusive_i64(ctx, icnt, (int64_t)np + 1));
+            PEM_TRY(pem_alloc(ctx, &pptr_s, (size_t)n_items + 1));
+            PEM_TRY(pem_alloc(ctx, &bfirst_s, (size_t)n_items));
+            PEM_TRY(pem_alloc(ctx, &item_p, (size_t)n_items));
+            PEM_TRY(pem_alloc(ctx, &item_mask, (size_t)n_items));
             k_items<<<pem_div_up(np, 256), 256, 0, ctx->stream>>>(p0, np, A->tile_col_idx, A->col_occ, srow_ptr, icnt, n_items,
                                                                   pptr_s, bfirst_s, item_p, item_mask);
-            ++ctx->launches;
-            E_CK(cudaGetLastError());
-            E_TRY(pem_scan_exclusive_i64(ctx, pptr_s, n_items + 1));
+            PEM_LAUNCHED();
+            PEM_TRY(pem_scan_exclusive_i64(ctx, pptr_s, n_items + 1));
             if (wbits + rbits <= 32)
-                rc = esc_run<uint32_t, true>(ctx, A, B, C, p0, (int)n_items, P_sliced, wbits, rbits, pptr_s, bfirst_s, item_mask, item_p, jmin);
+                return esc_run<uint32_t, true>(ctx, A, B, C, p0, (int)n_items, P_sliced, wbits, rbits, pptr_s, bfirst_s, item_mask, item_p, jmin);
             else
-                rc = esc_run<uint64_t, true>(ctx, A, B, C, p0, (int)n_items, P_sliced, wbits, rbits, pptr_s, bfirst_s, item_mask, item_p, jmin);
+                return esc_run<uint64_t, true>(ctx, A, B, C, p0, (int)n_items, P_sliced, wbits, rbits, pptr_s, bfirst_s, item_mask, item_p, jmin);
         } else if (wbits + rbits <= 32)
-            rc = esc_run<uint32_t, false>(ctx, A, B, C, p0, np, P_tile, wbits, rbits, pptr, bfirst, A->col_occ + p0, nullptr, jmin);
+            return esc_run<uint32_t, false>(ctx, A, B, C, p0, np, P_tile, wbits, rbits, pptr, bfirst, A->col_occ + p0, nullptr, jmin);
         else
-            rc = esc_run<uint64_t, false>(ctx, A, B, C, p0, np, P_tile, wbits, rbits, pptr, bfirst, A->col_occ + p0, nullptr, jmin);
+            return esc_run<uint64_t, false>(ctx, A, B, C, p0, np, P_tile, wbits, rbits, pptr, bfirst, A->col_occ + p0, nullptr, jmin);
     }
-#undef E_TRY
-#undef E_CK
-    cleanup();
-    return rc;
+    return PEM_OK;
 }

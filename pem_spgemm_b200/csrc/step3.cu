@@ -536,6 +536,7 @@ static int launch_windows(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, 
     const int64_t n_windows = (C->pairs + NP - 1) / NP;
     if (n_windows > 0x7fffffffLL) return ctx->fail(PEM_ERR_LIMIT, "more than 2^37 tile pairs");
     int32_t* win_tile = nullptr;
+    pem_guard g(ctx, win_tile);
     PEM_TRY(pem_alloc(ctx, &win_tile, (size_t)n_windows + 1));
     k_window_tiles<<<pem_div_up(C->tiles + 1, 256), 256, 0, ctx->stream>>>(C->tiles, n_windows, NP, C->pair_ptr, win_tile);
     PEM_LAUNCHED();
@@ -662,7 +663,6 @@ extern "C" int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_til
     PEM_TRY(pem_tiled_wait_vals(ctx, B));
     if (C->dtype == PEM_F32 && (!C->s2_pairs || !C->s3_entries))
         return ctx->fail(PEM_ERR_ARG, "fp32 products run the default kernels only (PEM_OPT_OWNER 0 / 2 / 4)");
-    PEM_TRY(pem_alloc_bytes(ctx, (void**)&C->vals, std::max<size_t>(1, (size_t)C->nnz * pem_vsize(C->dtype))));
     const bool by_records = C->s2_pairs;                    // step 2 ran the pair kernel
     // dense-tile mode of step 2 (no hit words): only the window kernel can run
     if (by_records && !C->pair_hit && !(C->s3_entries && (ctx->opt_owner == 0 || ctx->opt_owner == 4)))
@@ -674,15 +674,18 @@ extern "C" int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_til
     // (at least four nonzeros per pair: stencil / FEM products), else the entry-owner kernel
     const bool windows = by_records && C->s3_entries &&
                          (ctx->opt_owner == 4 || !C->pair_hit || (ctx->opt_owner == 0 && C->nnz >= 4 * C->pairs));
+    const int64_t nblk_e = (C->nnz + S3E_ENTRIES - 1) / S3E_ENTRIES;      // blocks of the entry-owner kernel
+    if (by_records && C->s3_entries && !windows && nblk_e > 0x7fffffffLL) return ctx->fail(PEM_ERR_LIMIT, "C has more than 2^39 nonzeros");
+    // buffers of an earlier call that failed part-way: a retry must not overwrite live blocks
+    pem_free(ctx, C->vals); pem_free(ctx, C->blk_tile);
+    PEM_TRY(pem_alloc_bytes(ctx, (void**)&C->vals, std::max<size_t>(1, (size_t)C->nnz * pem_vsize(C->dtype))));
     if (C->nnz > 0 && by_records) {                          // views are cached on the handles after the first product
         PEM_TRY(pem_tiled_build_views(ctx, A, true, false));
         PEM_TRY(pem_tiled_build_views(ctx, B, false, true));
         if (use_rc) PEM_TRY(pem_result_make_rowcolidx(ctx, C));   // Ctiles_rowColIdx: every nonzero's (r, c), one byte (spgemm.cu:552-591)
     }
     if (C->nnz > 0 && by_records && C->s3_entries && !windows) {   // entry-owner needs the first tile of each of its blocks
-        const int64_t nblk = (C->nnz + S3E_ENTRIES - 1) / S3E_ENTRIES;
-        if (nblk > 0x7fffffffLL) return ctx->fail(PEM_ERR_LIMIT, "C has more than 2^39 nonzeros");
-        PEM_TRY(pem_alloc(ctx, &C->blk_tile, (size_t)nblk + 1));
+        PEM_TRY(pem_alloc(ctx, &C->blk_tile, (size_t)nblk_e + 1));
         k_block_tiles<<<pem_div_up(C->tiles, 256), 256, 0, ctx->stream>>>(C->tiles, C->tile_nnz_ptr, C->blk_tile);
         PEM_LAUNCHED();
     }
@@ -702,16 +705,15 @@ extern "C" int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_til
     }
     KT_BEGIN(KT_NUMERIC);
     if (C->nnz > 0 && by_records && C->s3_entries) {
-        const int64_t nblk = (C->nnz + S3E_ENTRIES - 1) / S3E_ENTRIES;
 #define S3E_ARGS C->nnz, C->tiles, C->blk_tile, C->tile_nnz_ptr, C->row_col_idx, reinterpret_cast<const uint32_t*>(C->masks), \
             C->pair_ptr, C->pair_list, C->pair_hit, A->tile_nnz_ptr, A->vals, A->row_rec, B->tile_nnz_ptr, B->vals_t, B->col_rec, C->vals
         if (C->dtype == PEM_F32)
-            k_step3_entries<float><<<(unsigned)nblk, S3E_ENTRIES, 0, ctx->stream>>>(
+            k_step3_entries<float><<<(unsigned)nblk_e, S3E_ENTRIES, 0, ctx->stream>>>(
                 C->nnz, C->tiles, C->blk_tile, C->tile_nnz_ptr, C->row_col_idx, reinterpret_cast<const uint32_t*>(C->masks),
                 C->pair_ptr, C->pair_list, C->pair_hit, A->tile_nnz_ptr, reinterpret_cast<const float*>(A->vals), A->row_rec,
                 B->tile_nnz_ptr, reinterpret_cast<const float*>(B->vals_t), B->col_rec, reinterpret_cast<float*>(C->vals));
         else
-            k_step3_entries<double><<<(unsigned)nblk, S3E_ENTRIES, 0, ctx->stream>>>(S3E_ARGS);
+            k_step3_entries<double><<<(unsigned)nblk_e, S3E_ENTRIES, 0, ctx->stream>>>(S3E_ARGS);
 #undef S3E_ARGS
         PEM_LAUNCHED();
     } else if (C->nnz > 0 && by_records) {
