@@ -117,7 +117,14 @@ typedef enum pem_option {
     /* budget for the device memory held by product graphs, MiB (default: a quarter of the memory free at pem_ctx_create);
      * a single graph may hold an eighth of it: products that move gigabytes do not wait for their launches, and the
      * sequential panels of a large product must not park their buffers in graphs */
-    PEM_OPT_GRAPH_LIMIT_MB = 13
+    PEM_OPT_GRAPH_LIMIT_MB = 13,
+    /* tests only: 0 (default) = off; 0x100 | b (0 <= b <= 255) = every device block the context's allocator hands
+     * out (a cached block in full, a new pool block, a block of a product graph's arena) is filled with byte b on the
+     * context's stream before use, so a kernel that reads memory nothing wrote sees b, not the block's previous
+     * contents or fresh zeros.  Inside a graph capture the fill becomes a node of the graph.  Not filled: the
+     * context's scalar slots, pinned host memory and caller buffers.  Costs no kernel launch (memsets only).
+     * Setting the option clears the remembered sizes and graphs, as PEM_OPT_SIZE_PLANS does. */
+    PEM_OPT_POISON = 14
 } pem_option;
 
 /* Milliseconds.  Device times are CUDA-event times on the context's stream; wall times are

@@ -36,6 +36,7 @@ OPT_CACHE_LIMIT_MB = 10
 OPT_SIZE_PLANS = 11
 OPT_GRAPHS = 12
 OPT_GRAPH_LIMIT_MB = 13
+OPT_POISON = 14                  # tests only: 0 or 0x100 | byte fills every allocated device block with that byte
 
 # pem_tiled_array / pem_result_array -> (index, dtype)
 T_ARRAYS = {
@@ -406,6 +407,14 @@ class Result:
         speed); each must hold ``info.nnz`` entries; 0 skips an array."""
         self.ctx._check(load().pem_result_to_coo(self.ctx._h, self._h, C.c_void_p(rows_ptr or None),
                                                  C.c_void_p(cols_ptr or None), C.c_void_p(vals_ptr or None)))
+
+    def to_coo_device(self, rows_ptr, cols_ptr, vals_ptr, row_ptr_ptr=0):
+        """Same, into caller-owned DEVICE buffers given as integer addresses: ``info.nnz`` rows / cols / vals (fp32
+        values for an fp32 result) and, when ``row_ptr_ptr`` is given, the CSR row pointer of the result's tile rows,
+        int64 [(tile_row_end - tile_row_begin) * 16 + 1]; 0 skips an array."""
+        self.ctx._check(load().pem_result_to_coo_device(self.ctx._h, self._h, C.c_void_p(rows_ptr or None),
+                                                        C.c_void_p(cols_ptr or None), C.c_void_p(vals_ptr or None),
+                                                        C.c_void_p(row_ptr_ptr or None)))
 
     def checksum(self):
         s, a = C.c_double(), C.c_double()

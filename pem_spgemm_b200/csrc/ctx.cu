@@ -25,6 +25,19 @@
 // capture reuse them: the graph is one chain, so stream order holds), never back to the shared cache, because
 // the graph bakes their addresses in.  A miss goes to the pool on the COPY stream (the engine's stream is
 // capturing); pem_spgemm_panel drains that stream before the first launch of the graph.
+//
+// PEM_OPT_POISON fills every block handed out with one byte pattern, in stream order on the engine's stream, before
+// the caller sees it: all of it, also the part of a cached block beyond the request.  Every user of a block runs on
+// that stream or waits on an event recorded there after the allocation (the copy stream's value upload and gather
+// in convert.cu), so the fill lands before the block's first use.  Inside a capture the fill is a memset node of the
+// graph, so every launch of the graph poisons its arena again.
+static int poison(pem_ctx* ctx, void* p, size_t bytes)
+{
+    if (!ctx->opt_poison || !bytes) return PEM_OK;
+    PEM_CK(cudaMemsetAsync(p, ctx->opt_poison & 0xFF, bytes, ctx->stream));
+    return PEM_OK;
+}
+
 static int graph_alloc_bytes(pem_ctx* ctx, void** p, size_t bytes)
 {
     pem_graph& g = *ctx->cap;
@@ -36,17 +49,19 @@ static int graph_alloc_bytes(pem_ctx* ctx, void** p, size_t bytes)
     auto it = g.idle.lower_bound(bytes);
     if (it != g.idle.end() && it->first - bytes <= it->first / 4) {
         *p = it->second;
+        size_t sz = it->first;
         g.idle.erase(it);
-        return PEM_OK;
+        return poison(ctx, *p, sz);
     }
     it = ctx->free_blocks.lower_bound(bytes);
     if (it != ctx->free_blocks.end() && it->first - bytes <= it->first / 4) {
         *p = it->second;
-        ctx->live_blocks[*p] = it->first;
-        ctx->cached_bytes -= it->first;
-        own(*p, it->first);
+        size_t sz = it->first;
+        ctx->live_blocks[*p] = sz;
+        ctx->cached_bytes -= sz;
+        own(*p, sz);
         ctx->free_blocks.erase(it);
-        return PEM_OK;
+        return poison(ctx, *p, sz);
     }
     cudaError_t e = cudaMallocFromPoolAsync(p, bytes, ctx->pool, ctx->copy_stream);
     if (e != cudaSuccess) return ctx->fail_cuda(e, "cudaMallocFromPoolAsync (graph arena)", __FILE__, __LINE__);
@@ -55,7 +70,7 @@ static int graph_alloc_bytes(pem_ctx* ctx, void** p, size_t bytes)
     ctx->pool_taken += bytes;
     ++ctx->pool_mallocs;
     own(*p, bytes);
-    return PEM_OK;
+    return poison(ctx, *p, bytes);
 }
 
 int pem_alloc_bytes(pem_ctx* ctx, void** p, size_t bytes)
@@ -66,10 +81,11 @@ int pem_alloc_bytes(pem_ctx* ctx, void** p, size_t bytes)
     auto it = ctx->free_blocks.lower_bound(bytes);
     if (it != ctx->free_blocks.end() && it->first - bytes <= it->first / 4) {
         *p = it->second;
-        ctx->live_blocks[*p] = it->first;
-        ctx->cached_bytes -= it->first;
+        size_t sz = it->first;
+        ctx->live_blocks[*p] = sz;
+        ctx->cached_bytes -= sz;
         ctx->free_blocks.erase(it);
-        return PEM_OK;
+        return poison(ctx, *p, sz);
     }
     if (ctx->cached_bytes > ctx->cache_limit) pem_cache_release(ctx);
     cudaError_t e = cudaMallocFromPoolAsync(p, bytes, ctx->pool, ctx->stream);
@@ -82,7 +98,7 @@ int pem_alloc_bytes(pem_ctx* ctx, void** p, size_t bytes)
     ctx->live_blocks[*p] = bytes;
     ctx->pool_taken += bytes;
     ++ctx->pool_mallocs;
-    return PEM_OK;
+    return poison(ctx, *p, bytes);
 }
 
 void pem_free_bytes(pem_ctx* ctx, void* p)
@@ -253,6 +269,12 @@ int pem_ctx_set_option(pem_ctx* ctx, int option, int64_t value)
         case PEM_OPT_S3_SMALL_PAIRS:
             if (value < 0 || value > (1 << 20)) return ctx->fail(PEM_ERR_ARG, "PEM_OPT_S3_SMALL_PAIRS must be 0..2^20");
             ctx->opt_s3_small_np = (int)value;
+            return PEM_OK;
+        case PEM_OPT_POISON:
+            if (value != 0 && (value < 0x100 || value > 0x1FF))
+                return ctx->fail(PEM_ERR_ARG, "PEM_OPT_POISON must be 0 or 0x100 | byte");
+            ctx->opt_poison = (int)value;
+            ctx->plans.clear();      // a graph captured without the fill nodes must not run again
             return PEM_OK;
     }
     return ctx->fail(PEM_ERR_ARG, "unknown option");

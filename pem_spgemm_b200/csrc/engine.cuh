@@ -62,6 +62,7 @@ struct pem_ctx {
     int opt_async_vals = 0;      // PEM_OPT_ASYNC_VALUES: pem_convert_coo returns while the values' upload is still in flight
     int opt_s3_small_e = 8;      // PEM_OPT_S3_SMALL_NNZ: step 3 handles a tile with at most this many nonzeros ...
     int opt_s3_small_np = 64;    // PEM_OPT_S3_SMALL_PAIRS: ... and at most this many pairs with one thread
+    int opt_poison = 0;          // PEM_OPT_POISON: 0 or 0x100 | byte every allocated block is filled with (tests)
     int sm_count = 148;
     int smem_optin = 227 * 1024; // max dynamic shared memory per block
     int64_t* h_scalars = nullptr; // pinned, PEM_NSCALARS entries: size read-backs
