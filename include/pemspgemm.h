@@ -168,7 +168,7 @@ int pem_ctx_sync(pem_ctx* ctx);
 /* Number of kernels this library launched on ctx since creation (bench.py's gpu_launches). */
 int64_t pem_ctx_launch_count(const pem_ctx* ctx);
 /* Device time (ms, CUDA events on the context's stream) of the four individually timed kernels of
- * the last pem_spgemm / pem_spgemm_panel call: [0] k_expand (step 1 product expansion), [1] the
+ * the last pem_spgemm / pem_spgemm_panel call (pem_spgemm_numeric: [3] only, the others 0): [0] k_expand (step 1 product expansion), [1] the
  * step-1 radix sort, [2] k_step2_pairs, [3] the step-3 numeric kernel.  Returns the count (4). */
 int pem_ctx_kernel_ms(const pem_ctx* ctx, double* ms, int n);
 /* How step 1 of the last product ordered its tile pairs: -1 = no sort (per-row bitmap path), 0 = block-local
@@ -238,11 +238,26 @@ typedef enum pem_tiled_array {
     PEM_T_TILE_ROW_IDX = 7, /* int32   [tiles]    tile row of each tile */
     PEM_T_COL_OCC = 8,      /* uint16  [tiles]    OR of the tile's row masks    */
     PEM_T_ROW_OCC = 9,      /* uint16  [tiles]    OR of the tile's column masks */
-    PEM_T_ROW_COL_IDX = 10  /* uint8   [nnz]      *tiles_rowColIdx: (r<<4)|c per value (spgemm.cu:195,221) */
+    PEM_T_ROW_COL_IDX = 10, /* uint8   [nnz]      *tiles_rowColIdx: (r<<4)|c per value (spgemm.cu:195,221) */
+    PEM_T_VAL_POS = 11      /* uint32  [nnz]      index of each value in the COO / CSR arrays the matrix was converted
+                             *                    from (for a pem_tiled_transpose result: its source's input), the
+                             *                    order pem_tiled_set_values reads V in */
 } pem_tiled_array;
 int pem_tiled_get(pem_ctx* ctx, const pem_tiled* t, int which, void* host_dst, size_t bytes);
 /* Device pointer of the same arrays (no copy; owned by the handle). */
 const void* pem_tiled_device_ptr(const pem_tiled* t, int which);
+
+/* ---- new values on the same pattern ----------------------------------------------------- */
+/* New values for a tiled matrix whose pattern stays: V[nnz] in the order of the COO / CSR arrays the handle was
+ * converted from (for a pem_tiled_transpose result: the order of its source's input, so one V refreshes A and A^T).
+ * Host or device pointer.  Values are written in place: device pointers of the handle, size plans and product graphs
+ * stay valid, and every later product reads the new values.  Results computed earlier keep theirs (see
+ * pem_spgemm_numeric).  A host V is free again when the call returns.  A device V is read in the order of the
+ * context's stream (pem_ctx_stream) without a host wait: the caller orders its own writes to V before this call and
+ * after it on that stream.  A handle converted under PEM_OPT_ASYNC_VALUES first waits for its pending upload.  The
+ * fp64 entry refuses an fp32 matrix and the reverse (PEM_ERR_ARG); nnz == 0 is a no-op. */
+int pem_tiled_set_values(pem_ctx* ctx, pem_tiled* t, const double* V);
+int pem_tiled_set_values_f32(pem_ctx* ctx, pem_tiled* t, const float* V);
 
 /* ---- flop count and panel partition ---------------------------------------------------- */
 /* flop = sum over a_ik of nnz(B row k); replaces the host thread at spgemm.cu:1068-1079. */
@@ -270,6 +285,14 @@ int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B,
                        int32_t tile_row_begin, int32_t tile_row_end, pem_result** C);
 int pem_step2_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C);
 int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C);
+
+/* Recomputes the values of a complete result C of A*B (or of a panel of it) in place from the current values of
+ * A and B, on C's existing structure: step 3 only, same kernel as C's first computation, no allocation of C's
+ * buffers, no size read-back.  Bit-identical to a new pem_spgemm_panel of the same operands and panel.
+ * A and B must be the handles C was computed from (A == B for A^2); PEM_ERR_ARG otherwise, and for a result that
+ * has not completed step 3.  Works on a result handed out by a product graph.  Ends with one synchronisation;
+ * times (may be NULL) gets step3_ms, kernel_ms, total_ms and malloc_ms, with steps 1 and 2 at 0. */
+int pem_spgemm_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C, pem_times* times);
 
 int pem_result_info_get(const pem_result* C, pem_result_info* info);
 void pem_result_free(pem_ctx* ctx, pem_result* C);

@@ -43,7 +43,7 @@ T_ARRAYS = {
     "vals": (0, np.float64), "tile_nnz_ptr": (1, np.uint32), "masks": (2, np.uint16),
     "row_ptr": (3, np.uint8), "masks_t": (4, np.uint16), "tile_row_ptr": (5, np.int32),
     "tile_col_idx": (6, np.int32), "tile_row_idx": (7, np.int32), "col_occ": (8, np.uint16),
-    "row_occ": (9, np.uint16), "row_col_idx": (10, np.uint8),
+    "row_occ": (9, np.uint16), "row_col_idx": (10, np.uint8), "val_pos": (11, np.uint32),
 }
 R_ARRAYS = {
     "row_ptr": (0, np.int64), "tile_row": (1, np.int32), "tile_col": (2, np.int32),
@@ -81,7 +81,7 @@ class ResultInfo(C.Structure):
 EXPORTS = [
     "pem_ctx_create", "pem_ctx_destroy", "pem_last_error", "pem_ctx_set_option", "pem_ctx_stream",
     "pem_ctx_sync", "pem_ctx_launch_count", "pem_ctx_last_sort_passes", "pem_ctx_kernel_ms", "pem_ctx_pool_mallocs", "pem_ctx_size_stalls", "pem_ctx_graph_replays", "pem_ctx_last_step3_kernel", "pem_ctx_pool_bytes", "pem_ctx_trim", "pem_convert_coo", "pem_convert_coo_f32", "pem_tiled_dtype", "pem_result_dtype", "pem_convert_csr", "pem_tiled_transpose",
-    "pem_tiled_info_get", "pem_tiled_values_ready",
+    "pem_tiled_info_get", "pem_tiled_values_ready", "pem_tiled_set_values", "pem_tiled_set_values_f32", "pem_spgemm_numeric",
     "pem_tiled_free", "pem_tiled_get", "pem_tiled_device_ptr", "pem_count_flop", "pem_partition_panels",
     "pem_spgemm", "pem_spgemm_panel", "pem_step1_symbolic", "pem_step2_symbolic", "pem_step3_numeric",
     "pem_result_info_get", "pem_result_free", "pem_result_get", "pem_result_device_ptr",
@@ -133,6 +133,9 @@ def load():
         "pem_tiled_transpose": (C.c_int, [vp, vp, C.POINTER(vp)]),
         "pem_tiled_info_get": (C.c_int, [vp, C.POINTER(TiledInfo)]),
         "pem_tiled_values_ready": (C.c_int, [vp, vp]),
+        "pem_tiled_set_values": (C.c_int, [vp, vp, vp]),
+        "pem_tiled_set_values_f32": (C.c_int, [vp, vp, vp]),
+        "pem_spgemm_numeric": (C.c_int, [vp, vp, vp, vp, C.POINTER(Times)]),
         "pem_tiled_free": (None, [vp, vp]),
         "pem_tiled_get": (C.c_int, [vp, vp, C.c_int, vp, C.c_size_t]),
         "pem_tiled_device_ptr": (vp, [vp, C.c_int]),
@@ -309,6 +312,11 @@ class Context:
         self._check(rc)
         return Result(self, h)
 
+    def spgemm_numeric(self, A: "Tiled", B: "Tiled", Cr: "Result", times: Times | None = None):
+        """Recompute Cr's values in place from the current values of A and B (the handles Cr was computed from),
+        on Cr's structure: step 3 only, the kernel Cr was built with."""
+        self._check(load().pem_spgemm_numeric(self._h, A._h, B._h, Cr._h, C.byref(times) if times is not None else None))
+
     def step1(self, A: "Tiled", B: "Tiled", panel=None) -> "Result":
         h = C.c_void_p()
         rb, re = (0, A.info.tile_rows) if panel is None else panel
@@ -343,10 +351,23 @@ class Tiled:
         i = self.info
         n = {"vals": i.nnz, "tile_nnz_ptr": i.tiles + 1, "masks": i.tiles * 16, "row_ptr": i.tiles * 16,
              "masks_t": i.tiles * 16, "tile_row_ptr": i.tile_rows + 1, "tile_col_idx": i.tiles,
-             "tile_row_idx": i.tiles, "col_occ": i.tiles, "row_occ": i.tiles, "row_col_idx": i.nnz}[name]
+             "tile_row_idx": i.tiles, "col_occ": i.tiles, "row_occ": i.tiles, "row_col_idx": i.nnz,
+             "val_pos": i.nnz}[name]
         out = np.empty(n, dt)
         self.ctx._check(load().pem_tiled_get(self.ctx._h, self._h, idx, _ptr(out), out.nbytes))
         return out
+
+    def set_values(self, V):
+        """New values on the same pattern, in place: V is a numpy array (host) or an integer device pointer, nnz
+        entries in the order of the input this matrix was converted from (for a transpose: its source's input),
+        fp32 or fp64 by the matrix's dtype.  A device V is read in the context's stream order."""
+        f32 = self.dtype == np.float32
+        if V is not None and not isinstance(V, (int, np.integer)):
+            V = np.ascontiguousarray(V, np.float32 if f32 else np.float64)
+            if V.size != self.info.nnz:
+                raise ValueError(f"set_values: {V.size} values for a matrix with {self.info.nnz} nonzeros")
+        fn = load().pem_tiled_set_values_f32 if f32 else load().pem_tiled_set_values
+        self.ctx._check(fn(self.ctx._h, self._h, _ptr(V)))
 
     def values_ready(self):
         """Block until the engine no longer reads the host value array this matrix was converted from."""

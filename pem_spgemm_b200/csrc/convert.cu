@@ -293,6 +293,45 @@ k_col_views(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint16_t* 
     }
 }
 
+// ---- value refresh (pem_tiled_set_values) -----------------------------------------------------------
+// vals[x] = V[pos[x]] and, when the step-3 view exists, the same value into its column-major slot of vals_t (the slot
+// k_col_views computes).  A warp takes 32 consecutive tiles and walks their nonzeros, which are contiguous, one per lane,
+// so the map, the (r, c) bytes and both value arrays move in whole sectors; a lane finds its tile among the warp's 32 in
+// five shuffles over the tiles' first offsets, which the lanes hold in registers.
+template <class T>
+__global__ void __launch_bounds__(256)
+k_refresh_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint32_t* __restrict__ pos,
+               const T* __restrict__ V, const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec,
+               T* __restrict__ vals, T* __restrict__ vals_t)
+{
+    const int64_t t0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32;
+    if (t0 >= cnt) return;                          // whole warps leave together
+    const int lane = threadIdx.x & 31;
+    const int nt = (int)(cnt - t0 < 32 ? cnt - t0 : 32);
+    const uint32_t first = tile_nnz_ptr[t0 + min(lane, nt)];   // lanes >= nt hold the end: above every x
+    const uint32_t s = __shfl_sync(0xffffffffu, first, 0), e = tile_nnz_ptr[t0 + nt];
+    for (uint32_t b = s; b < e; b += 32) {
+        const uint32_t x = b + lane;
+        int j = 0;                                  // last tile of the warp whose first offset is <= x
+        uint32_t ts = s;
+#pragma unroll
+        for (int step = 16; step > 0; step >>= 1) {
+            const uint32_t f = __shfl_sync(0xffffffffu, first, j + step);
+            if (f <= x) { j += step; ts = f; }
+        }
+        if (x < e) {
+            const T v = V[pos[x]];
+            vals[x] = v;
+            if (vals_t) {
+                const unsigned rc = rc_idx[x];
+                const unsigned r = rc >> 4, c = rc & 15u;
+                const uint32_t cr = col_rec[(size_t)(t0 + j) * 16 + c];
+                vals_t[ts + (cr >> 24) + __popc(cr & ((1u << r) - 1u))] = v;
+            }
+        }
+    }
+}
+
 // tile products of one A tile, at tile level (length of B's tile row) and through B's row slices;
 // the smaller of the two is what step 1 will expand.  Summed per tile row.
 __global__ void __launch_bounds__(256)
@@ -336,18 +375,19 @@ k_transpose_counts(const int32_t* __restrict__ perm, const uint32_t* __restrict_
     out[t] = t < cnt ? (int64_t)(nnz_ptr[perm[t] + 1] - nnz_ptr[perm[t]]) : 0;
 }
 
-// thread per tile of the transpose: masks swap roles, values move to their column-major position
+// thread per tile of the transpose: masks swap roles, values (and their value-map entries) move to their column-major
+// position
 template <class T>
 __global__ void __launch_bounds__(128)
 k_transpose_tiles(int cnt, int tile_rows_new, const int32_t* __restrict__ perm, const int64_t* __restrict__ new_ptr,
                   const uint32_t* __restrict__ o_nnz_ptr, const uint16_t* __restrict__ o_masks,
                   const uint16_t* __restrict__ o_masks_t, const int32_t* __restrict__ o_row, const int32_t* __restrict__ o_col,
                   const uint16_t* __restrict__ o_col_occ, const uint16_t* __restrict__ o_row_occ,
-                  const uint8_t* __restrict__ o_rc, const T* __restrict__ o_vals,
+                  const uint8_t* __restrict__ o_rc, const T* __restrict__ o_vals, const uint32_t* __restrict__ o_pos,
                   uint32_t* __restrict__ n_nnz_ptr, uint16_t* __restrict__ n_masks, uint16_t* __restrict__ n_masks_t,
                   uint8_t* __restrict__ n_row_ptr, int32_t* __restrict__ n_row, int32_t* __restrict__ n_col,
                   int32_t* __restrict__ n_tile_row_ptr, uint16_t* __restrict__ n_col_occ, uint16_t* __restrict__ n_row_occ,
-                  uint8_t* __restrict__ n_rc, T* __restrict__ n_vals)
+                  uint8_t* __restrict__ n_rc, T* __restrict__ n_vals, uint32_t* __restrict__ n_pos)
 {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= cnt) return;
@@ -394,6 +434,7 @@ k_transpose_tiles(int cnt, int tile_rows_new, const int32_t* __restrict__ perm, 
         }
         const uint32_t at = ns + first + __popc(m & ((1u << r) - 1u));
         n_vals[at] = o_vals[x];
+        n_pos[at] = o_pos[x];
         n_rc[at] = (uint8_t)((c << 4) | r);
     }
 }
@@ -537,8 +578,7 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
             PEM_LAUNCHED();
             PEM_CK(cudaEventRecord(T->ev_vals, ctx->copy_stream));
             T->vals_pending = true;
-            T->pend_buf[0] = std::exchange(pos_sorted, nullptr);                  // freed once the gather is known to be done
-            T->pend_buf[1] = std::exchange(sV, nullptr);
+            T->pend_buf = std::exchange(sV, nullptr);                             // freed once the gather is known to be done
         } else {
             if (dtype == PEM_F32)
                 k_gather_vals<float><<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(pos_sorted, reinterpret_cast<const float*>(dV), nnz, reinterpret_cast<float*>(T->vals));
@@ -547,7 +587,8 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
             PEM_LAUNCHED();
         }
         pem_free(ctx, pos);
-        pem_free(ctx, pos_sorted);
+        // the sorted positions are the value map: slot x of vals holds V[val_pos[x]] (pem_tiled_set_values)
+        T->val_pos = std::exchange(pos_sorted, nullptr);
         PEM_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, PEM_NSCALARS * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
         PEM_CK(cudaStreamSynchronize(ctx->stream));
         pem_free(ctx, tmp);
@@ -591,7 +632,7 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
         PEM_TRY(pem_alloc(ctx, &T->vals, 0)); PEM_TRY(pem_alloc(ctx, &T->masks, 0)); PEM_TRY(pem_alloc(ctx, &T->masks_t, 0));
         PEM_TRY(pem_alloc(ctx, &T->row_ptr, 0)); PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, 0));
         PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, 0)); PEM_TRY(pem_alloc(ctx, &T->col_occ, 0)); PEM_TRY(pem_alloc(ctx, &T->row_occ, 0));
-        PEM_TRY(pem_alloc(ctx, &T->rc_idx, 0));
+        PEM_TRY(pem_alloc(ctx, &T->rc_idx, 0)); PEM_TRY(pem_alloc(ctx, &T->val_pos, 0));
         T->h_tile_row_ptr.assign((size_t)T->tile_rows + 1, 0);
         PEM_CK(cudaStreamSynchronize(ctx->stream));
     }
@@ -678,7 +719,8 @@ int pem_tiled_wait_vals(pem_ctx* ctx, const pem_tiled* Tc)
     if (!T->vals_pending) return PEM_OK;
     PEM_CK(cudaStreamWaitEvent(ctx->stream, T->ev_vals, 0));
     // the staging buffers go back to the cache in the engine's stream order, i.e. behind the wait above
-    for (void*& b : T->pend_buf) { if (b) pem_free_bytes(ctx, b); b = nullptr; }
+    if (T->pend_buf) pem_free_bytes(ctx, T->pend_buf);
+    T->pend_buf = nullptr;
     T->vals_pending = false;
     return PEM_OK;
 }
@@ -760,7 +802,48 @@ int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* Tc, bool as_a, bool as_
     return PEM_OK;
 }
 
+// new values on an existing pattern, in place (pem_tiled_set_values / _f32)
+static int set_values_any(pem_ctx* ctx, pem_tiled* T, const void* V, int dtype)
+{
+    PEM_RANGE("pem_tiled_set_values");
+    if (!ctx || !T) return PEM_ERR_ARG;
+    if (T->dtype != dtype)
+        return ctx->fail(PEM_ERR_ARG, T->dtype == PEM_F32 ? "fp32 matrix: refresh its values with pem_tiled_set_values_f32"
+                                                          : "fp64 matrix: refresh its values with pem_tiled_set_values");
+    if (T->nnz == 0) return PEM_OK;
+    if (!V) return ctx->fail(PEM_ERR_ARG, "null value array");
+    PEM_CK(cudaSetDevice(ctx->device));
+    PEM_TRY(pem_tiled_wait_vals(ctx, T));           // a gather still running on the copy stream would overwrite the new values
+    const size_t bytes = (size_t)T->nnz * pem_vsize(dtype);
+    char* staged = nullptr;
+    pem_guard g(ctx, staged);
+    const void* dV = V;
+    if (!is_device_ptr(V)) {
+        PEM_TRY(pem_alloc_bytes(ctx, (void**)&staged, bytes));
+        PEM_CK(cudaMemcpyAsync(staged, V, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        PEM_CK(cudaEventRecord(ctx->ev_copy[1], ctx->stream));
+        dV = staged;
+    }
+    if (T->tiles) {
+        if (dtype == PEM_F32)
+            k_refresh_vals<float><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
+                T->tiles, T->tile_nnz_ptr, T->val_pos, static_cast<const float*>(dV), T->rc_idx, T->col_rec,
+                reinterpret_cast<float*>(T->vals), reinterpret_cast<float*>(T->vals_t));
+        else
+            k_refresh_vals<double><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
+                T->tiles, T->tile_nnz_ptr, T->val_pos, static_cast<const double*>(dV), T->rc_idx, T->col_rec, T->vals, T->vals_t);
+        PEM_LAUNCHED();
+    }
+    // default contract, as for conversion: a host V is free again when the call returns (the kernel may still run)
+    if (staged) PEM_CK(cudaEventSynchronize(ctx->ev_copy[1]));
+    return PEM_OK;
+}
+
 extern "C" {
+
+int pem_tiled_set_values(pem_ctx* ctx, pem_tiled* t, const double* V) { return set_values_any(ctx, t, V, PEM_F64); }
+
+int pem_tiled_set_values_f32(pem_ctx* ctx, pem_tiled* t, const float* V) { return set_values_any(ctx, t, V, PEM_F32); }
 
 int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
 {
@@ -784,6 +867,7 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
     PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
     PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
     PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype)))); PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz));
+    PEM_TRY(pem_alloc(ctx, &T->val_pos, (size_t)T->nnz));
     PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
     PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
     PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
@@ -811,13 +895,14 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
     if (A->dtype == PEM_F32)
         k_transpose_tiles<float><<<pem_div_up((int64_t)n, 128), 128, 0, ctx->stream>>>(
             (int)n, T->tile_rows, perm, nptr, A->tile_nnz_ptr, A->masks, A->masks_t, A->tile_row_idx, A->tile_col_idx, A->col_occ,
-            A->row_occ, A->rc_idx, reinterpret_cast<const float*>(A->vals), T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr,
-            T->tile_row_idx, T->tile_col_idx, T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx, reinterpret_cast<float*>(T->vals));
+            A->row_occ, A->rc_idx, reinterpret_cast<const float*>(A->vals), A->val_pos, T->tile_nnz_ptr, T->masks, T->masks_t,
+            T->row_ptr, T->tile_row_idx, T->tile_col_idx, T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx,
+            reinterpret_cast<float*>(T->vals), T->val_pos);
     else
         k_transpose_tiles<double><<<pem_div_up((int64_t)n, 128), 128, 0, ctx->stream>>>(
             (int)n, T->tile_rows, perm, nptr, A->tile_nnz_ptr, A->masks, A->masks_t, A->tile_row_idx, A->tile_col_idx, A->col_occ,
-            A->row_occ, A->rc_idx, A->vals, T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr, T->tile_row_idx, T->tile_col_idx,
-            T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx, T->vals);
+            A->row_occ, A->rc_idx, A->vals, A->val_pos, T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr, T->tile_row_idx,
+            T->tile_col_idx, T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx, T->vals, T->val_pos);
     PEM_LAUNCHED();
     T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
     PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));

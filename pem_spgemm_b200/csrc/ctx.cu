@@ -347,6 +347,7 @@ static const void* tiled_array(const pem_tiled* t, int which, size_t* bytes)
         case PEM_T_COL_OCC: *bytes = n * 2; return t->col_occ;
         case PEM_T_ROW_OCC: *bytes = n * 2; return t->row_occ;
         case PEM_T_ROW_COL_IDX: *bytes = (size_t)t->nnz; return t->rc_idx;
+        case PEM_T_VAL_POS: *bytes = (size_t)t->nnz * 4; return t->val_pos;
     }
     *bytes = 0;
     return nullptr;
@@ -374,7 +375,7 @@ int pem_tiled_get(pem_ctx* ctx, const pem_tiled* t, int which, void* host_dst, s
     if (!ctx || !t || !host_dst) return PEM_ERR_ARG;
     size_t have = 0;
     const void* src = tiled_array(t, which, &have);
-    if (!src && have == 0 && which > PEM_T_ROW_COL_IDX) return ctx->fail(PEM_ERR_ARG, "unknown tiled array");
+    if (!src && have == 0 && which > PEM_T_VAL_POS) return ctx->fail(PEM_ERR_ARG, "unknown tiled array");
     if (bytes != have) return ctx->fail(PEM_ERR_ARG, "pem_tiled_get: size mismatch");
     if (bytes == 0) return PEM_OK;
     if (which == PEM_T_VALS) PEM_TRY(pem_tiled_wait_vals(ctx, t));
@@ -395,7 +396,7 @@ void pem_tiled_free(pem_ctx* ctx, pem_tiled* t)
     pem_free(ctx, t->vals); pem_free(ctx, t->tile_nnz_ptr); pem_free(ctx, t->masks);
     pem_free(ctx, t->masks_t); pem_free(ctx, t->row_ptr); pem_free(ctx, t->tile_row_ptr);
     pem_free(ctx, t->tile_col_idx); pem_free(ctx, t->tile_row_idx); pem_free(ctx, t->col_occ);
-    pem_free(ctx, t->row_occ); pem_free(ctx, t->rc_idx); pem_free(ctx, t->srow_ptr); pem_free(ctx, t->srow_tile);
+    pem_free(ctx, t->row_occ); pem_free(ctx, t->rc_idx); pem_free(ctx, t->val_pos); pem_free(ctx, t->srow_ptr); pem_free(ctx, t->srow_tile);
     pem_free(ctx, t->row_rec); pem_free(ctx, t->col_rec); pem_free(ctx, t->vals_t);
     delete t;
 }

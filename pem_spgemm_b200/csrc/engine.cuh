@@ -26,7 +26,8 @@ enum { PEM_NSCALARS = 24, PEM_NEVENTS = 8, PEM_PLAN_MAX = 96 };
 // Sizes a product read back from the device (tile products, kept pairs, C' tiles, nnz ...), in program order.
 // A repeated product of the same operands replays them instead of stalling the host at every read-back: the
 // kernels still compute every size on the device, the copies are only compared after the product's final sync
-// (a mismatch cannot happen for immutable handles; if it does, the product is redone with the stalls).
+// (a mismatch cannot happen: a handle's pattern is immutable, only its values may be refreshed; if it does, the
+// product is redone with the stalls).
 struct pem_graph;
 struct pem_plan {
     int64_t v[PEM_PLAN_MAX];
@@ -186,7 +187,7 @@ enum { PEM_F64 = 0, PEM_F32 = 1 };
 static inline size_t pem_vsize(int dtype) { return dtype == PEM_F32 ? 4 : 8; }
 
 struct pem_tiled {
-    uint64_t uid = 0;                 // unique per conversion (handles are immutable): key of the size plans
+    uint64_t uid = 0;                 // unique per conversion (the pattern is immutable, the values may be refreshed): key of the size plans
     int dtype = PEM_F64;
     int32_t rows = 0, cols = 0;
     int64_t nnz = 0;
@@ -202,12 +203,13 @@ struct pem_tiled {
     uint16_t* col_occ = nullptr;      // [tiles]
     uint16_t* row_occ = nullptr;      // [tiles]
     uint8_t* rc_idx = nullptr;        // [nnz] (r<<4)|c of every value, tile-major (the reference's *tiles_rowColIdx)
+    uint32_t* val_pos = nullptr;      // [nnz] index of every value slot in the input the handle was built from (pem_tiled_set_values)
     // conversion from host memory: the values' upload and their gather into tile order run on the context's
     // copy stream, BEHIND the call that returns this handle, so the symbolic steps of a product (which read
     // masks only) overlap them; whoever reads `vals` first makes the engine's stream wait (pem_tiled_wait_vals)
     cudaEvent_t ev_vals = nullptr;    // recorded on the copy stream after the gather
     bool vals_pending = false;
-    void* pend_buf[2] = {nullptr, nullptr};   // staging buffers the gather still reads (sorted positions, uploaded values)
+    void* pend_buf = nullptr;         // staging buffer the gather still reads (uploaded values)
     std::vector<int32_t> h_tile_row_ptr;  // host copy of tile_row_ptr: panel calls find their tile range without a device read
     // row slices, built on first use as a B operand of step 1 (pem_tiled_build_srow): for every
     // matrix row s the ids of the tiles that hold a nonzero of row s (in no particular order)
@@ -233,6 +235,8 @@ struct pem_result {
     int stage = 0;                    // 1, 2, 3 = last completed step
     bool s3_entries = false;          // step 3 runs the entry-owner kernel (PEM_OPT_OWNER = 2)
     bool s2_pairs = false;            // step 2 ran the pair kernel (pair_hit may still be null: dense-tile mode, see pem_step2_symbolic)
+    int s3_kernel = 0;                // numeric kernel step 3 ran (pem_ctx_last_step3_kernel's numbering); pem_spgemm_numeric reruns it
+    uint64_t a_uid = 0, b_uid = 0;    // operands of step 1: pem_spgemm_numeric accepts these handles only
     int64_t* row_ptr = nullptr;       // [re-rb+1]
     int32_t* tile_row = nullptr;      // [tiles]
     int32_t* tile_col = nullptr;      // [tiles]
@@ -331,3 +335,4 @@ int pem_step1_esc(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_resu
 int pem_tiled_build_srow(pem_ctx* ctx, const pem_tiled* B);                              // convert.cu
 int pem_tiled_wait_vals(pem_ctx* ctx, const pem_tiled* T);                               // convert.cu
 int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* T, bool as_a, bool as_b);       // convert.cu
+int pem_step3_launch(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C);  // step3.cu: C->s3_kernel on C's buffers

@@ -708,4 +708,44 @@ int pem_spgemm(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result*
     return pem_spgemm_panel(ctx, A, B, 0, A->tile_rows, C, times);
 }
 
+// Step 3 again on a complete result, from the operands' current values: the kernel C's own step 3 ran (the choice
+// PEM_OPT_OWNER made then is baked into C: a dense-tile-mode result has no hit words for any other kernel), on C's
+// buffers, with no size read-back.  A result borrowed from a product graph is fine: the graph does not run while
+// the result is alive.
+int pem_spgemm_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C, pem_times* times)
+{
+    PEM_RANGE("pem_spgemm_numeric");
+    if (!ctx || !A || !B || !C) return PEM_ERR_ARG;
+    if (C->stage != 3) return ctx->fail(PEM_ERR_ARG, "pem_spgemm_numeric needs a complete result (step 3 done)");
+    if (C->a_uid != A->uid || C->b_uid != B->uid)
+        return ctx->fail(PEM_ERR_ARG, "pem_spgemm_numeric: A and B are not the handles the result was computed from");
+    if (A->dtype != C->dtype || B->dtype != C->dtype) return ctx->fail(PEM_ERR_ARG, "operands and result have different value types");
+    PEM_CK(cudaSetDevice(ctx->device));
+    PEM_CK(cudaStreamSynchronize(ctx->stream));
+    auto w0 = std::chrono::high_resolution_clock::now();
+    PEM_TRY(pem_tiled_wait_vals(ctx, A));
+    PEM_TRY(pem_tiled_wait_vals(ctx, B));
+    for (int i = 0; i < KT_N; ++i) { ctx->kt_seen[i] = false; ctx->kt_ms[i] = 0.0; }
+    PEM_CK(pem_event_record(ctx, ctx->ev[4]));
+    PEM_TRY(pem_step3_launch(ctx, A, B, C));
+    PEM_CK(pem_event_record(ctx, ctx->ev[5]));
+    PEM_CK(cudaStreamSynchronize(ctx->stream));
+    ctx->last_step3_kernel = C->s3_kernel;
+    auto w1 = std::chrono::high_resolution_clock::now();
+    float ms = 0.f;
+    if (ctx->kt_seen[KT_NUMERIC] && cudaEventElapsedTime(&ms, ctx->kev[2 * KT_NUMERIC], ctx->kev[2 * KT_NUMERIC + 1]) == cudaSuccess)
+        ctx->kt_ms[KT_NUMERIC] = ms;
+    else
+        (void)cudaGetLastError();
+    if (times) {
+        float s3 = 0.f;
+        if (cudaEventElapsedTime(&s3, ctx->ev[4], ctx->ev[5]) != cudaSuccess) { s3 = 0.f; (void)cudaGetLastError(); }
+        times->step1_ms = 0; times->step2_ms = 0; times->step3_ms = s3;
+        times->kernel_ms = s3;
+        times->total_ms = std::chrono::duration<double, std::milli>(w1 - w0).count();
+        times->malloc_ms = times->total_ms - times->kernel_ms;
+    }
+    return PEM_OK;
+}
+
 }  // extern "C"

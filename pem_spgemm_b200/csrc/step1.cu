@@ -616,6 +616,7 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     auto result_free = [ctx](pem_result* r) { pem_result_free(ctx, r); };
     std::unique_ptr<pem_result, decltype(result_free)> C(new pem_result(), result_free);
     C->dtype = A->dtype;
+    C->a_uid = A->uid; C->b_uid = B->uid;
     C->rb = rb; C->re = re; C->rows = A->rows; C->cols = B->cols; C->tile_cols = B->tile_cols;
     const int nrows = re - rb;
     ctx->last_sort_passes = -1;

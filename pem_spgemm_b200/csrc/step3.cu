@@ -689,7 +689,19 @@ extern "C" int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_til
         k_block_tiles<<<pem_div_up(C->tiles, 256), 256, 0, ctx->stream>>>(C->tiles, C->tile_nnz_ptr, C->blk_tile);
         PEM_LAUNCHED();
     }
-    ctx->last_step3_kernel = windows ? 4 : !by_records ? 1 : C->s3_entries ? 2 : 3;
+    C->s3_kernel = windows ? 4 : !by_records ? 1 : C->s3_entries ? 2 : 3;
+    ctx->last_step3_kernel = C->s3_kernel;
+    PEM_TRY(pem_step3_launch(ctx, A, B, C));
+    C->stage = 3;
+    return PEM_OK;
+}
+
+// The numeric kernel C->s3_kernel on C's existing buffers: C->vals, the views of A and B, and what that kernel reads
+// besides (blk_tile for the entry-owner kernel, row_col_idx for the tile-class kernel) are in place.
+int pem_step3_launch(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C)
+{
+    const bool windows = C->s3_kernel == 4, by_records = C->s2_pairs;
+    const int64_t nblk_e = (C->nnz + S3E_ENTRIES - 1) / S3E_ENTRIES;
     if (C->nnz > 0 && windows) {
         // 128-pair windows, 144 staged pairs, 1024 nonzeros per decode pass: 26 KB of shared memory and 32 registers, so
         // that eight blocks (64 warps) stay resident per SM: the kernel is bound by the latency of its value gathers, and
@@ -700,7 +712,6 @@ extern "C" int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_til
         else
             PEM_TRY(C->dtype == PEM_F32 ? (launch_windows<float, 128, 144, 1024, 8, false>(ctx, A, B, C))
                                         : (launch_windows<double, 128, 144, 1024, 8, false>(ctx, A, B, C)));
-        C->stage = 3;
         return PEM_OK;
     }
     KT_BEGIN(KT_NUMERIC);
@@ -733,6 +744,5 @@ extern "C" int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_til
         PEM_LAUNCHED();
     }
     KT_END(KT_NUMERIC);
-    C->stage = 3;
     return PEM_OK;
 }
