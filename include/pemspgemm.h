@@ -294,6 +294,28 @@ int pem_step3_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_
  * times (may be NULL) gets step3_ms, kernel_ms, total_ms and malloc_ms, with steps 1 and 2 at 0. */
 int pem_spgemm_numeric(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C, pem_times* times);
 
+/* ---- results as operands ---------------------------------------------------------------- */
+/* A complete result C (or panel of C) as a new, independent tiled matrix: the next product of a chain (AMG's
+ * P^T*(A*P), matrix powers, Markov clustering) without exporting C and converting it again.  Every array and
+ * pem_tiled_info are identical to what pem_convert_coo builds from pem_result_to_coo(C)'s output (same dtype), so
+ * the value map (PEM_T_VAL_POS) is the position of each value in C's sorted COO / CSR order, the order
+ * pem_tiled_set_values then takes.  Empty C' tiles (PEM_OPT_KEEP_EMPTY_TILES) are dropped; explicit zeros of C stay.
+ * A panel [tile_row_begin, tile_row_end) becomes a matrix of C's full shape whose tile rows outside the panel are
+ * empty, so a panel product of it is the panel of the chained product.  The handle shares no memory with C: C may
+ * be freed right after the call (a result borrowed from a product graph too, whose graph may then run again).  It
+ * has an identity of its own for size plans and graphs.  PEM_ERR_ARG for a result before step 3, PEM_ERR_LIMIT for
+ * nnz >= 2^32-1 or 2^31-1 tiles and more (as pem_convert_coo), both before anything is allocated.  Ends with one
+ * synchronisation; a result made under PEM_OPT_KEEP_EMPTY_TILES = 1 adds one size read-back. */
+int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out);
+/* Writes the current values of C into a matrix t built by pem_result_to_tiled, in place, e.g. after
+ * pem_spgemm_numeric recomputed C.  C must be a complete result of the same product and panel as the one t was
+ * built from (the same A and B handles: C's structure depends on these alone), e.g. a later result of that product
+ * handed out by its graph; PEM_ERR_ARG otherwise, and for a matrix not built by pem_result_to_tiled (a converted one,
+ * or the pem_tiled_transpose of a built one: refresh those with pem_tiled_set_values).  As with pem_tiled_set_values,
+ * device pointers of t (its values and, if built, their column-major view), size plans and product graphs stay
+ * valid.  Stream-ordered on the context's stream: no allocation, no host wait. */
+int pem_tiled_refresh_from_result(pem_ctx* ctx, pem_tiled* t, const pem_result* C);
+
 int pem_result_info_get(const pem_result* C, pem_result_info* info);
 void pem_result_free(pem_ctx* ctx, pem_result* C);
 

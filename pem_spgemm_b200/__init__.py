@@ -84,6 +84,7 @@ EXPORTS = [
     "pem_tiled_info_get", "pem_tiled_values_ready", "pem_tiled_set_values", "pem_tiled_set_values_f32", "pem_spgemm_numeric",
     "pem_tiled_free", "pem_tiled_get", "pem_tiled_device_ptr", "pem_count_flop", "pem_partition_panels",
     "pem_spgemm", "pem_spgemm_panel", "pem_step1_symbolic", "pem_step2_symbolic", "pem_step3_numeric",
+    "pem_result_to_tiled", "pem_tiled_refresh_from_result",
     "pem_result_info_get", "pem_result_free", "pem_result_get", "pem_result_device_ptr",
     "pem_result_to_coo", "pem_result_to_coo_f32", "pem_result_to_csr", "pem_result_to_coo_device", "pem_result_checksum", "pem_mtx_read", "pem_mtx_write",
     "pem_free_host", "pem_write_lines_i32", "pem_write_lines_f64",
@@ -146,6 +147,8 @@ def load():
         "pem_step1_symbolic": (C.c_int, [vp, vp, vp, i32, i32, C.POINTER(vp)]),
         "pem_step2_symbolic": (C.c_int, [vp, vp, vp, vp]),
         "pem_step3_numeric": (C.c_int, [vp, vp, vp, vp]),
+        "pem_result_to_tiled": (C.c_int, [vp, vp, C.POINTER(vp)]),
+        "pem_tiled_refresh_from_result": (C.c_int, [vp, vp, vp]),
         "pem_result_info_get": (C.c_int, [vp, C.POINTER(ResultInfo)]),
         "pem_result_free": (None, [vp, vp]),
         "pem_result_get": (C.c_int, [vp, vp, C.c_int, vp, C.c_size_t]),
@@ -369,6 +372,11 @@ class Tiled:
         fn = load().pem_tiled_set_values_f32 if f32 else load().pem_tiled_set_values
         self.ctx._check(fn(self.ctx._h, self._h, _ptr(V)))
 
+    def refresh_from(self, result: "Result"):
+        """Write ``result``'s current values into this matrix in place; it must have been built by
+        ``Result.to_tiled`` from a result of the same product and panel (e.g. after ``Context.spgemm_numeric``)."""
+        self.ctx._check(load().pem_tiled_refresh_from_result(self.ctx._h, self._h, result._h))
+
     def values_ready(self):
         """Block until the engine no longer reads the host value array this matrix was converted from."""
         self.ctx._check(load().pem_tiled_values_ready(self.ctx._h, self._h))
@@ -436,6 +444,13 @@ class Result:
         self.ctx._check(load().pem_result_to_coo_device(self.ctx._h, self._h, C.c_void_p(rows_ptr or None),
                                                         C.c_void_p(cols_ptr or None), C.c_void_p(vals_ptr or None),
                                                         C.c_void_p(row_ptr_ptr or None)))
+
+    def to_tiled(self) -> Tiled:
+        """This result as a new, independent tiled matrix (the next operand of a chain of products): the arrays
+        ``convert_coo(*self.to_coo())`` would build, C's full shape for a panel.  The result may be freed after."""
+        h = C.c_void_p()
+        self.ctx._check(load().pem_result_to_tiled(self.ctx._h, self._h, C.byref(h)))
+        return Tiled(self.ctx, h)
 
     def checksum(self):
         s, a = C.c_double(), C.c_double()

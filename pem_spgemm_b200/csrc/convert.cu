@@ -297,16 +297,18 @@ k_col_views(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint16_t* 
 // vals[x] = V[pos[x]] and, when the step-3 view exists, the same value into its column-major slot of vals_t (the slot
 // k_col_views computes).  A warp takes 32 consecutive tiles and walks their nonzeros, which are contiguous, one per lane,
 // so the map, the (r, c) bytes and both value arrays move in whole sectors; a lane finds its tile among the warp's 32 in
-// five shuffles over the tiles' first offsets, which the lanes hold in registers.
-template <class T>
-__global__ void __launch_bounds__(256)
-k_refresh_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint32_t* __restrict__ pos,
-               const T* __restrict__ V, const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec,
-               T* __restrict__ vals, T* __restrict__ vals_t)
+// five shuffles over the tiles' first offsets, which the lanes hold in registers.  MAPPED = false reads V in slot order
+// (V[x], no map): pem_tiled_refresh_from_result, whose source result holds its values in the handle's slots.  The
+// thread indices are read in the kernels, where their launch bounds limit them.
+template <class T, bool MAPPED>
+__device__ __forceinline__ void
+refresh_vals(int64_t gid, unsigned tid, int cnt, const uint32_t* __restrict__ tile_nnz_ptr,
+             const uint32_t* __restrict__ pos, const T* __restrict__ V, const uint8_t* __restrict__ rc_idx,
+             const uint32_t* __restrict__ col_rec, T* __restrict__ vals, T* __restrict__ vals_t)
 {
-    const int64_t t0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32;
+    const int64_t t0 = (gid >> 5) * 32;
     if (t0 >= cnt) return;                          // whole warps leave together
-    const int lane = threadIdx.x & 31;
+    const int lane = tid & 31;
     const int nt = (int)(cnt - t0 < 32 ? cnt - t0 : 32);
     const uint32_t first = tile_nnz_ptr[t0 + min(lane, nt)];   // lanes >= nt hold the end: above every x
     const uint32_t s = __shfl_sync(0xffffffffu, first, 0), e = tile_nnz_ptr[t0 + nt];
@@ -320,7 +322,7 @@ k_refresh_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint32_
             if (f <= x) { j += step; ts = f; }
         }
         if (x < e) {
-            const T v = V[pos[x]];
+            const T v = MAPPED ? V[pos[x]] : V[x];
             vals[x] = v;
             if (vals_t) {
                 const unsigned rc = rc_idx[x];
@@ -330,6 +332,24 @@ k_refresh_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint32_
             }
         }
     }
+}
+template <class T>
+__global__ void __launch_bounds__(256)
+k_refresh_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint32_t* __restrict__ pos,
+               const T* __restrict__ V, const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec,
+               T* __restrict__ vals, T* __restrict__ vals_t)
+{
+    refresh_vals<T, true>((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, pos, V, rc_idx,
+                          col_rec, vals, vals_t);
+}
+template <class T>
+__global__ void __launch_bounds__(256)
+k_refresh_slots(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const T* __restrict__ V,
+                const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec, T* __restrict__ vals,
+                T* __restrict__ vals_t)
+{
+    refresh_vals<T, false>((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, nullptr, V,
+                           rc_idx, col_rec, vals, vals_t);
 }
 
 // tile products of one A tile, at tile level (length of B's tile row) and through B's row slices;
@@ -836,6 +856,26 @@ static int set_values_any(pem_ctx* ctx, pem_tiled* T, const void* V, int dtype)
     }
     // default contract, as for conversion: a host V is free again when the call returns (the kernel may still run)
     if (staged) PEM_CK(cudaEventSynchronize(ctx->ev_copy[1]));
+    return PEM_OK;
+}
+
+// new values already in T's slot order (device array of T->nnz values of T's dtype), in place: a copy into vals, or,
+// when the column-major view exists, one pass that writes vals and vals_t
+int pem_tiled_write_slots(pem_ctx* ctx, pem_tiled* T, const void* dV)
+{
+    if (T->nnz == 0) return PEM_OK;
+    if (!T->vals_t) {
+        PEM_CK(cudaMemcpyAsync(T->vals, dV, (size_t)T->nnz * pem_vsize(T->dtype), cudaMemcpyDeviceToDevice, ctx->stream));
+        return PEM_OK;
+    }
+    if (T->dtype == PEM_F32)
+        k_refresh_slots<float><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
+            T->tiles, T->tile_nnz_ptr, static_cast<const float*>(dV), T->rc_idx, T->col_rec, reinterpret_cast<float*>(T->vals),
+            reinterpret_cast<float*>(T->vals_t));
+    else
+        k_refresh_slots<double><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
+            T->tiles, T->tile_nnz_ptr, static_cast<const double*>(dV), T->rc_idx, T->col_rec, T->vals, T->vals_t);
+    PEM_LAUNCHED();
     return PEM_OK;
 }
 

@@ -221,6 +221,10 @@ struct pem_tiled {
     uint32_t* row_rec = nullptr;      // [tiles*16]  masks[i]   | row_ptr[i] << 16          (operand A)
     uint32_t* col_rec = nullptr;      // [tiles*16]  masks_t[i] | first value of column << 24 (operand B)
     double* vals_t = nullptr;         // [nnz] tile-major, column-major inside a tile        (operand B)
+    // built by pem_result_to_tiled: the product (and panel) the result came from, whose structure this handle holds;
+    // pem_tiled_refresh_from_result accepts results of that product only.  src_a_uid == 0: not built from a result
+    uint64_t src_a_uid = 0, src_b_uid = 0;
+    int32_t src_rb = 0, src_re = 0;
 };
 
 // ---------------------------------------------------------------------------------------
@@ -237,6 +241,7 @@ struct pem_result {
     bool s2_pairs = false;            // step 2 ran the pair kernel (pair_hit may still be null: dense-tile mode, see pem_step2_symbolic)
     int s3_kernel = 0;                // numeric kernel step 3 ran (pem_ctx_last_step3_kernel's numbering); pem_spgemm_numeric reruns it
     uint64_t a_uid = 0, b_uid = 0;    // operands of step 1: pem_spgemm_numeric accepts these handles only
+    bool keep_empty = false;          // step 1 ran under PEM_OPT_KEEP_EMPTY_TILES: C' may hold tiles with no nonzero
     int64_t* row_ptr = nullptr;       // [re-rb+1]
     int32_t* tile_row = nullptr;      // [tiles]
     int32_t* tile_col = nullptr;      // [tiles]
@@ -335,4 +340,5 @@ int pem_step1_esc(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_resu
 int pem_tiled_build_srow(pem_ctx* ctx, const pem_tiled* B);                              // convert.cu
 int pem_tiled_wait_vals(pem_ctx* ctx, const pem_tiled* T);                               // convert.cu
 int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* T, bool as_a, bool as_b);       // convert.cu
+int pem_tiled_write_slots(pem_ctx* ctx, pem_tiled* T, const void* dV);                   // convert.cu: V in T's slot order
 int pem_step3_launch(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C);  // step3.cu: C->s3_kernel on C's buffers

@@ -617,6 +617,7 @@ extern "C" int pem_step1_symbolic(pem_ctx* ctx, const pem_tiled* A, const pem_ti
     std::unique_ptr<pem_result, decltype(result_free)> C(new pem_result(), result_free);
     C->dtype = A->dtype;
     C->a_uid = A->uid; C->b_uid = B->uid;
+    C->keep_empty = ctx->opt_keep_empty != 0;
     C->rb = rb; C->re = re; C->rows = A->rows; C->cols = B->cols; C->tile_cols = B->tile_cols;
     const int nrows = re - rb;
     ctx->last_sort_passes = -1;
