@@ -316,6 +316,35 @@ int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out);
  * valid.  Stream-ordered on the context's stream: no allocation, no host wait. */
 int pem_tiled_refresh_from_result(pem_ctx* ctx, pem_tiled* t, const pem_result* C);
 
+/* ---- sums ------------------------------------------------------------------------------- */
+/* S = alpha*A + beta*B as a new, independent tiled matrix (smoothed-aggregation prolongators P0 - w*(D^-1 A)*P0,
+ * shifted operators A - s*I, A + A^T, graph Laplacians D - A), built on the device from the operands' tiles.
+ *   Pattern: the union of the patterns of A and B.  Nothing is dropped: entries that cancel stay as explicit zeros,
+ *     alpha = 0 or beta = 0 keeps the entries too, and explicit zeros of the operands stay.
+ *   Values, exactly: an entry of both operands is fl(fl(alpha*a) + fl(beta*b)); an entry of A only is fl(alpha*a), one
+ *     of B only fl(beta*b).  An absent entry is not a zero, so -0 and 0*Inf = NaN come out as IEEE says.  There is no
+ *     fused multiply-add (e.g. alpha = 0.1, a = 10, beta = -1, b = 1 gives +0.0, where a fused form gives 2^-54 in
+ *     fp64 and 2^-26 in fp32).  For fp32 operands alpha and beta are first rounded to float.
+ *   The handle: every array and pem_tiled_info are identical to what pem_convert_coo builds from S's COO sorted by
+ *     (row, col), in the operands' dtype; so the value map (PEM_T_VAL_POS) is each value's position in S's row-major
+ *     order, the order pem_tiled_set_values then takes.  S shares no memory with A or B, which may be freed right after
+ *     the call, and has an identity of its own for size plans and graphs.
+ *   Operands: A and B may be the same handle, a pem_tiled_transpose, a pem_result_to_tiled handle or another sum.  An
+ *     operand whose values are still uploading (PEM_OPT_ASYNC_VALUES) is waited for.
+ *   Refusals: PEM_ERR_ARG for null handles, different shapes or different dtypes, before anything is allocated;
+ *     PEM_ERR_LIMIT when the union holds 2^32-1 nonzeros or 2^31-1 tiles or more (as pem_convert_coo), after the size
+ *     read-back, with nothing left allocated.
+ *   Host waits: two size read-backs (the union's tiles, then its nnz) and one final synchronisation; a setup call, like
+ *     a conversion. */
+int pem_tiled_add(pem_ctx* ctx, double alpha, const pem_tiled* A, double beta, const pem_tiled* B, pem_tiled** out);
+/* Rewrites the values of a sum S in place from the current values of A and B, with alpha and beta that may differ
+ * from the build's: bit-identical to a new pem_tiled_add of the same values.  S must have been built by pem_tiled_add
+ * from these two handles in this order; PEM_ERR_ARG otherwise: swapped operands, other handles, a matrix not built by
+ * pem_tiled_add (a converted or pem_result_to_tiled one) and the pem_tiled_transpose of a sum.  S's device pointers
+ * (its values and, if built, their column-major view), size plans and product graphs that read S stay valid.  No
+ * allocation, no host wait: stream-ordered on the context's stream, after any pending upload of A or B. */
+int pem_tiled_add_values(pem_ctx* ctx, pem_tiled* S, double alpha, const pem_tiled* A, double beta, const pem_tiled* B);
+
 int pem_result_info_get(const pem_result* C, pem_result_info* info);
 void pem_result_free(pem_ctx* ctx, pem_result* C);
 

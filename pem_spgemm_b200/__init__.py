@@ -84,7 +84,7 @@ EXPORTS = [
     "pem_tiled_info_get", "pem_tiled_values_ready", "pem_tiled_set_values", "pem_tiled_set_values_f32", "pem_spgemm_numeric",
     "pem_tiled_free", "pem_tiled_get", "pem_tiled_device_ptr", "pem_count_flop", "pem_partition_panels",
     "pem_spgemm", "pem_spgemm_panel", "pem_step1_symbolic", "pem_step2_symbolic", "pem_step3_numeric",
-    "pem_result_to_tiled", "pem_tiled_refresh_from_result",
+    "pem_result_to_tiled", "pem_tiled_refresh_from_result", "pem_tiled_add", "pem_tiled_add_values",
     "pem_result_info_get", "pem_result_free", "pem_result_get", "pem_result_device_ptr",
     "pem_result_to_coo", "pem_result_to_coo_f32", "pem_result_to_csr", "pem_result_to_coo_device", "pem_result_checksum", "pem_mtx_read", "pem_mtx_write",
     "pem_free_host", "pem_write_lines_i32", "pem_write_lines_f64",
@@ -149,6 +149,8 @@ def load():
         "pem_step3_numeric": (C.c_int, [vp, vp, vp, vp]),
         "pem_result_to_tiled": (C.c_int, [vp, vp, C.POINTER(vp)]),
         "pem_tiled_refresh_from_result": (C.c_int, [vp, vp, vp]),
+        "pem_tiled_add": (C.c_int, [vp, C.c_double, vp, C.c_double, vp, C.POINTER(vp)]),
+        "pem_tiled_add_values": (C.c_int, [vp, vp, C.c_double, vp, C.c_double, vp]),
         "pem_result_info_get": (C.c_int, [vp, C.POINTER(ResultInfo)]),
         "pem_result_free": (None, [vp, vp]),
         "pem_result_get": (C.c_int, [vp, vp, C.c_int, vp, C.c_size_t]),
@@ -303,6 +305,19 @@ class Context:
         b = np.zeros(nparts + 1, np.int32)
         self._check(load().pem_partition_panels(self._h, A._h, B._h, nparts, _ptr(b)))
         return b
+
+    # -- sums -----------------------------------------------------------------------------
+    def add(self, A: "Tiled", B: "Tiled", alpha: float = 1.0, beta: float = 1.0) -> "Tiled":
+        """S = alpha*A + beta*B as a new tiled matrix on the union of the patterns (nothing dropped, no fused
+        multiply-add); A and B may be freed after."""
+        h = C.c_void_p()
+        self._check(load().pem_tiled_add(self._h, float(alpha), A._h, float(beta), B._h, C.byref(h)))
+        return Tiled(self, h)
+
+    def add_values(self, S: "Tiled", A: "Tiled", B: "Tiled", alpha: float = 1.0, beta: float = 1.0):
+        """Recompute S = alpha*A + beta*B in place from the current values of A and B, the handles S was built from by
+        ``add``, in that order."""
+        self._check(load().pem_tiled_add_values(self._h, S._h, float(alpha), A._h, float(beta), B._h))
 
     # -- SpGEMM ---------------------------------------------------------------------------
     def spgemm(self, A: "Tiled", B: "Tiled", times: Times | None = None, panel=None) -> "Result":

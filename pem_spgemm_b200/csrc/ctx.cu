@@ -398,6 +398,7 @@ void pem_tiled_free(pem_ctx* ctx, pem_tiled* t)
     pem_free(ctx, t->tile_col_idx); pem_free(ctx, t->tile_row_idx); pem_free(ctx, t->col_occ);
     pem_free(ctx, t->row_occ); pem_free(ctx, t->rc_idx); pem_free(ctx, t->val_pos); pem_free(ctx, t->srow_ptr); pem_free(ctx, t->srow_tile);
     pem_free(ctx, t->row_rec); pem_free(ctx, t->col_rec); pem_free(ctx, t->vals_t);
+    pem_free(ctx, t->add_src);
     delete t;
 }
 

@@ -225,6 +225,10 @@ struct pem_tiled {
     // pem_tiled_refresh_from_result accepts results of that product only.  src_a_uid == 0: not built from a result
     uint64_t src_a_uid = 0, src_b_uid = 0;
     int32_t src_rb = 0, src_re = 0;
+    // built by pem_tiled_add: the operands S = alpha*A + beta*B was built from (pem_tiled_add_values accepts these, in
+    // this order) and, per tile of S, the tile of A and of B it holds (-1: none).  add_a_uid == 0: not a sum
+    uint64_t add_a_uid = 0, add_b_uid = 0;
+    int2* add_src = nullptr;          // [tiles]
 };
 
 // ---------------------------------------------------------------------------------------
@@ -341,4 +345,5 @@ int pem_tiled_build_srow(pem_ctx* ctx, const pem_tiled* B);                     
 int pem_tiled_wait_vals(pem_ctx* ctx, const pem_tiled* T);                               // convert.cu
 int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* T, bool as_a, bool as_b);       // convert.cu
 int pem_tiled_write_slots(pem_ctx* ctx, pem_tiled* T, const void* dV);                   // convert.cu: V in T's slot order
+int pem_operand_structure(pem_ctx* ctx, const pem_result* C, const int32_t* keep, pem_tiled* T);  // operand.cu
 int pem_step3_launch(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C);  // step3.cu: C->s3_kernel on C's buffers

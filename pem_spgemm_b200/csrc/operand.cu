@@ -120,6 +120,42 @@ k_operand_slots(int n_tile_rows, const int64_t* __restrict__ c_row_ptr, const ui
 
 }  // namespace
 
+// The structure of T from a result-shaped tile list C (tile-row pointer over [rb, re), tile rows and columns, row masks,
+// value offsets): the arrays of T, T->vals included, allocated for T->tiles tiles (C' tile keep[i] for tile i, or tile i
+// when keep is null) and T->nnz values, and every array but vals written.  T's shape is set by the caller.  Stream order;
+// the caller fills vals, copies h_tile_row_ptr and synchronises.  pem_result_to_tiled and pem_tiled_add (sum.cu).
+int pem_operand_structure(pem_ctx* ctx, const pem_result* C, const int32_t* keep, pem_tiled* T)
+{
+    const int ntr = C->re - C->rb;
+    const int64_t cnt = T->tiles;
+    const size_t n = (size_t)cnt;
+    int64_t* row_pos = nullptr;
+    pem_guard g(ctx, row_pos);
+    PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype))));
+    PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz)); PEM_TRY(pem_alloc(ctx, &T->val_pos, (size_t)T->nnz));
+    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
+    PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
+    PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
+    PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
+    PEM_TRY(pem_alloc(ctx, &T->col_occ, n)); PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
+
+    const int64_t threads = std::max<int64_t>(cnt, T->tile_rows) + 1;
+    k_operand_tiles<<<pem_div_up(threads, 128), 128, 0, ctx->stream>>>(
+        (int)cnt, keep, C->masks, C->tile_row, C->tile_col, C->tile_nnz_ptr, (uint32_t)C->nnz, C->rb, C->re, T->tile_rows,
+        T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr, T->tile_row_idx, T->tile_col_idx, T->tile_row_ptr, T->col_occ,
+        T->row_occ);
+    PEM_LAUNCHED();
+    if (T->nnz) {
+        // first position of every row of the panel in C's row-major order: the export's row count and scan
+        PEM_TRY(pem_alloc(ctx, &row_pos, (size_t)ntr * 16 + 1));
+        PEM_TRY(pem_result_to_coo_device(ctx, C, nullptr, nullptr, nullptr, row_pos));
+        k_operand_slots<<<pem_div_up((int64_t)ntr * 16, 256), 256, 0, ctx->stream>>>(
+            ntr, C->row_ptr, C->masks, C->tile_nnz_ptr, row_pos, T->rc_idx, T->val_pos);
+        PEM_LAUNCHED();
+    }
+    return PEM_OK;
+}
+
 extern "C" {
 
 int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out)
@@ -139,11 +175,9 @@ int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out)
     T->tile_rows = (int32_t)(((int64_t)C->rows + PEM_TILE - 1) / PEM_TILE);
     T->tile_cols = C->tile_cols;
     T->src_a_uid = C->a_uid; T->src_b_uid = C->b_uid; T->src_rb = C->rb; T->src_re = C->re;
-    const int ntr = C->re - C->rb;
     int32_t* keep = nullptr;                  // kept C' tile of every tile of T (keep-empty results only)
-    int64_t* row_pos = nullptr;
     char* tmp = nullptr;
-    pem_guard g(ctx, keep, row_pos, tmp);
+    pem_guard g(ctx, keep, tmp);
 
     // a result of the default mode holds non-empty tiles only; otherwise the empty ones are dropped here (one read-back)
     int64_t cnt = C->tiles;
@@ -163,31 +197,9 @@ int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out)
         pem_free(ctx, tmp);
     }
     T->tiles = (int32_t)cnt;
-    const size_t n = (size_t)cnt;
-    PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype))));
-    PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz)); PEM_TRY(pem_alloc(ctx, &T->val_pos, (size_t)T->nnz));
-    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
-    PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
-    PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
-    PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
-    PEM_TRY(pem_alloc(ctx, &T->col_occ, n)); PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
-
+    PEM_TRY(pem_operand_structure(ctx, C, keep, T.get()));
     // every value keeps its slot: empty tiles hold none
     if (T->nnz) PEM_CK(cudaMemcpyAsync(T->vals, C->vals, (size_t)T->nnz * pem_vsize(T->dtype), cudaMemcpyDeviceToDevice, ctx->stream));
-    const int64_t threads = std::max<int64_t>(cnt, T->tile_rows) + 1;
-    k_operand_tiles<<<pem_div_up(threads, 128), 128, 0, ctx->stream>>>(
-        (int)cnt, keep, C->masks, C->tile_row, C->tile_col, C->tile_nnz_ptr, (uint32_t)C->nnz, C->rb, C->re, T->tile_rows,
-        T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr, T->tile_row_idx, T->tile_col_idx, T->tile_row_ptr, T->col_occ,
-        T->row_occ);
-    PEM_LAUNCHED();
-    if (T->nnz) {
-        // first position of every row of the panel in C's row-major order: the export's row count and scan
-        PEM_TRY(pem_alloc(ctx, &row_pos, (size_t)ntr * 16 + 1));
-        PEM_TRY(pem_result_to_coo_device(ctx, C, nullptr, nullptr, nullptr, row_pos));
-        k_operand_slots<<<pem_div_up((int64_t)ntr * 16, 256), 256, 0, ctx->stream>>>(
-            ntr, C->row_ptr, C->masks, C->tile_nnz_ptr, row_pos, T->rc_idx, T->val_pos);
-        PEM_LAUNCHED();
-    }
     T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
     PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
     PEM_CK(cudaStreamSynchronize(ctx->stream));
