@@ -289,67 +289,30 @@ k_col_views(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint16_t* 
         const unsigned rc = rc_idx[x];
         const unsigned r = rc >> 4, c = rc & 15u;
         const unsigned cr = my[c];
-        vals_t[s + (cr >> 24) + __popc(cr & ((1u << r) - 1u))] = vals[x];
+        vals_t[pem_col_slot(s, cr, r)] = vals[x];
     }
 }
 
 // ---- value refresh (pem_tiled_set_values) -----------------------------------------------------------
-// vals[x] = V[pos[x]] and, when the step-3 view exists, the same value into its column-major slot of vals_t (the slot
-// k_col_views computes).  A warp takes 32 consecutive tiles and walks their nonzeros, which are contiguous, one per lane,
-// so the map, the (r, c) bytes and both value arrays move in whole sectors; a lane finds its tile among the warp's 32 in
-// five shuffles over the tiles' first offsets, which the lanes hold in registers.  MAPPED = false reads V in slot order
-// (V[x], no map): pem_tiled_refresh_from_result, whose source result holds its values in the handle's slots.  The
-// thread indices are read in the kernels, where their launch bounds limit them.
-template <class T, bool MAPPED>
-__device__ __forceinline__ void
-refresh_vals(int64_t gid, unsigned tid, int cnt, const uint32_t* __restrict__ tile_nnz_ptr,
-             const uint32_t* __restrict__ pos, const T* __restrict__ V, const uint8_t* __restrict__ rc_idx,
-             const uint32_t* __restrict__ col_rec, T* __restrict__ vals, T* __restrict__ vals_t)
-{
-    const int64_t t0 = (gid >> 5) * 32;
-    if (t0 >= cnt) return;                          // whole warps leave together
-    const int lane = tid & 31;
-    const int nt = (int)(cnt - t0 < 32 ? cnt - t0 : 32);
-    const uint32_t first = tile_nnz_ptr[t0 + min(lane, nt)];   // lanes >= nt hold the end: above every x
-    const uint32_t s = __shfl_sync(0xffffffffu, first, 0), e = tile_nnz_ptr[t0 + nt];
-    for (uint32_t b = s; b < e; b += 32) {
-        const uint32_t x = b + lane;
-        int j = 0;                                  // last tile of the warp whose first offset is <= x
-        uint32_t ts = s;
-#pragma unroll
-        for (int step = 16; step > 0; step >>= 1) {
-            const uint32_t f = __shfl_sync(0xffffffffu, first, j + step);
-            if (f <= x) { j += step; ts = f; }
-        }
-        if (x < e) {
-            const T v = MAPPED ? V[pos[x]] : V[x];
-            vals[x] = v;
-            if (vals_t) {
-                const unsigned rc = rc_idx[x];
-                const unsigned r = rc >> 4, c = rc & 15u;
-                const uint32_t cr = col_rec[(size_t)(t0 + j) * 16 + c];
-                vals_t[ts + (cr >> 24) + __popc(cr & ((1u << r) - 1u))] = v;
-            }
-        }
-    }
-}
+// vals[x] = V[pos[x]], and the same value into vals_t when the step-3 view exists (pem_write_slots)
 template <class T>
 __global__ void __launch_bounds__(256)
 k_refresh_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint32_t* __restrict__ pos,
                const T* __restrict__ V, const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec,
                T* __restrict__ vals, T* __restrict__ vals_t)
 {
-    refresh_vals<T, true>((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, pos, V, rc_idx,
-                          col_rec, vals, vals_t);
+    pem_write_slots((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, rc_idx, col_rec, vals,
+                    vals_t, [=](uint32_t x, int64_t) { return V[pos[x]]; });
 }
+// V in slot order, no map: pem_tiled_refresh_from_result, whose source result holds its values in the handle's slots
 template <class T>
 __global__ void __launch_bounds__(256)
 k_refresh_slots(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const T* __restrict__ V,
                 const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec, T* __restrict__ vals,
                 T* __restrict__ vals_t)
 {
-    refresh_vals<T, false>((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, nullptr, V,
-                           rc_idx, col_rec, vals, vals_t);
+    pem_write_slots((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, rc_idx, col_rec, vals,
+                    vals_t, [=](uint32_t x, int64_t) { return V[x]; });
 }
 
 // tile products of one A tile, at tile level (length of B's tile row) and through B's row slices;
@@ -510,21 +473,15 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
     auto wall0 = std::chrono::high_resolution_clock::now();
     if (transpose) { int32_t t = rows; rows = cols; cols = t; }
 
-    auto tiled_free = [ctx](pem_tiled* t) { pem_tiled_free(ctx, t); };
-    std::unique_ptr<pem_tiled, decltype(tiled_free)> T(new pem_tiled(), tiled_free);
-    T->uid = pem_next_uid();
-    T->dtype = dtype;
-    T->rows = rows; T->cols = cols; T->nnz = nnz;
-    T->tile_rows = (int32_t)(((int64_t)rows + PEM_TILE - 1) / PEM_TILE);
-    T->tile_cols = (int32_t)(((int64_t)cols + PEM_TILE - 1) / PEM_TILE);
+    pem_tiled_ptr T = pem_tiled_new(ctx, dtype, rows, cols, nnz);
     int32_t *sI = nullptr, *sJ = nullptr;      // device copies of a COO that came from the host
     char* sV = nullptr;
     uint64_t *keys = nullptr, *keys_sorted = nullptr;
-    uint32_t *pos = nullptr, *pos_sorted = nullptr, *start_tmp = nullptr;
+    uint32_t *pos = nullptr, *start_tmp = nullptr;
     char* tmp = nullptr;
-    pem_guard g(ctx, sI, sJ, sV, keys, keys_sorted, pos, pos_sorted, start_tmp, tmp);
+    pem_guard g(ctx, sI, sJ, sV, keys, keys_sorted, pos, start_tmp, tmp);
     // on failure nothing may still be writing a buffer that goes back to the cache (the copy stream may still be
-    // filling sV or reading pos_sorted): declared after the guard, so it waits before the guard frees
+    // filling sV or reading T->val_pos): declared after T and the guard, so it waits before either frees
     struct wait_on_failure {
         pem_ctx* ctx;
         pem_tiled** out;
@@ -536,8 +493,6 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
         }
     } idle{ctx, out};
 
-    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
-    PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
     float kernel_ms = 0.f;
 
     if (nnz > 0) {
@@ -562,8 +517,8 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
         PEM_TRY(pem_alloc(ctx, &keys, (size_t)nnz));
         PEM_TRY(pem_alloc(ctx, &keys_sorted, (size_t)nnz));
         PEM_TRY(pem_alloc(ctx, &pos, (size_t)nnz));
-        PEM_TRY(pem_alloc(ctx, &pos_sorted, (size_t)nnz));
-        PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, (size_t)nnz * vsz));
+        // the sorted positions are the value map: slot x of vals holds V[val_pos[x]] (pem_tiled_set_values)
+        PEM_TRY(pem_tiled_alloc_values(ctx, T.get()));
         PEM_CK(cudaMemsetAsync(ctx->d_scalars, 0, PEM_NSCALARS * sizeof(int64_t), ctx->stream));
 
         int grid = (int)std::min<int64_t>(pem_div_up(nnz, 256), (int64_t)ctx->sm_count * 32);
@@ -572,18 +527,18 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
 
         // one radix sort of (key, original position) over the bits in use
         size_t tmp_bytes = 0, tmp2 = 0;
-        PEM_CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys, keys_sorted, pos, pos_sorted, nnz, 0, 8 + cb + rb, ctx->stream));
+        PEM_CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys, keys_sorted, pos, T->val_pos, nnz, 0, 8 + cb + rb, ctx->stream));
         PEM_TRY(pem_alloc(ctx, &start_tmp, (size_t)nnz + 1));
         cub::CountingInputIterator<uint32_t> iota(0);
         HeadPred pred{keys_sorted};
         int64_t* d_count = ctx->d_scalars + SC_COUNT;
         PEM_CK(cub::DeviceSelect::If(nullptr, tmp2, iota, start_tmp, d_count, nnz, pred, ctx->stream));
         PEM_TRY(pem_alloc(ctx, &tmp, std::max(tmp_bytes, tmp2)));
-        PEM_CK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, keys_sorted, pos, pos_sorted, nnz, 0, 8 + cb + rb, ctx->stream));
+        PEM_CK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, keys_sorted, pos, T->val_pos, nnz, 0, 8 + cb + rb, ctx->stream));
         PEM_CK(cub::DeviceSelect::If(tmp, tmp2, iota, start_tmp, d_count, nnz, pred, ctx->stream));
-        PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)nnz));
         k_rc_idx<<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(keys_sorted, nnz, T->rc_idx);
         PEM_LAUNCHED();
+        cudaStream_t gather = ctx->stream;
         if (own) {
             // The values are gathered into tile order on the COPY stream, behind their upload; the engine's
             // stream does not wait here: tile build and the symbolic steps of a product need masks only, so
@@ -591,24 +546,19 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
             PEM_CK(cudaEventCreateWithFlags(&T->ev_vals, cudaEventDisableTiming));
             PEM_CK(cudaEventRecord(ctx->ev_copy[0], ctx->stream));                  // sorted positions are final
             PEM_CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
-            if (dtype == PEM_F32)
-                k_gather_vals<float><<<pem_div_up(nnz, 256), 256, 0, ctx->copy_stream>>>(pos_sorted, reinterpret_cast<const float*>(dV), nnz, reinterpret_cast<float*>(T->vals));
-            else
-                k_gather_vals<double><<<pem_div_up(nnz, 256), 256, 0, ctx->copy_stream>>>(pos_sorted, reinterpret_cast<const double*>(dV), nnz, T->vals);
-            PEM_LAUNCHED();
+            gather = ctx->copy_stream;
+        }
+        pem_by_dtype(dtype, [&](auto v) {
+            using VT = decltype(v);
+            k_gather_vals<VT><<<pem_div_up(nnz, 256), 256, 0, gather>>>(T->val_pos, pem_vals<VT>(dV), nnz, pem_vals<VT>(T->vals));
+        });
+        PEM_LAUNCHED();
+        if (own) {
             PEM_CK(cudaEventRecord(T->ev_vals, ctx->copy_stream));
             T->vals_pending = true;
             T->pend_buf = std::exchange(sV, nullptr);                             // freed once the gather is known to be done
-        } else {
-            if (dtype == PEM_F32)
-                k_gather_vals<float><<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(pos_sorted, reinterpret_cast<const float*>(dV), nnz, reinterpret_cast<float*>(T->vals));
-            else
-                k_gather_vals<double><<<pem_div_up(nnz, 256), 256, 0, ctx->stream>>>(pos_sorted, reinterpret_cast<const double*>(dV), nnz, T->vals);
-            PEM_LAUNCHED();
         }
         pem_free(ctx, pos);
-        // the sorted positions are the value map: slot x of vals holds V[val_pos[x]] (pem_tiled_set_values)
-        T->val_pos = std::exchange(pos_sorted, nullptr);
         PEM_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, PEM_NSCALARS * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
         PEM_CK(cudaStreamSynchronize(ctx->stream));
         pem_free(ctx, tmp);
@@ -622,39 +572,25 @@ static int convert_coo_any(pem_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz
         int64_t cnt = ctx->h_scalars[SC_COUNT];
         if (cnt >= (int64_t(1) << 31) - 1) return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 tiles");
         T->tiles = (int32_t)cnt;
-        size_t n = (size_t)cnt;
-        PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1));
-        PEM_CK(cudaMemcpyAsync(T->tile_nnz_ptr, start_tmp, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+        PEM_TRY(pem_tiled_alloc_tiles(ctx, T.get()));
+        PEM_CK(cudaMemcpyAsync(T->tile_nnz_ptr, start_tmp, (size_t)cnt * 4, cudaMemcpyDeviceToDevice, ctx->stream));
         pem_free(ctx, start_tmp);
-        PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
-        PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16));
-        PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
-        PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n));
-        PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
-        PEM_TRY(pem_alloc(ctx, &T->col_occ, n));
-        PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
         PEM_CK(cudaEventRecord(ctx->ev[0], ctx->stream));
         k_build_tiles<<<pem_div_up(cnt, 128), 128, 0, ctx->stream>>>(
             keys_sorted, T->tile_nnz_ptr, (int)cnt, (uint32_t)nnz, cb, T->tile_rows, T->masks, T->masks_t,
             T->row_ptr, T->tile_col_idx, T->tile_row_idx, T->tile_row_ptr, T->col_occ, T->row_occ, ctx->d_scalars);
         PEM_LAUNCHED();
         PEM_CK(cudaEventRecord(ctx->ev[1], ctx->stream));
-        T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
-        PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
         PEM_CK(cudaMemcpyAsync(ctx->h_scalars, ctx->d_scalars, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        PEM_CK(cudaStreamSynchronize(ctx->stream));
+        PEM_TRY(pem_tiled_publish(ctx, T.get()));
         pem_free(ctx, keys_sorted);
         if (ctx->h_scalars[SC_ERR] & 2) return ctx->fail(PEM_ERR_DUPLICATE, "duplicate (i,j) in the COO input");
         cudaEventElapsedTime(&kernel_ms, ctx->ev[0], ctx->ev[1]);
     } else {
-        PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, 1));
+        PEM_TRY(pem_tiled_alloc(ctx, T.get()));
+        PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
         PEM_CK(cudaMemsetAsync(T->tile_nnz_ptr, 0, 4, ctx->stream));
-        PEM_TRY(pem_alloc(ctx, &T->vals, 0)); PEM_TRY(pem_alloc(ctx, &T->masks, 0)); PEM_TRY(pem_alloc(ctx, &T->masks_t, 0));
-        PEM_TRY(pem_alloc(ctx, &T->row_ptr, 0)); PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, 0));
-        PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, 0)); PEM_TRY(pem_alloc(ctx, &T->col_occ, 0)); PEM_TRY(pem_alloc(ctx, &T->row_occ, 0));
-        PEM_TRY(pem_alloc(ctx, &T->rc_idx, 0)); PEM_TRY(pem_alloc(ctx, &T->val_pos, 0));
-        T->h_tile_row_ptr.assign((size_t)T->tile_rows + 1, 0);
-        PEM_CK(cudaStreamSynchronize(ctx->stream));
+        PEM_TRY(pem_tiled_publish(ctx, T.get()));
     }
     if (times) {
         auto wall1 = std::chrono::high_resolution_clock::now();
@@ -808,12 +744,11 @@ int pem_tiled_build_views(pem_ctx* ctx, const pem_tiled* Tc, bool as_a, bool as_
         PEM_TRY(pem_alloc(ctx, &rec, n16));
         PEM_TRY(pem_alloc_bytes(ctx, (void**)&vt, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype))));
         if (T->tiles) {
-            if (T->dtype == PEM_F32)
-                k_col_views<float><<<pem_div_up(T->tiles, 128), 128, 0, ctx->stream>>>(
-                    T->tiles, T->tile_nnz_ptr, T->masks_t, T->rc_idx, reinterpret_cast<const float*>(T->vals), rec, reinterpret_cast<float*>(vt));
-            else
-                k_col_views<double><<<pem_div_up(T->tiles, 128), 128, 0, ctx->stream>>>(T->tiles, T->tile_nnz_ptr, T->masks_t, T->rc_idx,
-                                                                                       T->vals, rec, vt);
+            pem_by_dtype(T->dtype, [&](auto v) {
+                using VT = decltype(v);
+                k_col_views<VT><<<pem_div_up(T->tiles, 128), 128, 0, ctx->stream>>>(
+                    T->tiles, T->tile_nnz_ptr, T->masks_t, T->rc_idx, pem_vals<VT>(T->vals), rec, pem_vals<VT>(vt));
+            });
             PEM_LAUNCHED();
         }
         T->col_rec = std::exchange(rec, nullptr);
@@ -845,13 +780,12 @@ static int set_values_any(pem_ctx* ctx, pem_tiled* T, const void* V, int dtype)
         dV = staged;
     }
     if (T->tiles) {
-        if (dtype == PEM_F32)
-            k_refresh_vals<float><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
-                T->tiles, T->tile_nnz_ptr, T->val_pos, static_cast<const float*>(dV), T->rc_idx, T->col_rec,
-                reinterpret_cast<float*>(T->vals), reinterpret_cast<float*>(T->vals_t));
-        else
-            k_refresh_vals<double><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
-                T->tiles, T->tile_nnz_ptr, T->val_pos, static_cast<const double*>(dV), T->rc_idx, T->col_rec, T->vals, T->vals_t);
+        pem_by_dtype(dtype, [&](auto v) {
+            using VT = decltype(v);
+            k_refresh_vals<VT><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
+                T->tiles, T->tile_nnz_ptr, T->val_pos, pem_vals<VT>(dV), T->rc_idx, T->col_rec, pem_vals<VT>(T->vals),
+                pem_vals<VT>(T->vals_t));
+        });
         PEM_LAUNCHED();
     }
     // default contract, as for conversion: a host V is free again when the call returns (the kernel may still run)
@@ -868,13 +802,11 @@ int pem_tiled_write_slots(pem_ctx* ctx, pem_tiled* T, const void* dV)
         PEM_CK(cudaMemcpyAsync(T->vals, dV, (size_t)T->nnz * pem_vsize(T->dtype), cudaMemcpyDeviceToDevice, ctx->stream));
         return PEM_OK;
     }
-    if (T->dtype == PEM_F32)
-        k_refresh_slots<float><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
-            T->tiles, T->tile_nnz_ptr, static_cast<const float*>(dV), T->rc_idx, T->col_rec, reinterpret_cast<float*>(T->vals),
-            reinterpret_cast<float*>(T->vals_t));
-    else
-        k_refresh_slots<double><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
-            T->tiles, T->tile_nnz_ptr, static_cast<const double*>(dV), T->rc_idx, T->col_rec, T->vals, T->vals_t);
+    pem_by_dtype(T->dtype, [&](auto v) {
+        using VT = decltype(v);
+        k_refresh_slots<VT><<<pem_div_up(T->tiles, 256), 256, 0, ctx->stream>>>(
+            T->tiles, T->tile_nnz_ptr, pem_vals<VT>(dV), T->rc_idx, T->col_rec, pem_vals<VT>(T->vals), pem_vals<VT>(T->vals_t));
+    });
     PEM_LAUNCHED();
     return PEM_OK;
 }
@@ -892,29 +824,19 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
     *out = nullptr;
     PEM_CK(cudaSetDevice(ctx->device));
     PEM_TRY(pem_tiled_wait_vals(ctx, A));
-    auto tiled_free = [ctx](pem_tiled* t) { pem_tiled_free(ctx, t); };
-    std::unique_ptr<pem_tiled, decltype(tiled_free)> T(new pem_tiled(), tiled_free);
-    T->uid = pem_next_uid();
-    T->dtype = A->dtype;
-    T->rows = A->cols; T->cols = A->rows; T->nnz = A->nnz;
-    T->tile_rows = A->tile_cols; T->tile_cols = A->tile_rows; T->tiles = A->tiles;
+    pem_tiled_ptr T = pem_tiled_new(ctx, A->dtype, A->cols, A->rows, A->nnz);
+    T->tiles = A->tiles;
     const size_t n = (size_t)A->tiles;
     uint64_t *keys = nullptr, *keys2 = nullptr;
     int32_t *ids = nullptr, *perm = nullptr;
     int64_t* nptr = nullptr;
     char* tmp = nullptr;
     pem_guard g(ctx, keys, keys2, ids, perm, nptr, tmp);
-    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
-    PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
-    PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype)))); PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz));
-    PEM_TRY(pem_alloc(ctx, &T->val_pos, (size_t)T->nnz));
-    PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
-    PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
-    PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
-    PEM_TRY(pem_alloc(ctx, &T->col_occ, n)); PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
+    PEM_TRY(pem_tiled_alloc(ctx, T.get()));
     if (n == 0) {
+        PEM_CK(cudaMemsetAsync(T->tile_row_ptr, 0, ((size_t)T->tile_rows + 1) * 4, ctx->stream));
         PEM_CK(cudaMemsetAsync(T->tile_nnz_ptr, 0, 4, ctx->stream));
-        T->h_tile_row_ptr.assign((size_t)T->tile_rows + 1, 0);
+        PEM_TRY(pem_tiled_publish(ctx, T.get()));
         *out = T.release();
         return PEM_OK;
     }
@@ -932,21 +854,16 @@ int pem_tiled_transpose(pem_ctx* ctx, const pem_tiled* A, pem_tiled** out)
     k_transpose_counts<<<pem_div_up((int64_t)n + 1, 256), 256, 0, ctx->stream>>>(perm, A->tile_nnz_ptr, (int)n, nptr);
     PEM_LAUNCHED();
     PEM_TRY(pem_scan_exclusive_i64(ctx, nptr, (int64_t)n + 1));
-    if (A->dtype == PEM_F32)
-        k_transpose_tiles<float><<<pem_div_up((int64_t)n, 128), 128, 0, ctx->stream>>>(
+    pem_by_dtype(A->dtype, [&](auto v) {
+        using VT = decltype(v);
+        k_transpose_tiles<VT><<<pem_div_up((int64_t)n, 128), 128, 0, ctx->stream>>>(
             (int)n, T->tile_rows, perm, nptr, A->tile_nnz_ptr, A->masks, A->masks_t, A->tile_row_idx, A->tile_col_idx, A->col_occ,
-            A->row_occ, A->rc_idx, reinterpret_cast<const float*>(A->vals), A->val_pos, T->tile_nnz_ptr, T->masks, T->masks_t,
-            T->row_ptr, T->tile_row_idx, T->tile_col_idx, T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx,
-            reinterpret_cast<float*>(T->vals), T->val_pos);
-    else
-        k_transpose_tiles<double><<<pem_div_up((int64_t)n, 128), 128, 0, ctx->stream>>>(
-            (int)n, T->tile_rows, perm, nptr, A->tile_nnz_ptr, A->masks, A->masks_t, A->tile_row_idx, A->tile_col_idx, A->col_occ,
-            A->row_occ, A->rc_idx, A->vals, A->val_pos, T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr, T->tile_row_idx,
-            T->tile_col_idx, T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx, T->vals, T->val_pos);
+            A->row_occ, A->rc_idx, pem_vals<VT>(A->vals), A->val_pos, T->tile_nnz_ptr, T->masks, T->masks_t, T->row_ptr,
+            T->tile_row_idx, T->tile_col_idx, T->tile_row_ptr, T->col_occ, T->row_occ, T->rc_idx, pem_vals<VT>(T->vals),
+            T->val_pos);
+    });
     PEM_LAUNCHED();
-    T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
-    PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PEM_CK(cudaStreamSynchronize(ctx->stream));
+    PEM_TRY(pem_tiled_publish(ctx, T.get()));
     pem_free(ctx, keys); pem_free(ctx, keys2); pem_free(ctx, ids); pem_free(ctx, perm); pem_free(ctx, nptr); pem_free(ctx, tmp);
     *out = T.release();
     return PEM_OK;

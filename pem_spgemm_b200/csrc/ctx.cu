@@ -393,12 +393,7 @@ void pem_tiled_free(pem_ctx* ctx, pem_tiled* t)
         if ((uint64_t)it->first[0] == t->uid || (uint64_t)it->first[1] == t->uid) it = ctx->plans.erase(it);
         else ++it;
     }
-    pem_free(ctx, t->vals); pem_free(ctx, t->tile_nnz_ptr); pem_free(ctx, t->masks);
-    pem_free(ctx, t->masks_t); pem_free(ctx, t->row_ptr); pem_free(ctx, t->tile_row_ptr);
-    pem_free(ctx, t->tile_col_idx); pem_free(ctx, t->tile_row_idx); pem_free(ctx, t->col_occ);
-    pem_free(ctx, t->row_occ); pem_free(ctx, t->rc_idx); pem_free(ctx, t->val_pos); pem_free(ctx, t->srow_ptr); pem_free(ctx, t->srow_tile);
-    pem_free(ctx, t->row_rec); pem_free(ctx, t->col_rec); pem_free(ctx, t->vals_t);
-    pem_free(ctx, t->add_src);
+    for (void** f : t->buffers()) pem_free(ctx, *f);
     delete t;
 }
 

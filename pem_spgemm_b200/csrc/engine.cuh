@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 
+#include <algorithm>
 #include <array>
 #include <cstdint>
 #include <cstdio>
@@ -186,6 +187,25 @@ static inline int pem_div_up(int64_t a, int64_t b) { return (int)((a + b - 1) / 
 enum { PEM_F64 = 0, PEM_F32 = 1 };
 static inline size_t pem_vsize(int dtype) { return dtype == PEM_F32 ? 4 : 8; }
 
+// A launch written once for both value types: launch(float{}) or launch(double{}) by dtype, the lambda taking the type
+// as `using VT = decltype(v)`; pem_vals<VT> views a value array (double* in the handles, void* at the ABI) as VT.
+template <class F>
+static inline void pem_by_dtype(int dtype, F&& launch)
+{
+    if (dtype == PEM_F32) launch(float{});
+    else launch(double{});
+}
+template <class V> static inline V* pem_vals(void* p) { return static_cast<V*>(p); }
+template <class V> static inline const V* pem_vals(const void* p) { return static_cast<const V*>(p); }
+
+// What built a tiled matrix: the entry points that rewrite its values from the same sources accept those only
+enum { PEM_BUILT_INPUT = 0, PEM_BUILT_RESULT = 1, PEM_BUILT_SUM = 2 };
+struct pem_origin {
+    int kind = PEM_BUILT_INPUT;       // conversion or transpose: new values come through pem_tiled_set_values
+    uint64_t a_uid = 0, b_uid = 0;    // result: the operands of its product; sum: A and B, in that order
+    int32_t rb = 0, re = 0;           // result: its panel
+};
+
 struct pem_tiled {
     uint64_t uid = 0;                 // unique per conversion (the pattern is immutable, the values may be refreshed): key of the size plans
     int dtype = PEM_F64;
@@ -221,15 +241,119 @@ struct pem_tiled {
     uint32_t* row_rec = nullptr;      // [tiles*16]  masks[i]   | row_ptr[i] << 16          (operand A)
     uint32_t* col_rec = nullptr;      // [tiles*16]  masks_t[i] | first value of column << 24 (operand B)
     double* vals_t = nullptr;         // [nnz] tile-major, column-major inside a tile        (operand B)
-    // built by pem_result_to_tiled: the product (and panel) the result came from, whose structure this handle holds;
-    // pem_tiled_refresh_from_result accepts results of that product only.  src_a_uid == 0: not built from a result
-    uint64_t src_a_uid = 0, src_b_uid = 0;
-    int32_t src_rb = 0, src_re = 0;
-    // built by pem_tiled_add: the operands S = alpha*A + beta*B was built from (pem_tiled_add_values accepts these, in
-    // this order) and, per tile of S, the tile of A and of B it holds (-1: none).  add_a_uid == 0: not a sum
-    uint64_t add_a_uid = 0, add_b_uid = 0;
-    int2* add_src = nullptr;          // [tiles]
+    // pem_tiled_refresh_from_result accepts results of the product (and panel) a result handle came from, whose structure
+    // it holds; pem_tiled_add_values the operands of a sum.  A transpose records nothing.
+    pem_origin origin;
+    int2* add_src = nullptr;          // [tiles] sum S = alpha*A + beta*B: per tile of S the tile of A and of B it holds (-1: none)
+    // every device array above, in the order pem_tiled_free releases them: the twelve of the structure
+    // (pem_tiled_alloc_values / _tiles), the caches built on first use and a sum's source tiles
+    std::array<void**, 18> buffers()
+    {
+        return {(void**)&vals, (void**)&tile_nnz_ptr, (void**)&masks, (void**)&masks_t, (void**)&row_ptr,
+                (void**)&tile_row_ptr, (void**)&tile_col_idx, (void**)&tile_row_idx, (void**)&col_occ,
+                (void**)&row_occ, (void**)&rc_idx, (void**)&val_pos, (void**)&srow_ptr, (void**)&srow_tile,
+                (void**)&row_rec, (void**)&col_rec, (void**)&vals_t, (void**)&add_src};
+    }
 };
+
+// A handle under construction: freed with everything it holds unless the builder releases it into *out
+struct pem_tiled_deleter {
+    pem_ctx* ctx;
+    void operator()(pem_tiled* t) const { pem_tiled_free(ctx, t); }
+};
+using pem_tiled_ptr = std::unique_ptr<pem_tiled, pem_tiled_deleter>;
+
+// A new rows x cols handle of nnz values: its own uid (the key of the size plans), its tile counts from the shape
+static inline pem_tiled_ptr pem_tiled_new(pem_ctx* ctx, int dtype, int32_t rows, int32_t cols, int64_t nnz)
+{
+    pem_tiled_ptr T(new pem_tiled(), pem_tiled_deleter{ctx});
+    T->uid = pem_next_uid();
+    T->dtype = dtype;
+    T->rows = rows; T->cols = cols; T->nnz = nnz;
+    T->tile_rows = pem_div_up(rows, PEM_TILE);
+    T->tile_cols = pem_div_up(cols, PEM_TILE);
+    return T;
+}
+// The structure arrays of a handle: the per-value ones (vals, rc_idx, val_pos) for T->nnz values, the per-tile ones
+// (tile_row_ptr included) for T->tiles tiles and T->tile_rows tile rows.  Nothing is written.
+static inline int pem_tiled_alloc_values(pem_ctx* ctx, pem_tiled* T)
+{
+    PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype))));
+    PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz));
+    return pem_alloc(ctx, &T->val_pos, (size_t)T->nnz);
+}
+static inline int pem_tiled_alloc_tiles(pem_ctx* ctx, pem_tiled* T)
+{
+    const size_t n = (size_t)T->tiles;
+    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1)); PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1));
+    PEM_TRY(pem_alloc(ctx, &T->masks, n * 16)); PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16));
+    PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16)); PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n));
+    PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n)); PEM_TRY(pem_alloc(ctx, &T->col_occ, n));
+    return pem_alloc(ctx, &T->row_occ, n);
+}
+static inline int pem_tiled_alloc(pem_ctx* ctx, pem_tiled* T)
+{
+    PEM_TRY(pem_tiled_alloc_values(ctx, T));
+    return pem_tiled_alloc_tiles(ctx, T);
+}
+// Every builder's last step before it releases T into *out: mirror tile_row_ptr into h_tile_row_ptr (panel calls find
+// their tile range there without a device read) and wait for the stream.  Read-backs the builder enqueued before are
+// then on the host, for its last checks.
+static inline int pem_tiled_publish(pem_ctx* ctx, pem_tiled* T)
+{
+    T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
+    PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+    PEM_CK(cudaStreamSynchronize(ctx->stream));
+    return PEM_OK;
+}
+
+// ---- value slots of a tiled matrix: k_refresh_vals, k_refresh_slots, k_col_views (convert.cu), k_add_vals (sum.cu) ----
+// Slot in vals_t (column-major inside a tile) of the value in row r of a column whose record (col_rec) is cr, in the
+// tile whose values start at ts: the column's first value (top byte of the record) plus the column's rows above r.
+__device__ __forceinline__ uint32_t pem_col_slot(uint32_t ts, uint32_t cr, unsigned r)
+{
+    return ts + (cr >> 24) + __popc(cr & ((1u << r) - 1u));
+}
+
+// Writes value(x, t) into every value slot x of tile t of a tiled matrix: into vals and, when the column-major view
+// exists, into vals_t.  A warp takes 32 consecutive tiles and walks their slots, which are contiguous, one per lane, so
+// the (r, c) bytes and the value arrays move in whole sectors; a lane finds its tile among the warp's 32 in five
+// shuffles over the tiles' first offsets, which the lanes hold in registers.  The caller passes the thread indices, read
+// in the kernel, where its launch bounds limit them.
+template <class T, class F>
+__device__ __forceinline__ void
+pem_write_slots(int64_t gid, unsigned tid, int cnt, const uint32_t* __restrict__ tile_nnz_ptr,
+                const uint8_t* __restrict__ rc_idx, const uint32_t* __restrict__ col_rec, T* __restrict__ vals,
+                T* __restrict__ vals_t, F value)
+{
+    const int64_t t0 = (gid >> 5) * 32;
+    if (t0 >= cnt) return;                          // whole warps leave together
+    const int lane = tid & 31;
+    const int nt = (int)(cnt - t0 < 32 ? cnt - t0 : 32);
+    const uint32_t first = tile_nnz_ptr[t0 + min(lane, nt)];   // lanes >= nt hold the end: above every x
+    const uint32_t s = __shfl_sync(0xffffffffu, first, 0), e = tile_nnz_ptr[t0 + nt];
+    for (uint32_t b = s; b < e; b += 32) {
+        const uint32_t x = b + lane;
+        int j = 0;                                  // last tile of the warp whose first offset is <= x
+        uint32_t ts = s;
+#pragma unroll
+        for (int step = 16; step > 0; step >>= 1) {
+            const uint32_t f = __shfl_sync(0xffffffffu, first, j + step);
+            if (f <= x) { j += step; ts = f; }
+        }
+        if (x < e) {
+            const T v = value(x, t0 + j);
+            vals[x] = v;
+            if (vals_t) {
+                const unsigned rc = rc_idx[x];
+                const unsigned r = rc >> 4, c = rc & 15u;
+                const uint32_t cr = col_rec[(size_t)(t0 + j) * 16 + c];
+                vals_t[pem_col_slot(ts, cr, r)] = v;
+            }
+        }
+    }
+}
 
 // ---------------------------------------------------------------------------------------
 // result: C or a tile-row panel of C

@@ -123,21 +123,14 @@ k_operand_slots(int n_tile_rows, const int64_t* __restrict__ c_row_ptr, const ui
 // The structure of T from a result-shaped tile list C (tile-row pointer over [rb, re), tile rows and columns, row masks,
 // value offsets): the arrays of T, T->vals included, allocated for T->tiles tiles (C' tile keep[i] for tile i, or tile i
 // when keep is null) and T->nnz values, and every array but vals written.  T's shape is set by the caller.  Stream order;
-// the caller fills vals, copies h_tile_row_ptr and synchronises.  pem_result_to_tiled and pem_tiled_add (sum.cu).
+// the caller fills vals and publishes T.  pem_result_to_tiled and pem_tiled_add (sum.cu).
 int pem_operand_structure(pem_ctx* ctx, const pem_result* C, const int32_t* keep, pem_tiled* T)
 {
     const int ntr = C->re - C->rb;
     const int64_t cnt = T->tiles;
-    const size_t n = (size_t)cnt;
     int64_t* row_pos = nullptr;
     pem_guard g(ctx, row_pos);
-    PEM_TRY(pem_alloc_bytes(ctx, (void**)&T->vals, std::max<size_t>(1, (size_t)T->nnz * pem_vsize(T->dtype))));
-    PEM_TRY(pem_alloc(ctx, &T->rc_idx, (size_t)T->nnz)); PEM_TRY(pem_alloc(ctx, &T->val_pos, (size_t)T->nnz));
-    PEM_TRY(pem_alloc(ctx, &T->tile_row_ptr, (size_t)T->tile_rows + 1));
-    PEM_TRY(pem_alloc(ctx, &T->tile_nnz_ptr, n + 1)); PEM_TRY(pem_alloc(ctx, &T->masks, n * 16));
-    PEM_TRY(pem_alloc(ctx, &T->masks_t, n * 16)); PEM_TRY(pem_alloc(ctx, &T->row_ptr, n * 16));
-    PEM_TRY(pem_alloc(ctx, &T->tile_col_idx, n)); PEM_TRY(pem_alloc(ctx, &T->tile_row_idx, n));
-    PEM_TRY(pem_alloc(ctx, &T->col_occ, n)); PEM_TRY(pem_alloc(ctx, &T->row_occ, n));
+    PEM_TRY(pem_tiled_alloc(ctx, T));
 
     const int64_t threads = std::max<int64_t>(cnt, T->tile_rows) + 1;
     k_operand_tiles<<<pem_div_up(threads, 128), 128, 0, ctx->stream>>>(
@@ -167,14 +160,8 @@ int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out)
     if (C->nnz >= (int64_t(1) << 32) - 1) return ctx->fail(PEM_ERR_LIMIT, "nnz must be below 2^32-1 (32-bit tile value offsets)");
     if (C->tiles >= (int64_t(1) << 31) - 1) return ctx->fail(PEM_ERR_LIMIT, "more than 2^31 tiles");
     PEM_CK(cudaSetDevice(ctx->device));
-    auto tiled_free = [ctx](pem_tiled* t) { pem_tiled_free(ctx, t); };
-    std::unique_ptr<pem_tiled, decltype(tiled_free)> T(new pem_tiled(), tiled_free);
-    T->uid = pem_next_uid();
-    T->dtype = C->dtype;
-    T->rows = C->rows; T->cols = C->cols; T->nnz = C->nnz;
-    T->tile_rows = (int32_t)(((int64_t)C->rows + PEM_TILE - 1) / PEM_TILE);
-    T->tile_cols = C->tile_cols;
-    T->src_a_uid = C->a_uid; T->src_b_uid = C->b_uid; T->src_rb = C->rb; T->src_re = C->re;
+    pem_tiled_ptr T = pem_tiled_new(ctx, C->dtype, C->rows, C->cols, C->nnz);
+    T->origin = {PEM_BUILT_RESULT, C->a_uid, C->b_uid, C->rb, C->re};
     int32_t* keep = nullptr;                  // kept C' tile of every tile of T (keep-empty results only)
     char* tmp = nullptr;
     pem_guard g(ctx, keep, tmp);
@@ -200,9 +187,7 @@ int pem_result_to_tiled(pem_ctx* ctx, const pem_result* C, pem_tiled** out)
     PEM_TRY(pem_operand_structure(ctx, C, keep, T.get()));
     // every value keeps its slot: empty tiles hold none
     if (T->nnz) PEM_CK(cudaMemcpyAsync(T->vals, C->vals, (size_t)T->nnz * pem_vsize(T->dtype), cudaMemcpyDeviceToDevice, ctx->stream));
-    T->h_tile_row_ptr.resize((size_t)T->tile_rows + 1);
-    PEM_CK(cudaMemcpyAsync(T->h_tile_row_ptr.data(), T->tile_row_ptr, ((size_t)T->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PEM_CK(cudaStreamSynchronize(ctx->stream));
+    PEM_TRY(pem_tiled_publish(ctx, T.get()));
     *out = T.release();
     return PEM_OK;
 }
@@ -211,11 +196,12 @@ int pem_tiled_refresh_from_result(pem_ctx* ctx, pem_tiled* T, const pem_result* 
 {
     PEM_RANGE("pem_tiled_refresh_from_result");
     if (!ctx || !T || !C) return PEM_ERR_ARG;
-    if (!T->src_a_uid)
+    const pem_origin& o = T->origin;
+    if (o.kind != PEM_BUILT_RESULT)
         return ctx->fail(PEM_ERR_ARG, "pem_tiled_refresh_from_result: the matrix was not built by pem_result_to_tiled "
                                       "(refresh it with pem_tiled_set_values)");
     if (C->stage != 3) return ctx->fail(PEM_ERR_ARG, "pem_tiled_refresh_from_result needs a complete result (step 3 done)");
-    if (C->a_uid != T->src_a_uid || C->b_uid != T->src_b_uid || C->rb != T->src_rb || C->re != T->src_re)
+    if (C->a_uid != o.a_uid || C->b_uid != o.b_uid || C->rb != o.rb || C->re != o.re)
         return ctx->fail(PEM_ERR_ARG, "pem_tiled_refresh_from_result: the result is not of the product the matrix was built from");
     PEM_CK(cudaSetDevice(ctx->device));
     return pem_tiled_write_slots(ctx, T, C->vals);

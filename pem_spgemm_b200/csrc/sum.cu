@@ -115,10 +115,9 @@ __device__ __forceinline__ bool operand_slot(int t, unsigned r, unsigned c, cons
     return (m >> c) & 1u;
 }
 
-// S's values from A's and B's, one lane per value slot of S, laid out as refresh_vals (convert.cu): a warp takes 32
-// consecutive tiles of S and walks their slots; a lane finds its tile among the warp's 32 in five shuffles over the
-// tiles' first offsets.  An entry of both operands is fl(fl(alpha*a) + fl(beta*b)), one of A only fl(alpha*a), one of B
-// only fl(beta*b).  When S's column-major view exists the value also goes to its slot of vals_t (k_col_views' slot).
+// S's values from A's and B's, one lane per value slot of S (pem_write_slots), into vals_t too when S's column-major
+// view exists.  An entry of both operands is fl(fl(alpha*a) + fl(beta*b)), one of A only fl(alpha*a), one of B only
+// fl(beta*b).
 template <class T>
 __global__ void __launch_bounds__(256)
 k_add_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint8_t* __restrict__ rc_idx,
@@ -129,38 +128,18 @@ k_add_vals(int cnt, const uint32_t* __restrict__ tile_nnz_ptr, const uint8_t* __
            const uint8_t* __restrict__ b_row_ptr, const T* __restrict__ b_vals, T* __restrict__ vals,
            T* __restrict__ vals_t)
 {
-    const int64_t t0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32;
-    if (t0 >= cnt) return;                          // whole warps leave together
-    const int lane = threadIdx.x & 31;
-    const int nt = (int)(cnt - t0 < 32 ? cnt - t0 : 32);
-    const uint32_t first = tile_nnz_ptr[t0 + min(lane, nt)];   // lanes >= nt hold the end: above every x
-    const uint32_t s = __shfl_sync(0xffffffffu, first, 0), e = tile_nnz_ptr[t0 + nt];
-    for (uint32_t b = s; b < e; b += 32) {
-        const uint32_t x = b + lane;
-        int j = 0;                                  // last tile of the warp whose first offset is <= x
-        uint32_t ts = s;
-#pragma unroll
-        for (int step = 16; step > 0; step >>= 1) {
-            const uint32_t f = __shfl_sync(0xffffffffu, first, j + step);
-            if (f <= x) { j += step; ts = f; }
-        }
-        if (x < e) {
-            const unsigned rc = rc_idx[x];
-            const unsigned r = rc >> 4, c = rc & 15u;
-            const int2 st = src[t0 + j];
-            uint32_t xa = 0, xb = 0;
-            const bool in_a = operand_slot(st.x, r, c, a_nnz_ptr, a_masks, a_row_ptr, &xa);
-            const bool in_b = operand_slot(st.y, r, c, b_nnz_ptr, b_masks, b_row_ptr, &xb);
-            const T pa = in_a ? mul_rn(alpha, a_vals[xa]) : T(0);
-            const T pb = in_b ? mul_rn(beta, b_vals[xb]) : T(0);
-            const T v = in_a && in_b ? add_rn(pa, pb) : in_a ? pa : pb;
-            vals[x] = v;
-            if (vals_t) {
-                const uint32_t cr = col_rec[(size_t)(t0 + j) * 16 + c];
-                vals_t[ts + (cr >> 24) + __popc(cr & ((1u << r) - 1u))] = v;
-            }
-        }
-    }
+    pem_write_slots((int64_t)blockIdx.x * blockDim.x + threadIdx.x, threadIdx.x, cnt, tile_nnz_ptr, rc_idx, col_rec, vals,
+                    vals_t, [=](uint32_t x, int64_t t) {
+                        const unsigned rc = rc_idx[x];
+                        const unsigned r = rc >> 4, c = rc & 15u;
+                        const int2 st = src[t];
+                        uint32_t xa = 0, xb = 0;
+                        const bool in_a = operand_slot(st.x, r, c, a_nnz_ptr, a_masks, a_row_ptr, &xa);
+                        const bool in_b = operand_slot(st.y, r, c, b_nnz_ptr, b_masks, b_row_ptr, &xb);
+                        const T pa = in_a ? mul_rn(alpha, a_vals[xa]) : T(0);
+                        const T pb = in_b ? mul_rn(beta, b_vals[xb]) : T(0);
+                        return in_a && in_b ? add_rn(pa, pb) : in_a ? pa : pb;
+                    });
 }
 
 }  // namespace
@@ -170,15 +149,13 @@ static int add_vals_launch(pem_ctx* ctx, pem_tiled* S, double alpha, const pem_t
 {
     if (!S->tiles) return PEM_OK;
     const int grid = pem_div_up(S->tiles, 256);        // a warp per 32 tiles
-    if (S->dtype == PEM_F32)
-        k_add_vals<float><<<grid, 256, 0, ctx->stream>>>(
-            S->tiles, S->tile_nnz_ptr, S->rc_idx, S->add_src, S->col_rec, (float)alpha, A->tile_nnz_ptr, A->masks,
-            A->row_ptr, reinterpret_cast<const float*>(A->vals), (float)beta, B->tile_nnz_ptr, B->masks, B->row_ptr,
-            reinterpret_cast<const float*>(B->vals), reinterpret_cast<float*>(S->vals), reinterpret_cast<float*>(S->vals_t));
-    else
-        k_add_vals<double><<<grid, 256, 0, ctx->stream>>>(
-            S->tiles, S->tile_nnz_ptr, S->rc_idx, S->add_src, S->col_rec, alpha, A->tile_nnz_ptr, A->masks, A->row_ptr,
-            A->vals, beta, B->tile_nnz_ptr, B->masks, B->row_ptr, B->vals, S->vals, S->vals_t);
+    pem_by_dtype(S->dtype, [&](auto v) {
+        using VT = decltype(v);
+        k_add_vals<VT><<<grid, 256, 0, ctx->stream>>>(
+            S->tiles, S->tile_nnz_ptr, S->rc_idx, S->add_src, S->col_rec, (VT)alpha, A->tile_nnz_ptr, A->masks, A->row_ptr,
+            pem_vals<VT>(A->vals), (VT)beta, B->tile_nnz_ptr, B->masks, B->row_ptr, pem_vals<VT>(B->vals),
+            pem_vals<VT>(S->vals), pem_vals<VT>(S->vals_t));
+    });
     PEM_LAUNCHED();
     return PEM_OK;
 }
@@ -193,12 +170,8 @@ int pem_tiled_add(pem_ctx* ctx, double alpha, const pem_tiled* A, double beta, c
     if (A->rows != B->rows || A->cols != B->cols) return ctx->fail(PEM_ERR_ARG, "pem_tiled_add: the operands' shapes differ");
     if (A->dtype != B->dtype) return ctx->fail(PEM_ERR_ARG, "pem_tiled_add: the operands' value types differ");
     PEM_CK(cudaSetDevice(ctx->device));
-    auto tiled_free = [ctx](pem_tiled* t) { pem_tiled_free(ctx, t); };
-    std::unique_ptr<pem_tiled, decltype(tiled_free)> S(new pem_tiled(), tiled_free);
-    S->uid = pem_next_uid();
-    S->dtype = A->dtype;
-    S->rows = A->rows; S->cols = A->cols;
-    S->tile_rows = A->tile_rows; S->tile_cols = A->tile_cols;
+    pem_tiled_ptr S = pem_tiled_new(ctx, A->dtype, A->rows, A->cols, 0);       // nnz: read back below
+    S->origin = {PEM_BUILT_SUM, A->uid, B->uid};
     const int na = A->tiles, nb = B->tiles;
     const int64_t n = (int64_t)na + nb;
     int32_t *a_rank = nullptr, *b_rank = nullptr, *s_row = nullptr, *s_col = nullptr;
@@ -252,10 +225,7 @@ int pem_tiled_add(pem_ctx* ctx, double alpha, const pem_tiled* A, double beta, c
     PEM_TRY(pem_tiled_wait_vals(ctx, A));
     PEM_TRY(pem_tiled_wait_vals(ctx, B));
     PEM_TRY(add_vals_launch(ctx, S.get(), alpha, A, beta, B));
-    S->h_tile_row_ptr.resize((size_t)S->tile_rows + 1);
-    PEM_CK(cudaMemcpyAsync(S->h_tile_row_ptr.data(), S->tile_row_ptr, ((size_t)S->tile_rows + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PEM_CK(cudaStreamSynchronize(ctx->stream));
-    S->add_a_uid = A->uid; S->add_b_uid = B->uid;
+    PEM_TRY(pem_tiled_publish(ctx, S.get()));
     *out = S.release();
     return PEM_OK;
 }
@@ -264,9 +234,9 @@ int pem_tiled_add_values(pem_ctx* ctx, pem_tiled* S, double alpha, const pem_til
 {
     PEM_RANGE("pem_tiled_add_values");
     if (!ctx || !S || !A || !B) return PEM_ERR_ARG;
-    if (!S->add_a_uid)
+    if (S->origin.kind != PEM_BUILT_SUM)
         return ctx->fail(PEM_ERR_ARG, "pem_tiled_add_values: the matrix was not built by pem_tiled_add");
-    if (A->uid != S->add_a_uid || B->uid != S->add_b_uid)
+    if (A->uid != S->origin.a_uid || B->uid != S->origin.b_uid)
         return ctx->fail(PEM_ERR_ARG, "pem_tiled_add_values: A and B are not the operands the sum was built from, in that order");
     PEM_CK(cudaSetDevice(ctx->device));
     PEM_TRY(pem_tiled_wait_vals(ctx, A));
