@@ -348,7 +348,7 @@ k_expand(int np, int p0, int rb, int64_t P, const int64_t* __restrict__ pptr, co
     }
 }
 
-// ---- block-local sort of short rows --------------------------------------------------------------------
+// ---- sort of short rows in shared memory, row by row ---------------------------------------------------
 // The compacted pairs are grouped by C' row in row order (products are expanded in A-tile order):
 // off[r] = first pair of row r (lower bound of r among the keys' row fields), off[nrows] = F.
 template <class KeyT>
@@ -375,181 +375,184 @@ k_max_segment(int nrows, const int* __restrict__ off, int64_t* __restrict__ scal
     if ((threadIdx.x & 31) == 0 && len > 0) atomicMax((long long*)&scalars[SC_MAXD], (long long)len);
 }
 
-// One block per C' row.  The row's pairs become (tile column, position) words in shared memory - position in the
-// low bits makes the words distinct, so the order of equal tile columns is the expansion order (ascending A tile),
-// as a stable sort would give.  Rows whose window of tile columns fits a small bitmap (stencil / FEM products: a
-// few hundred pairs over a few thousand columns) are ordered WITHOUT a comparison network: bitmap of the occupied
-// columns -> popcount prefix = rank of every column = the pair's group (its C' tile), counting scatter into the
-// groups, then each group (a tile's handful of pairs) is put in position order by one thread.  Seven block
-// barriers where the bitonic network needs one per stage (36 for 256 pairs); rows with a wide window or a long
-// group fall back to the network.  One pass over the data either way, where the radix sort needs one per digit.
+// One warp per C' row, several independent rows per block (no block barrier).  The row's pairs become (tile column,
+// position) words in shared memory - position in the low bits makes the words distinct, so the order of equal tile
+// columns is the expansion order (ascending A tile), as a stable sort would give.  Rows whose window of tile columns
+// fits a small bitmap (stencil / FEM products: a few hundred pairs over a few thousand columns) are ordered WITHOUT a
+// comparison network: bitmap of the occupied columns -> popcount prefix = rank of every column = the pair's group
+// (its C' tile); a histogram of the groups taken in input order, 32 pairs at a time, gives every pair its rank among
+// the earlier pairs of its group (the pairs of one group in a step are __match_any_sync peers, the last of them
+// advances the group's count); the scan of the counts gives the group starts, and pair i goes to start(group) + rank.
+// The scatter is stable, so every group comes out in position order whatever its size.  Rows with a wider window
+// sort the same words with a bitonic network run by the warp.  One pass over the data either way, where the radix
+// sort needs one per digit.
 constexpr int RS_BMW = 256;            // bitmap words of the counting path: windows of up to 8192 tile columns
-constexpr int RS_GROUP_MAX = 32;       // longest group one thread sorts by insertion
 
-template <int THREADS>
-__device__ __forceinline__ unsigned rs_block_scan(unsigned* a, int n, unsigned* wsum)   // in-place exclusive scan, returns the total
+// shared memory of one row (one warp) when no row holds more than cap pairs (cap: a power of two >= 32)
+constexpr int rs_warp_bytes(int cap) { return cap * 12 + RS_BMW * 6; }
+
+__device__ __forceinline__ unsigned rs_warp_scan(unsigned x, int lane)      // inclusive scan over the warp
 {
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int per = (n + THREADS - 1) / THREADS;
-    const int b = min(tid * per, n), e = min(b + per, n);
-    unsigned local = 0;
-    for (int i = b; i < e; ++i) local += a[i];
-    unsigned incl = local;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-        const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += t;
+        const unsigned t = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= o) x += t;
     }
-    if (lane == 31) wsum[warp] = incl;
-    __syncthreads();
-    unsigned woff = 0, total = 0;
-#pragma unroll
-    for (int w = 0; w < THREADS / 32; ++w) {
-        const unsigned x = wsum[w];
-        if (w < warp) woff += x;
-        total += x;
-    }
-    unsigned run = woff + incl - local;
-    for (int i = b; i < e; ++i) {
-        const unsigned x = a[i];
-        a[i] = run;
-        run += x;
-    }
-    __syncthreads();
-    return total;
+    return x;
 }
 
-template <class KeyT, int THREADS, int POS_BITS>
-__global__ void __launch_bounds__(THREADS)
-k_row_sort(int wbits, int CAP, const int* __restrict__ off, const KeyT* __restrict__ in_key, const int2* __restrict__ in_val,
-           KeyT* __restrict__ out_key, int2* __restrict__ out_val, int64_t* __restrict__ row_tiles)
+template <class KeyT, int POS_BITS>
+__global__ void __launch_bounds__(128)
+k_row_sort(int nrows, int wbits, int cap, const int* __restrict__ off, const KeyT* __restrict__ in_key,
+           const int2* __restrict__ in_val, KeyT* __restrict__ out_key, int2* __restrict__ out_val,
+           int64_t* __restrict__ row_tiles)
 {
-    // CAP: power of two >= the longest row of this product (<= 1 << POS_BITS) and >= RS_BMW: sizes the arrays below
-    extern __shared__ unsigned sk[];                     // [CAP] the row's words
-    unsigned* ow = sk + CAP;                             // [CAP] words in group order
-    unsigned* cnt = ow + CAP;                            // [CAP] pairs per group -> group starts -> group ends
-    unsigned* bm = cnt + CAP;                            // [RS_BMW] occupied tile columns, then their popcount prefix
-    unsigned short* sg = reinterpret_cast<unsigned short*>(bm + RS_BMW);     // [CAP] group of every pair
-    __shared__ unsigned wsum[THREADS / 32];
-    __shared__ unsigned s_maxcol, s_maxgroup, s_heads;
-    const int r = blockIdx.x, tid = threadIdx.x;
+    extern __shared__ __align__(16) unsigned char rs_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int r = blockIdx.x * (blockDim.x >> 5) + warp;
+    if (r >= nrows) return;
     const int s = off[r], n = off[r + 1] - s;
-    if (n == 0) return;                                  // uniform over the block
+    if (n == 0) return;                                  // uniform over the warp
+    unsigned* sk = reinterpret_cast<unsigned*>(rs_smem + (size_t)warp * rs_warp_bytes(cap));   // [cap] the row's words
+    unsigned* gr = sk + cap;                             // [cap] (group << 16) | rank among the group's earlier pairs
+    unsigned* bm = gr + cap;                             // [RS_BMW] occupied tile columns
+    unsigned short* cnt = reinterpret_cast<unsigned short*>(bm + RS_BMW);   // [cap] pairs per group -> group starts
+    unsigned short* ow = cnt + cap;                      // [cap] positions in output order
+    unsigned short* pre = ow + cap;                      // [RS_BMW] distinct columns below each bitmap word
+    constexpr int U = 8;                                 // 256 pairs per trip: eight independent global loads in flight
     const KeyT jmask = ((KeyT)1 << wbits) - 1;
-    if (tid == 0) { s_maxcol = 0; s_maxgroup = 0; s_heads = 0; }
-    for (int i = tid; i < RS_BMW; i += THREADS) bm[i] = 0;
-    __syncthreads();
+    reinterpret_cast<uint4*>(bm)[lane] = make_uint4(0u, 0u, 0u, 0u);
+    reinterpret_cast<uint4*>(bm)[lane + 32] = make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
     unsigned mc = 0;
-    for (int i = tid; i < n; i += THREADS) {
-        const unsigned col = (unsigned)(in_key[s + i] & jmask);
-        sk[i] = (col << POS_BITS) | (unsigned)i;
-        mc = max(mc, col);
-    }
+    for (int b = 0; b < n; b += 32 * U) {
+        KeyT k[U];
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) mc = max(mc, __shfl_xor_sync(0xffffffffu, mc, o));
-    if ((tid & 31) == 0) atomicMax(&s_maxcol, mc);
-    __syncthreads();
-    const unsigned* src = sk;                            // where the ordered words end up
-    bool counted = s_maxcol < (unsigned)RS_BMW * 32u;
-    if (counted) {
-        for (int i = tid; i < n; i += THREADS) {
-            const unsigned col = sk[i] >> POS_BITS;
-            atomicOr(&bm[col >> 5], 1u << (col & 31));
+        for (int u = 0; u < U; ++u) {
+            const int i = b + u * 32 + lane;
+            k[u] = i < n ? in_key[s + i] : (KeyT)0;
         }
-        __syncthreads();
-        // bm[w] := (columns below word w) << 6 | nothing lost: keep the word itself in registers while scanning counts
-        unsigned words[(RS_BMW + THREADS - 1) / THREADS];
 #pragma unroll
-        for (int q = 0; q < (RS_BMW + THREADS - 1) / THREADS; ++q) {
-            const int w = tid + q * THREADS;
-            words[q] = w < RS_BMW ? bm[w] : 0u;
-            if (w < RS_BMW) cnt[w] = __popc(words[q]);
-        }
-        __syncthreads();
-        const int D = (int)rs_block_scan<THREADS>(cnt, RS_BMW, wsum);       // cnt[w] = distinct columns below word w
-        unsigned pre[(RS_BMW + THREADS - 1) / THREADS];
-#pragma unroll
-        for (int q = 0; q < (RS_BMW + THREADS - 1) / THREADS; ++q) {
-            const int w = tid + q * THREADS;
-            pre[q] = w < RS_BMW ? cnt[w] : 0u;
-        }
-        __syncthreads();
-        // the prefix moves behind the bitmap's role: ow is free until the scatter, so park it there
-#pragma unroll
-        for (int q = 0; q < (RS_BMW + THREADS - 1) / THREADS; ++q) {
-            const int w = tid + q * THREADS;
-            if (w < RS_BMW) ow[w] = pre[q];
-        }
-        for (int g = tid; g < D; g += THREADS) cnt[g] = 0;
-        __syncthreads();
-        for (int i = tid; i < n; i += THREADS) {
-            const unsigned col = sk[i] >> POS_BITS;
-            const unsigned g = ow[col >> 5] + __popc(bm[col >> 5] & ((1u << (col & 31)) - 1u));
-            sg[i] = (unsigned short)g;
-            atomicAdd(&cnt[g], 1u);
-        }
-        __syncthreads();
-        unsigned mg = 0;
-        for (int g = tid; g < D; g += THREADS) mg = max(mg, cnt[g]);
-        if (mg) atomicMax(&s_maxgroup, mg);
-        __syncthreads();
-        counted = s_maxgroup <= (unsigned)RS_GROUP_MAX;
-        if (counted) {
-            rs_block_scan<THREADS>(cnt, D, wsum);                            // group starts
-            for (int i = tid; i < n; i += THREADS) ow[atomicAdd(&cnt[sg[i]], 1u)] = sk[i];   // cnt[g] ends as the group's end
-            __syncthreads();
-            for (int g = tid; g < D; g += THREADS) {                         // position order inside the group
-                const int b = g ? (int)cnt[g - 1] : 0, e = (int)cnt[g];
-                for (int i = b + 1; i < e; ++i) {
-                    const unsigned key = ow[i];
-                    int x = i - 1;
-                    while (x >= b && ow[x] > key) { ow[x + 1] = ow[x]; --x; }
-                    ow[x + 1] = key;
-                }
+        for (int u = 0; u < U; ++u) {
+            const int i = b + u * 32 + lane;
+            if (i < n) {
+                const unsigned col = (unsigned)(k[u] & jmask);
+                sk[i] = (col << POS_BITS) | (unsigned)i;
+                mc = max(mc, col);
+                atomicOr(&bm[(col >> 5) & (RS_BMW - 1)], col < (unsigned)RS_BMW * 32u ? 1u << (col & 31) : 0u);
             }
-            __syncthreads();
-            src = ow;
-            if (tid == 0) s_heads = (unsigned)D;         // the groups ARE the row's C' tiles
         }
     }
-    if (!counted) {                                      // bitonic network over the words
+    if (lane < (-n & 31)) sk[n + lane] = 0u;             // pad to whole steps of 32 (cap is a multiple of 32)
+    mc = __reduce_max_sync(0xffffffffu, mc);
+    __syncwarp();
+    const bool counted = mc < (unsigned)RS_BMW * 32u;    // (uniform over the warp)
+    unsigned tiles;
+    if (counted) {
+        {   // the lane's eight bitmap words: distinct columns below each, packed in pairs of 16 bits
+            const uint4 a = reinterpret_cast<const uint4*>(bm)[2 * lane], b = reinterpret_cast<const uint4*>(bm)[2 * lane + 1];
+            const unsigned c[8] = {(unsigned)__popc(a.x), (unsigned)__popc(a.y), (unsigned)__popc(a.z), (unsigned)__popc(a.w),
+                                   (unsigned)__popc(b.x), (unsigned)__popc(b.y), (unsigned)__popc(b.z), (unsigned)__popc(b.w)};
+            const unsigned local = c[0] + c[1] + c[2] + c[3] + c[4] + c[5] + c[6] + c[7];
+            const unsigned incl = rs_warp_scan(local, lane);
+            tiles = __shfl_sync(0xffffffffu, incl, 31);  // the groups ARE the row's C' tiles
+            unsigned x = incl - local, p[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                p[q] = x | ((x + c[2 * q]) << 16);
+                x += c[2 * q] + c[2 * q + 1];
+            }
+            reinterpret_cast<uint4*>(pre)[lane] = make_uint4(p[0], p[1], p[2], p[3]);
+        }
+        for (int g = lane; g < (int)tiles; g += 32) cnt[g] = 0;
+        __syncwarp();
+        const unsigned lt = (1u << lane) - 1u;
+        const int last = ((n + 31) & ~31) - 1;           // last padded word
+        for (int b = 0; b < n; b += 32 * U) {            // histogram in input order: rank = earlier pairs of the group
+            unsigned g[U];                               // groups of eight steps first: their loads overlap
+#pragma unroll
+            for (int u = 0; u < U; ++u) g[u] = sk[min(b + u * 32 + lane, last)] >> POS_BITS;
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const unsigned col = g[u];
+                g[u] = (pre[col >> 5] + __popc(bm[col >> 5] & ((1u << (col & 31)) - 1u))) | (b + u * 32 + lane < n ? 0u : 0xFFFFu);
+            }
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const int i = b + u * 32 + lane;
+                if (b + u * 32 >= n) break;              // (uniform over the warp)
+                const unsigned peers = __match_any_sync(0xffffffffu, g[u]);
+                const unsigned rank = cnt[i < n ? g[u] : 0u] + __popc(peers & lt);
+                __syncwarp();
+                gr[i] = (g[u] << 16) | rank;
+                if (i < n && (peers >> lane) == 1u) cnt[g[u]] = (unsigned short)(rank + 1);   // the last peer advances the count
+                __syncwarp();
+            }
+        }
+        unsigned carry = 0;                              // group starts: exclusive scan of the counts, 32 groups a step
+        for (int g0 = 0; g0 < (int)tiles; g0 += 32) {
+            const int g = g0 + lane;
+            const unsigned c = g < (int)tiles ? cnt[g] : 0u;
+            const unsigned incl = rs_warp_scan(c, lane);
+            if (g < (int)tiles) cnt[g] = (unsigned short)(carry + incl - c);
+            carry += __shfl_sync(0xffffffffu, incl, 31);
+        }
+        __syncwarp();
+        for (int b = 0; b < n; b += 32 * U) {
+            unsigned v[U], d[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) v[u] = gr[min(b + u * 32 + lane, last)];
+#pragma unroll
+            for (int u = 0; u < U; ++u) d[u] = cnt[(v[u] >> 16) & (cap - 1)] + (v[u] & 0xFFFFu);   // (padding: any start, not stored)
+#pragma unroll
+            for (int u = 0; u < U; ++u)
+                if (b + u * 32 + lane < n) ow[d[u]] = (unsigned short)(b + u * 32 + lane);
+        }
+        __syncwarp();
+    } else {                                             // bitonic network over the words
         int N = 2;
         while (N < n) N <<= 1;
-        for (int i = n + tid; i < N; i += THREADS) sk[i] = 0xFFFFFFFFu;
-        __syncthreads();
+        for (int i = n + lane; i < N; i += 32) sk[i] = 0xFFFFFFFFu;
+        __syncwarp();
         for (int k = 2; k <= N; k <<= 1)
             for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int t = tid; t < (N >> 1); t += THREADS) {
+                for (int t = lane; t < (N >> 1); t += 32) {
                     const int lo = ((t & ~(j - 1)) << 1) | (t & (j - 1));      // element with bit j clear
                     const int hi = lo | j;
                     const unsigned a = sk[lo], b = sk[hi];
                     const bool up = (lo & k) == 0;
                     if ((a > b) == up) { sk[lo] = b; sk[hi] = a; }
                 }
-                __syncthreads();
+                __syncwarp();
             }
+        unsigned heads = 0;                              // the network does not know the runs of equal tile columns: count them
+        for (int i = lane; i < n; i += 32) heads += (i == 0 || (sk[i - 1] >> POS_BITS) != (sk[i] >> POS_BITS)) ? 1u : 0u;
+        tiles = __reduce_add_sync(0xffffffffu, heads);
     }
     const KeyT rowbits = (KeyT)(unsigned)r << wbits;
-    if (counted) {                                       // (uniform over the block)
-        for (int i = tid; i < n; i += THREADS) {
-            const unsigned e = src[i];
-            out_key[s + i] = rowbits | (KeyT)(e >> POS_BITS);
-            out_val[s + i] = in_val[s + (int)(e & ((1u << POS_BITS) - 1u))];
-        }
-    } else {                                             // the network does not know the runs of equal tile columns: count them
-        unsigned heads = 0;
-        for (int i = tid; i < n; i += THREADS) {
-            const unsigned e = src[i];
-            heads += (i == 0 || (src[i - 1] >> POS_BITS) != (e >> POS_BITS)) ? 1u : 0u;
-            out_key[s + i] = rowbits | (KeyT)(e >> POS_BITS);
-            out_val[s + i] = in_val[s + (int)(e & ((1u << POS_BITS) - 1u))];
+    for (int b = 0; b < n; b += 32 * U) {
+        unsigned e[U];
+        int2 v[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int i = b + u * 32 + lane;
+            if (i < n) e[u] = counted ? sk[ow[i]] : sk[i];
         }
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) heads += __shfl_xor_sync(0xffffffffu, heads, o);
-        if ((tid & 31) == 0 && heads) atomicAdd(&s_heads, heads);
-        __syncthreads();
+        for (int u = 0; u < U; ++u) {
+            const int i = b + u * 32 + lane;
+            if (i < n) v[u] = in_val[s + (int)(e[u] & ((1u << POS_BITS) - 1u))];
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int i = b + u * 32 + lane;
+            if (i < n) {
+                out_key[s + i] = rowbits | (KeyT)(e[u] >> POS_BITS);
+                out_val[s + i] = v[u];
+            }
+        }
     }
-    if (tid == 0) row_tiles[r] = (int64_t)s_heads;      // C' tiles of this row: scanned into C's row pointer by the caller
+    if (lane == 0) row_tiles[r] = (int64_t)tiles;       // C' tiles of this row: scanned into C's row pointer by the caller
 }
 
 // C' tiles of the row-sorted pairs: one warp per C' row walks the row's sorted keys, numbers the runs of equal
@@ -789,12 +792,11 @@ int esc_run(pem_ctx* ctx, const pem_tiled* A, const pem_tiled* B, pem_result* C,
     ctx->last_sort_passes = by_rows ? 0 : (wbits + rbits + 7) / 8;
     if (by_rows) {
         KT_BEGIN(KT_SORT);
-        int cap = RS_BMW;                               // shared memory by the longest row: short rows keep more blocks per SM
+        int cap = 32;                                   // shared memory by the longest row: short rows keep more warps per SM
         while (cap < longest_row) cap <<= 1;
-        if (cap <= 256)
-            k_row_sort<KeyT, 64, RS_SMALL_BITS><<<nrows, 64, (size_t)cap * 14 + RS_BMW * 4, ctx->stream>>>(wbits, cap, seg_off, key_a, val_a, key_b, val_b, C->row_ptr);
-        else
-            k_row_sort<KeyT, 128, RS_SMALL_BITS><<<nrows, 128, (size_t)cap * 14 + RS_BMW * 4, ctx->stream>>>(wbits, cap, seg_off, key_a, val_a, key_b, val_b, C->row_ptr);
+        const int rows = std::min(4, std::max(1, 32768 / rs_warp_bytes(cap)));     // rows (warps) per block, <= 32 KB
+        k_row_sort<KeyT, RS_SMALL_BITS><<<pem_div_up(nrows, rows), 32 * rows, (size_t)rows * rs_warp_bytes(cap), ctx->stream>>>(
+            nrows, wbits, cap, seg_off, key_a, val_a, key_b, val_b, C->row_ptr);
         KT_END(KT_SORT);
         PEM_LAUNCHED();
         std::swap(key_a, key_b);
